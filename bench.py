@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W          # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K --warmup W   # the reference's CPU path (oracle port)
+    python bench.py ... --dump-outputs DIR   # also writes what the last timed step computed, as DIR/<name>.npy
 
 A "step" is ONE nnGParareal iteration (parareal.py:301-439) from the state after the coarse
 initialisation: fine solves of all N slices (batched RK8, sharded by slice over the ranks + one
@@ -69,7 +70,36 @@ def parse():
                     help="with --iteration 0: also time this later iteration (2 500-row dataset, steady-state neighbours); 0 = off")
     ap.add_argument("--e2e-steps", type=int, default=2)
     ap.add_argument("--profile-out", default=None, help="write the per-kernel-class event timings here (json)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the arrays the last timed step computed as DIR/<name>.npy (float64), to compare two builds")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl b200: the reference arm samples timings, it does not compute the iteration")
+    return args
+
+
+DUMP_LIMIT = 64 * 10 ** 6  # bytes on disk, .npy headers included
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes every array as out_dir/<name>.npy in float64.  The arrays share their first axis; when they would take more
+    than DUMP_LIMIT bytes, the same seeded sample of rows is taken from each and its row numbers go to sample_rows.npy."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    n = {a.shape[0] for a in arrays.values()}
+    assert len(n) == 1, "the dumped arrays must share their first axis"
+    n = n.pop()
+    total = sum(a.nbytes for a in arrays.values())
+    budget = DUMP_LIMIT - 1024 * (len(arrays) + 1)   # room for the headers
+    if total > budget:
+        keep = max(1, n * budget // (total + 8 * n))
+        rows = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        arrays = {k: a[rows] for k, a in arrays.items()}
+        arrays["sample_rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def nll_flops(m):
@@ -261,6 +291,8 @@ def run_synthetic(args):
     ev[1].record()
     sync_all()
     clk = clocks.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"pred": pred_all[:Q].cpu().numpy()})
     t = torch.tensor([ev[0].elapsed_time(ev[1])], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -379,10 +411,12 @@ def main():
 
     fp64_peak = None
 
-    def measure(iteration, steps, warmup, with_clocks):
+    def measure(iteration, steps, warmup, with_clocks, keep_outputs=False):
         """times `steps` repetitions of nnGParareal iteration number `iteration` (0-based) of the run: the run is
         advanced to the start of that iteration once (real iterations 0 .. iteration-1), its state is saved, and every
-        timed step restores it (device copies + dataset truncation, outside the kernels but inside the timed region)"""
+        timed step restores it (device copies + dataset truncation, outside the kernels but inside the timed region).
+        keep_outputs: also return, on the host, the state the last timed step left (new iterate, coarse and fine
+        values, per-slice errors)"""
         nonlocal fp64_peak
         model = nn.CudaNNGP(n=d, N=N, nn=m, seed=45, handle=h)
         st = par.device_setup(model)
@@ -435,6 +469,10 @@ def main():
         ev[1].record()
         sync_all()
         clk = clocks.stop() if clocks else None
+        outputs = None
+        if keep_outputs:
+            outputs = {"u_next": st["u_next"].cpu().numpy(), "uG_next": st["uG_next"].cpu().numpy(),
+                       "uF": st["uF"][:N + 1].cpu().numpy(), "err": err}
         ms_total = ev[0].elapsed_time(ev[1])
         t = torch.tensor([ms_total], dtype=torch.float64, device=dev)
         if world > 1:
@@ -458,9 +496,9 @@ def main():
         return dict(ms_step=ms_step, clk=clk, launches=int(launches), kernels=kernels, err=err, fit_ms=fit_ms, fit_n=fit_n,
                     fit_tf=fit_tf, fine_ms=fine_ms, fine_launches=fine_launches, f_flops=f_flops, rk_tf=rk_tf,
                     nm_runs=nm_runs / steps, nll_evals=nll_evals / steps, n_sweep=n_sweep, n_fine=n_fine,
-                    rows=int(h.dataset_rows()), I0=I0, steps=steps)
+                    rows=int(h.dataset_rows()), I0=I0, steps=steps, outputs=outputs)
 
-    R = measure(args.iteration, args.steps, args.warmup, with_clocks=True)
+    R = measure(args.iteration, args.steps, args.warmup, with_clocks=True, keep_outputs=bool(args.dump_outputs))
     ms_step, clk, steps = R["ms_step"], R["clk"], R["steps"]
     # ---- rooflines of the two kernels that share the step (fine propagator, GP fit): FP64 pipe ------
     peak_src = ("FP64 FMA micro-benchmark run in this process (nngp_bench_fp64: 8 independent DFMA chains per thread, "
@@ -572,6 +610,8 @@ def main():
         if args.profile_out:
             with open(args.profile_out, "w") as fh:
                 json.dump(line, fh, indent=1)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, R["outputs"])
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

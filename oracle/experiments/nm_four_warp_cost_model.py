@@ -10,7 +10,7 @@ import os, sys, collections, numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
 from oracle import nngp as onn
-z = np.load(os.path.join(ROOT, 'tests', 'golden', 'run_fhn_d512_replay.npz'))
+z = np.load(os.path.join(ROOT, 'tests', 'golden', 'run_fhn_d512_replay_k2.npz'))
 CF, CI, SYNC = 3300.0, 800.0, 150.0
 cost = lambda f: CI if not np.isfinite(f) else CF
 

@@ -1,6 +1,6 @@
 """TEST INFRASTRUCTURE / STUDY ONLY.  Which moves do the Nelder-Mead searches of a steady-state predict make?
 Traces SciPy's algorithm (oracle restatement) with the oracle objective on a replayed FHN d=512 predict
-(tests/golden/run_fhn_d512_replay.npz) and prints move counts for all searches and for the long finite ones.
+(tests/golden/run_fhn_d512_replay_k2.npz) and prints move counts for all searches and for the long finite ones.
 Result (profiles/r02/nm_moves.log): the long searches are runs of inside contraction + shrink (4 evaluations per
 iteration, all four points known when the iteration starts) -- the basis of the four-warp search kernel.
 usage: python oracle/experiments/nm_move_study.py [predict id = 3] [dimension stride = 8]"""
@@ -8,7 +8,7 @@ import os, sys, collections, numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
 from oracle import nngp as onn
-z = np.load(os.path.join(ROOT, 'tests', 'golden', 'run_fhn_d512_replay.npz'))
+z = np.load(os.path.join(ROOT, 'tests', 'golden', 'run_fhn_d512_replay_k2.npz'))
 
 def trace(func, x0, xatol=0.1, fatol=0.1):
     n = 2; maxfun = 400

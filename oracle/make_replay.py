@@ -1,4 +1,4 @@
-"""TEST INFRASTRUCTURE ONLY -- builds tests/golden/run_fhn_d512_replay.npz in the build container.
+"""TEST INFRASTRUCTURE ONLY -- builds tests/golden/run_fhn_d512_replay_k{2,3}.npz in the build container.
 
 Input: the state dump of a DEVICE run of the full-size FHN-PDE target (d=512, N=512, m=20, RK8 x 195 325 steps per
 slice -- a size the CPU reference cannot run), written by `scripts/parity_matrix.py --full --dump DIR` on the GPU box:
@@ -7,7 +7,8 @@ For a handful of predicts of iterations 3 and 4 (steady-state neighbours from sl
 dataset prefix exactly as parareal.py:336-339 does, positions the PCG64 stream of models.py:114,192 where the run
 had it, and calls the UNMODIFIED reference `NNGP_p.predict` (models.py:171-226) under oracle/ref_shim.py.  Stored per
 predict: query, the m neighbour rows in kNN order (x, F-G), the host-drawn starts, and the reference's prediction,
-per-search optimum (theta, fval) and selection.
+per-search optimum value (fval) and the theta of the search its rule selects (models.py:212-215).  One file per
+iteration keeps each under 1 MB.
 
 usage: python -m oracle.make_replay gpurun_out/replay/fhn_full_state_id.npz [workers]
 """
@@ -56,8 +57,9 @@ def main():
         xs.append(u[k][I - 1:N])
         ys.append(uF[k][I:N + 1] - uG[k][I:N + 1])
         rows_after.append(sum(a.shape[0] for a in xs))
-    out = dict(n_predicts=0, N=N, d=d, m=m, guard=float(dump["guard"]), I_sweep=I_sweep,
-               conv_int=dump["conv_int"], device_err=dump["err"])
+    meta = dict(N=N, d=d, m=m, guard=float(dump["guard"]), I_sweep=I_sweep, conv_int=dump["conv_int"],
+                device_err=dump["err"])
+    outs = {}
     for (k, i) in PICKS:
         if k >= uF.shape[0] or i < I_sweep[k]:
             continue
@@ -78,19 +80,21 @@ def main():
         probe.bit_generator.state = state
         starts = probe.integers(-8, 0, (n_tasks, 2)).astype(np.int8).reshape(d, 9, 1, 2)
         res = np.array([r[:5] for r in pool.last])          # theta0, theta1, fval, jitter, j in task order
-        idx, kq = onn.knn(q, x, m)
+        idx, _ = onn.knn(q, x, m)
+        thetas, fvals = res[:, :2].reshape(d, 9, 2), res[:, 2].reshape(d, 9)
+        sel = np.array([onn.select(fvals[j]) for j in range(d)])
+        out = outs.setdefault(k, dict(meta, n_predicts=0))
         p = out["n_predicts"]
-        out.update({f"p{p}_k": k, f"p{p}_i": i, f"p{p}_n_rows": x.shape[0], f"p{p}_query": q, f"p{p}_idx": idx,
-                    f"p{p}_xm": x[idx], f"p{p}_ym": y[idx], f"p{p}_kq": kq, f"p{p}_starts": starts,
-                    f"p{p}_preds": np.asarray(preds), f"p{p}_thetas": res[:, :2].reshape(d, 9, 2),
-                    f"p{p}_fvals": res[:, 2].reshape(d, 9),
-                    f"p{p}_device_pred": u[k + 1][i + 1] - uG[k + 1][i + 1]})
+        out.update({f"p{p}_k": k, f"p{p}_i": i, f"p{p}_n_rows": x.shape[0], f"p{p}_query": q,
+                    f"p{p}_xm": x[idx], f"p{p}_ym": y[idx], f"p{p}_starts": starts,
+                    f"p{p}_preds": np.asarray(preds), f"p{p}_theta_sel": thetas[np.arange(d), sel],
+                    f"p{p}_fvals": fvals})
         out["n_predicts"] = p + 1
-        dd = np.abs(out[f"p{p}_device_pred"] - preds)
+        dd = np.abs(u[k + 1][i + 1] - uG[k + 1][i + 1] - preds)
         print(f"predict k={k} i={i} rows={x.shape[0]} {secs:.0f}s  inf searches {np.isinf(res[:, 2]).mean():.3f}  "
               f"|device-reference| max {dd.max():.3e} median {np.median(dd):.3e}  |pred| max {np.abs(preds).max():.3e}",
               flush=True)
-        np.savez_compressed(os.path.join(OUT, "run_fhn_d512_replay.npz"), **out)
+        np.savez_compressed(os.path.join(OUT, f"run_fhn_d512_replay_k{k}.npz"), **out)
     pool.shutdown()
 
 

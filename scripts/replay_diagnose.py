@@ -9,17 +9,17 @@ from oracle import nngp as onn
 
 h = _lib.default_handle(0)
 dev = torch.device('cuda', 0)
-z = np.load(os.path.join(ROOT, "tests", "golden", "run_fhn_d512_replay.npz"))
-m, d = int(z["m"]), int(z["d"])
-for p in range(int(z["n_predicts"])):
-    P = {k: z[f"p{p}_{k}"] for k in ("k", "i", "query", "xm", "ym", "starts", "preds", "thetas", "fvals")}
+zs = [np.load(os.path.join(ROOT, "tests", "golden", f"run_fhn_d512_replay_k{k}.npz")) for k in (2, 3)]
+m, d = int(zs[0]["m"]), int(zs[0]["d"])
+for z, p in [(z, p) for z in zs for p in range(int(z["n_predicts"]))]:
+    P = {k: z[f"p{p}_{k}"] for k in ("k", "i", "query", "xm", "ym", "starts", "preds", "theta_sel", "fvals")}
     if np.abs(P["preds"]).max() < 1e-8:
         continue
     h.dataset_reset(); h.dataset_reserve(m, d); h.dataset_append_host(P["xm"], P["ym"])
     out = h.predict_host(P["query"][None], m, P["starts"][None], 1, 0.1, 0.1, details=True)
     r2 = onn.pairwise_sqdist(P["xm"], P["xm"])
     sel_r = np.array([onn.select(P["fvals"][j]) for j in range(d)])
-    th_r = P["thetas"][np.arange(d), sel_r]
+    th_r = P["theta_sel"]
     jit_r = onn.JITTERS[sel_r]
     f_r = P["fvals"][np.arange(d), sel_r]
     th_d, jit_d, f_d = out["theta_opt"][0], out["jitter_opt"][0], out["fval_opt"][0]

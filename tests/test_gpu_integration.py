@@ -2,17 +2,22 @@
 libnngpara.so through integration/cuda_backend.py -- classes that derive from the reference's own SolverRK / NNGP_p /
 ODE / Parareal, so its isinstance checks (parareal.py:37-41) and executor protocol are the real ones.
 
-Needs the reference's modules on the machine (NNGP_REFERENCE_DIR, /root/reference, or the git-ignored copy
-baseline/_ref made by scripts/stage_reference.sh); skipped otherwise."""
+The tests that execute the reference's code need its modules (NNGP_REFERENCE_DIR, or the git-ignored copy baseline/_ref
+made by scripts/stage_reference.sh) and skip without them.  What the reference driver computed on this backend is also
+stored (tests/golden/reference_driver_on_cuda_backend.json), and the package's own drivers are checked against it on
+every run."""
+import json
+import os
+
 import numpy as np
 import pytest
 
 import nearest_neighbors_gparareal_b200 as nn
-from helpers import load_run, case_system, device_system
+from helpers import GOLDEN, load_run, case_system, device_system
 from integration.ref_env import find_reference
 
-pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(find_reference() is None, reason="reference modules not on this machine")]
+pytestmark = pytest.mark.gpu
+needs_reference = pytest.mark.skipif(find_reference() is None, reason="reference modules not on this machine")
 
 
 def _ref_ode(B, key, kw):
@@ -20,6 +25,32 @@ def _ref_ode(B, key, kw):
             "burgers": lambda: B.Burgers(normalization="-11", **kw), "fhn_pde": lambda: B.FHN_PDE(**kw)}[key]()
 
 
+@pytest.mark.parametrize("name", ["lorenz_N32_m11", "fhn_d32_N32_m12", "hopf_N32_m15"])
+def test_package_drivers_reproduce_the_reference_driver_run(name):
+    """the host-protocol driver and the device-resident driver end with the K / conv_int that the reference's unmodified
+    driver reached on this backend (stored), agree bit for bit with each other, and meet the reference's own NumPy run"""
+    with open(os.path.join(GOLDEN, "reference_driver_on_cuda_backend.json")) as fh:
+        want = json.load(fh)[name]
+    z, cfg, mkw = load_run(name)
+    key, kw = case_system(name)
+    ode = device_system(key, **kw)
+    solver = nn.CudaSolverRK(ode.get_vector_field(), **{k: cfg[k] for k in ("Ng", "Nf", "F", "G")})
+    host = nn.Parareal(ode, solver, tspan=cfg["tspan"], N=cfg["N"], epsilon=float(z["epsilon"]), verbose='') \
+        .run(model='nngp', pool=nn.CudaPool(), parall='mpi', **mkw)
+    dev = nn.PararealDevice(ode, solver, tspan=cfg["tspan"], N=cfg["N"], epsilon=float(z["epsilon"]), verbose='') \
+        .run(model='nngp', **mkw)
+    K = host['k']
+    assert host['converged'] and K == want["K"] and host['conv_int'] == want["conv_int"]
+    assert dev['k'] == K and dev['conv_int'] == host['conv_int']
+    assert np.array_equal(dev['u'], host['u_last']) and np.array_equal(dev['err'], host['err'], equal_nan=True)
+    assert host['u'].shape == (cfg["N"] + 1, ode.get_dim(), K) and host['err'].shape == (cfg["N"] + 1, K)
+    if name != "hopf_N32_m15":
+        assert K == int(z["K"])
+    else:
+        assert abs(K - int(z["K"])) <= 1
+
+
+@needs_reference
 @pytest.mark.parametrize("name", ["lorenz_N32_m11", "fhn_d32_N32_m12", "hopf_N32_m15"])
 def test_unmodified_reference_driver_on_cuda_backend(name):
     from integration.cuda_backend import bind
@@ -63,6 +94,7 @@ def test_unmodified_reference_driver_on_cuda_backend(name):
         assert abs(K - int(z["K"])) <= 1
 
 
+@needs_reference
 def test_reference_plain_parareal_on_cuda_solver():
     """model='parareal' (BareParareal of the reference, models.py:74-83) with the CUDA solver and pool: the published
     Lorenz K = 15 (Table 2 of the reference)"""
@@ -75,6 +107,7 @@ def test_reference_plain_parareal_on_cuda_solver():
     assert out['k'] == 15 and out['conv_int'] == [1, 2, 3, 5, 8, 14, 17, 20, 26, 30, 33, 37, 40, 43, 50]
 
 
+@needs_reference
 def test_checkpoints_cross_the_boundary_in_both_directions(tmp_path):
     """intermediate dumps (parareal.py:114-209, 420-431): (a) written by the REFERENCE driver running on the CUDA
     backend and resumed by the reference's own load_int_dump; (b) the same dump resumed by this package's driver;

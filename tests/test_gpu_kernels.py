@@ -701,15 +701,19 @@ def test_nelder_mead_vs_oracle_on_steady_state_neighbours(handle):
 
 
 def _replay_predicts():
-    z = np.load(os.path.join(GOLDEN, "run_fhn_d512_replay.npz"))
-    return z, [{k: z[f"p{p}_{k}"] for k in ("k", "i", "n_rows", "query", "idx", "xm", "ym", "kq", "starts", "preds",
-                                                            "thetas", "fvals", "device_pred")} for p in range(int(z["n_predicts"]))]
+    """(metadata, predicts) of the replay fixtures, one file per iteration (iterations 3 and 4 of the run)"""
+    preds = []
+    for k in (2, 3):
+        z = np.load(os.path.join(GOLDEN, f"run_fhn_d512_replay_k{k}.npz"))
+        preds += [{key: z[f"p{p}_{key}"] for key in ("k", "i", "n_rows", "query", "xm", "ym", "starts", "preds",
+                                                      "theta_sel", "fvals")} for p in range(int(z["n_predicts"]))]
+    return z, preds
 
 
 def test_replayed_fhn_d512_predicts_against_the_reference(handle):
     """Predicts of iterations 3-4 of the FULL-SIZE FHN target (d=512, N=512, m=20; state dumped from a device
     run) replayed through the unmodified reference `NNGP_p.predict` under the shim (oracle/make_replay.py ->
-    tests/golden/run_fhn_d512_replay.npz): same neighbour rows, same host-drawn starts.  From slice ~20 on the
+    tests/golden/run_fhn_d512_replay_k*.npz): same neighbour rows, same host-drawn starts.  From slice ~20 on the
     trajectory sits at its steady state and the predicted correction is < 1e-9 -- nothing there can move K; the
     slices that decide K are the first ~15, where the correction is 1e-7 .. 4e-6 against epsilon = 5e-7.
     Asserted per predict, in BOTH directions:
@@ -750,7 +754,7 @@ def test_replayed_fhn_d512_predicts_against_the_reference(handle):
         tol = 1e-6 * np.maximum(1.0, np.abs(r_sel))
         dev_lower, ref_lower = g_sel < r_sel - tol, r_sel < g_sel - tol
         r_arg = np.array([onn.select(r_f[j]) for j in range(d)])
-        th_r, jit_r = P["thetas"][np.arange(d), r_arg], onn.JITTERS[r_arg]
+        th_r, jit_r = P["theta_sel"], onn.JITTERS[r_arg]
         th_d, jit_d = out["theta_opt"][0], out["jitter_opt"][0]
         r2 = onn.pairwise_sqdist(P["xm"], P["xm"])
         o = torch.empty((1, d, 1), dtype=torch.float64, device=dev)

@@ -42,6 +42,16 @@ def device_system(key, **kw):
             "fhn_pde": lambda: nn.FHN_PDE(**kw)}[key]()
 
 
+def make_dataset(rng, n, d):
+    x = rng.uniform(-1, 1, (n, d))
+    y = 1e-3 * np.sin(x @ (rng.standard_normal((d, d)) / np.sqrt(d)))
+    return x, y
+
+
+def scaled_err(a, b):
+    return float(np.max(np.abs(a - b)) / max(np.max(np.abs(b)), 1e-300))
+
+
 def samples(z):
     out = []
     for i in range(int(z["n_samples"])):

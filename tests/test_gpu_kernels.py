@@ -10,7 +10,7 @@ from nearest_neighbors_gparareal_b200 import _lib
 from oracle import nngp as onn
 from oracle import rk as ork
 from oracle import systems as osys
-from helpers import GOLDEN, load_run, samples
+from helpers import GOLDEN, load_run, make_dataset, samples, scaled_err
 
 pytestmark = pytest.mark.gpu
 
@@ -29,10 +29,6 @@ DEV = {"lorenz": lambda: nn.Lorenz(normalization='-11'), "lorenz_id": lambda: nn
 
 def relerr(a, b):
     return float(np.max(np.abs(a - b) / (np.abs(b) + 1e-300)))
-
-
-def scaled_err(a, b):
-    return float(np.max(np.abs(a - b)) / max(np.max(np.abs(b)), 1e-300))
 
 
 @pytest.fixture(scope="module")
@@ -237,12 +233,6 @@ def test_device_exp_and_rsqrt_accuracy(handle):
     assert np.max(np.abs(gl[sub] - wantl) / np.spacing(np.abs(wantl))) <= 1.0
 
 
-def make_dataset(rng, n, d):
-    x = rng.uniform(-1, 1, (n, d))
-    y = 1e-3 * np.sin(x @ (rng.standard_normal((d, d)) / np.sqrt(d)))
-    return x, y
-
-
 @pytest.mark.parametrize("n,d,m,nq", [(40, 3, 11, 1), (300, 3, 11, 5), (2000, 32, 12, 9), (3055, 512, 20, 1),
                                        (3055, 512, 20, 12), (5000, 128, 30, 33), (65, 7, 32, 3), (20, 2, 20, 2),
                                        (700, 1100, 5, 6), (20000, 8, 32, 2), (8193, 3, 20, 40), (4097, 5, 17, 1)])
@@ -279,15 +269,22 @@ def test_knn_ties_broken_by_index_and_edge_cases(handle):
     oi, od = onn.knn(q, x, 9)
     assert np.array_equal(idx[0], oi) and np.array_equal(dist[0], od)
     assert list(idx[0][:3]) == [3, 33, 63]  # same distance, ascending index
-    # exact ties across the 4096-row chunks of the two-level selection: still ascending index
+    # exact ties across the 256-row CTAs of the one-query scan (nq = 1) and across the 1024-row chunks of the two-level
+    # selection (nq = 5): still ascending index.  Only every 8th copy of row 3 is kept, so the 25 tied nearest rows
+    # reach past row 4096.
     big = np.tile(base, (300, 1))  # 9000 rows, every row repeated 300 times
+    big[np.arange(3, 9000, 30)[np.arange(300) % 8 != 0]] = base[0]
     handle.dataset_reset()
     handle.dataset_reserve(9000, 4)
     handle.dataset_append_host(big, np.zeros_like(big))
-    idx, dist = handle.knn_host(q[None], 25)
     oi, od = onn.knn(q, big, 25)
-    assert np.array_equal(idx[0], oi) and np.array_equal(dist[0], od)
-    assert list(idx[0][:4]) == [3, 33, 63, 93] and idx[0].max() > 4096 * 0  # same distance, ascending index
+    for nq, launches in ((1, 1), (5, 3)):
+        c0 = handle.launch_count()
+        idx, dist = handle.knn_host(np.repeat(q[None], nq, axis=0), 25)
+        assert handle.launch_count() - c0 == launches, nq  # scan_select_kernel / sqdist + two select_kernel levels
+        for qi in range(nq):
+            assert np.array_equal(idx[qi], oi) and np.array_equal(dist[qi], od)
+        assert list(idx[0][:4]) == [3, 243, 483, 723] and idx[0].max() > 4096  # same distance, ascending index
     handle.dataset_reset()
     handle.dataset_reserve(200, 4)
     handle.dataset_append_host(x, y)

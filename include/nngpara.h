@@ -186,6 +186,44 @@ int nngp_append_iteration(nngp_handle_t h, const double* d_u_cur, const double* 
 int nngp_rowwise_maxabs_diff(nngp_handle_t h, const double* d_a, const double* d_b, int rows,
                              int d, double* d_err, void* stream);
 
+/* ---- ensembles of independent runs (PararealEnsemble) -----------------------------------
+ * Segmented store: E members of `cap_rows` rows each share X, Y and the transposed copy of the dataset; member e's
+ * rows are the global rows [e cap, e cap + rows_e), so the GP kernels gather them by global index.  A handle holds
+ * either a plain dataset (nngp_dataset_*) or a segmented store: reserving one discards the other.
+ * nngp_seg_reserve: (re)lays the store out for E members of cap_rows rows; growing the capacity keeps every
+ * member's rows (copied to the new layout, synchronises); changing E or d needs an empty store (nngp_seg_reset). */
+int nngp_seg_reserve(nngp_handle_t h, int n_members, long long cap_rows, int d);
+/* every member back to 0 rows */
+int nngp_seg_reset(nngp_handle_t h);
+/* rows held by `member` (-1 outside [0, E)); rows per member the store has room for */
+long long nngp_seg_rows(nngp_handle_t h, int member);
+long long nngp_seg_cap(nngp_handle_t h);
+/* parareal.py:336-339 for n runs in one launch: position p of the state (device, member stride ld_state >= (N+1) d,
+ * row stride d) appends x <- u_cur[p, I_p-1:N], D <- uF[p, I_p:N+1] - uG_cur[p, I_p:N+1] to segment members[p].
+ * members[n], I[n]: host arrays, I_p in [1, N]. */
+int nngp_seg_append_iteration(nngp_handle_t h, int n, const int* members, const int* I, const double* d_u_cur,
+                              const double* d_uF, const double* d_uG_cur, long long ld_state, int N, int d,
+                              void* stream);
+/* kNN of nq queries, each in its own rows of the store: query q (device, row stride ld_q) searches global rows
+ * [base[q], base[q] + rows[q]) (host arrays, rows[q] >= m).  idx[nq,m]: global indices ordered by (distance, index),
+ * dist[nq,m]: squared distances -- idx - base[q] and dist equal nngp_knn on that segment alone.  r2 (optional,
+ * device [nq,m,m]): the neighbour distance matrix of the GP.  Segments up to 8192 rows with m <= 32 take one fused
+ * launch; larger ones or m up to 160 the distance + selection kernels. */
+int nngp_knn_segmented(nngp_handle_t h, const double* d_q, long long ld_q, int nq, int m, const long long* base,
+                       const long long* rows, long long* d_idx, double* d_dist, double* d_r2, void* stream);
+/* dst[dst_idx[r], :] = src[src_idx[r], :] for r < rows, rows of d doubles; a NULL index list is the
+ * identity.  Device pointers; gathers and scatters the rows of an ensemble's state. */
+int nngp_copy_rows(nngp_handle_t h, const double* d_src, const long long* d_src_idx, double* d_dst,
+                   const long long* d_dst_idx, long long rows, long long d, void* stream);
+/* nngp_sweep for E runs in lockstep, slices min(I) .. N-1, enqueued with no host round trip.  State u_next,
+ * uG_next: device [E, N+1, d]; position p belongs to segment members[p] (host) and sweeps slices I[p] .. N-1 (host,
+ * ascending in p, so the runs active at a slice are a prefix).  Per slice: one coarse launch over the active runs,
+ * one segmented kNN, one fit over all their predicts.  d_starts: the starts of every predict, slice-major -- for
+ * slice i the [d,9,R,2] blocks of the active positions in order.  Each run's results equal its nngp_sweep. */
+int nngp_ensemble_sweep(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g, const double* d_t, int N,
+                        int E, const int* members, const int* I, int m, int n_restarts, const signed char* d_starts,
+                        double fatol, double xatol, double* d_u_next, double* d_uG_next, int d, void* stream);
+
 /* test hook: the device exp(-|x|), 1/|x| and -- when d_exp10 (2n doubles) is not NULL -- [10**x | log|x| + 3 ln 2]
  * used inside the GP kernels */
 int nngp_selftest_math(nngp_handle_t h, const double* d_x, int n, double* d_exp_neg, double* d_rcp,

@@ -15,8 +15,9 @@ from .models import ModelAbstr, BareParareal, CudaNNGP, NNGP_p
 from .gp_full import CudaGP, GPjax_p
 from .pool import MyPool, CudaPool
 from .parareal import Parareal, PararealLight, PararealDevice
+from .ensemble import PararealEnsemble
 
 __all__ = ["Normalize", "ODE", "FHN_ODE", "Rossler", "Hopf", "DblPend", "Brusselator", "Lorenz",
            "ThomasLabyrinth", "FHN_PDE", "Burgers", "Config", "SolverAbstr", "CudaSolverRK",
            "SolverRK", "ModelAbstr", "BareParareal", "CudaNNGP", "NNGP_p", "CudaGP", "GPjax_p", "MyPool", "CudaPool",
-           "Parareal", "PararealLight", "PararealDevice"]
+           "Parareal", "PararealLight", "PararealDevice", "PararealEnsemble"]

@@ -64,6 +64,14 @@ SIGNATURES = {
     "nngp_counters": (ci, [vp, c_ll_p, c_ll_p, ci]),
     "nngp_profile_enable": (ci, [vp, ci]),
     "nngp_profile_read": (ci, [vp, vp, vp, ci]),
+    "nngp_seg_reserve": (ci, [vp, ci, cll, ci]),
+    "nngp_seg_reset": (ci, [vp]),
+    "nngp_seg_rows": (cll, [vp, ci]),
+    "nngp_seg_cap": (cll, [vp]),
+    "nngp_seg_append_iteration": (ci, [vp, ci, vp, vp, vp, vp, vp, cll, ci, ci, vp]),
+    "nngp_knn_segmented": (ci, [vp, vp, cll, ci, ci, vp, vp, vp, vp, vp, vp]),
+    "nngp_copy_rows": (ci, [vp, vp, vp, vp, vp, cll, cll, vp]),
+    "nngp_ensemble_sweep": (ci, [vp, ci, ci, ci, cll, vp, ci, ci, vp, vp, ci, ci, vp, cd, cd, vp, vp, ci, vp]),
 }
 
 SYSTEM_IDS = {"FHN_ODE": 0, "Rossler": 1, "Hopf": 2, "DblPend": 3, "Brusselator": 4, "Lorenz": 5,
@@ -287,6 +295,42 @@ class Handle:
 
     def rowwise_maxabs_diff(self, d_a, d_b, rows, d, d_err, stream=None):
         self.check(self.lib.nngp_rowwise_maxabs_diff(self.h, _ptr(d_a), _ptr(d_b), int(rows), int(d), _ptr(d_err), stream))
+
+    # -- segmented store and ensemble sweep (host int arrays are converted here)
+    def seg_reserve(self, n_members, cap_rows, d):
+        self.check(self.lib.nngp_seg_reserve(self.h, int(n_members), int(cap_rows), int(d)))
+
+    def seg_reset(self):
+        self.check(self.lib.nngp_seg_reset(self.h))
+
+    def seg_rows(self, member):
+        return int(self.lib.nngp_seg_rows(self.h, int(member)))
+
+    def seg_cap(self):
+        return int(self.lib.nngp_seg_cap(self.h))
+
+    def seg_append_iteration(self, members, I, d_u_cur, d_uF, d_uG_cur, ld_state, N, d, stream=None):
+        members, I = np.ascontiguousarray(members, dtype=np.int32), np.ascontiguousarray(I, dtype=np.int32)
+        self.check(self.lib.nngp_seg_append_iteration(self.h, members.size, _ptr(members), _ptr(I), _ptr(d_u_cur),
+                                                      _ptr(d_uF), _ptr(d_uG_cur), int(ld_state), int(N), int(d), stream))
+
+    def knn_segmented(self, d_q, ld_q, nq, m, base, rows, d_idx, d_dist, d_r2=None, stream=None):
+        base, rows = np.ascontiguousarray(base, dtype=np.int64), np.ascontiguousarray(rows, dtype=np.int64)
+        assert base.size == nq and rows.size == nq
+        self.check(self.lib.nngp_knn_segmented(self.h, _ptr(d_q), int(ld_q), int(nq), int(m), _ptr(base), _ptr(rows),
+                                               _ptr(d_idx), _ptr(d_dist), _ptr(d_r2), stream))
+
+    def copy_rows(self, d_src, d_src_idx, d_dst, d_dst_idx, rows, d, stream=None):
+        self.check(self.lib.nngp_copy_rows(self.h, _ptr(d_src), _ptr(d_src_idx), _ptr(d_dst), _ptr(d_dst_idx),
+                                           int(rows), int(d), stream))
+
+    def ensemble_sweep(self, sys, method_g, h_mode, steps_g, d_t, N, members, I, m, n_restarts, d_starts, fatol, xatol,
+                       d_u_next, d_uG_next, d, stream=None):
+        members, I = np.ascontiguousarray(members, dtype=np.int32), np.ascontiguousarray(I, dtype=np.int32)
+        self.check(self.lib.nngp_ensemble_sweep(self.h, sys, method_g, h_mode, int(steps_g), _ptr(d_t), int(N),
+                                                members.size, _ptr(members), _ptr(I), int(m), int(n_restarts),
+                                                _ptr(d_starts), float(fatol), float(xatol), _ptr(d_u_next),
+                                                _ptr(d_uG_next), int(d), stream))
 
     def selftest_math(self, d_x, n, d_exp, d_rcp, d_exp10=None, stream=None):
         self.check(self.lib.nngp_selftest_math(self.h, _ptr(d_x), int(n), _ptr(d_exp), _ptr(d_rcp),

@@ -2,6 +2,7 @@
 // host-buffer variants, the fused on-device sweep and the roofline micro-benchmarks.
 #include "common.cuh"
 
+#include <algorithm>
 #include <cstdarg>
 #include <cstdlib>
 #include <cstring>
@@ -143,6 +144,49 @@ struct Carver {
   static size_t pad(size_t bytes) { return ((bytes + 255) / 256) * 256; }
 };
 
+// Copies `bytes` of host data to the device buffer of upload slot `slot` on stream st (pinned staging; the staging is
+// overwritten only after the copy that last read it has completed).  nullptr on failure.
+static void* upload_table(nngp_handle_t h, int slot, const void* src, size_t bytes, cudaStream_t st) {
+  nngp_handle_s::Upload& u = h->up[slot];
+  if (u.done == nullptr && cudaEventCreateWithFlags(&u.done, cudaEventDisableTiming) != cudaSuccess) return nullptr;
+  if (u.host) cudaEventSynchronize(u.done);
+  if (bytes > u.bytes) {
+    cudaDeviceSynchronize();  // work already enqueued may still read the old device table
+    if (u.host) cudaFreeHost(u.host);
+    if (u.dev) cudaFree(u.dev);
+    u.host = u.dev = nullptr;
+    u.bytes = 0;
+    const size_t want = bytes + bytes / 2 + 256;
+    if (cudaMallocHost(&u.host, want) != cudaSuccess || cudaMalloc(&u.dev, want) != cudaSuccess) {
+      cudaGetLastError();
+      return nullptr;
+    }
+    u.bytes = want;
+  }
+  memcpy(u.host, src, bytes);
+  if (cudaMemcpyAsync(u.dev, u.host, bytes, cudaMemcpyHostToDevice, st) != cudaSuccess) return nullptr;
+  cudaEventRecord(u.done, st);
+  return u.dev;
+}
+
+// nq zeroed last-CTA counters for the segmented kNN (the kernel leaves them zero)
+static unsigned int* seg_tickets(nngp_handle_t h, int nq) {
+  if (nq > h->seg_tickets_n) {
+    cudaDeviceSynchronize();
+    if (h->seg_tickets) cudaFree(h->seg_tickets);
+    h->seg_tickets = nullptr;
+    h->seg_tickets_n = 0;
+    const int want = nq + 64;
+    if (cudaMalloc(&h->seg_tickets, sizeof(unsigned int) * want) != cudaSuccess ||
+        cudaMemset(h->seg_tickets, 0, sizeof(unsigned int) * want) != cudaSuccess) {
+      cudaGetLastError();
+      return nullptr;
+    }
+    h->seg_tickets_n = want;
+  }
+  return h->seg_tickets;
+}
+
 extern "C" {
 
 int nngp_abi_version(void) { return NNGP_ABI_VERSION; }
@@ -227,6 +271,12 @@ int nngp_destroy(nngp_handle_t h) {
   if (h->d_ticket) cudaFree(h->d_ticket);
   if (h->d_counters) cudaFree(h->d_counters);
   if (h->d_queues) cudaFree(h->d_queues);
+  if (h->seg_tickets) cudaFree(h->seg_tickets);
+  for (auto& u : h->up) {
+    if (u.host) cudaFreeHost(u.host);
+    if (u.dev) cudaFree(u.dev);
+    if (u.done) cudaEventDestroy(u.done);
+  }
   for (auto& r : h->prof_recs) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
   for (auto e : h->prof_free) cudaEventDestroy(e);
   delete h;
@@ -464,6 +514,7 @@ int nngp_dataset_reserve(nngp_handle_t h, long long cap_rows, int d) {
   double *ox = h->ds_x, *oy = h->ds_y, *oxt = h->ds_xt;
   h->ds_x = nx; h->ds_y = ny; h->ds_xt = nxt;
   h->ds_d = d; h->ds_cap = cap_rows; h->ds_rows = 0;
+  h->seg_E = 0;
   if (keep > 0) {
     if (int rc = dataset_append_launch(h, ox, oy, keep, nullptr)) return rc;
     NNGP_CUDA(h, cudaDeviceSynchronize());
@@ -814,6 +865,213 @@ int nngp_sweep_shard(nngp_handle_t h, int sys, int method_g, int h_mode, long lo
     if (int rc = gp_fit_predict_launch(h, idx, dist, fws, next_queue(h, st), order, 1, m, n_restarts, starts_i, fatol,
                                        xatol, un, gn, d, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, st, j0, dl))
       return rc;
+  }
+  return 0;
+}
+
+// ---- ensembles: segmented store, segmented kNN, ensemble sweep -------------------------
+int nngp_seg_reserve(nngp_handle_t h, int n_members, long long cap_rows, int d) {
+  NNGP_USE_DEVICE(h);
+  if (n_members < 1 || cap_rows < 1 || d < 1)
+    return nngp_fail(h, "seg_reserve: n_members=%d cap_rows=%lld d=%d", n_members, cap_rows, d);
+  const bool same = h->ds_x && h->seg_E == n_members && h->ds_d == d;
+  if (same && h->seg_cap >= cap_rows) return 0;
+  if (h->seg_E > 0 && !same)
+    for (long long r : h->seg_rows)
+      if (r > 0) return nngp_fail(h, "seg_reserve: layout change (%d members, d=%d) with rows held", n_members, d);
+  NNGP_CUDA(h, cudaDeviceSynchronize());
+  double *nx = nullptr, *ny = nullptr, *nxt = nullptr;
+  const size_t bytes = sizeof(double) * (size_t)n_members * (size_t)cap_rows * d;
+  NNGP_CUDA(h, cudaMalloc(&nx, bytes));
+  NNGP_CUDA(h, cudaMalloc(&ny, bytes));
+  NNGP_CUDA(h, cudaMalloc(&nxt, bytes));
+  double *ox = h->ds_x, *oy = h->ds_y, *oxt = h->ds_xt;
+  const long long ocap = h->seg_cap;
+  h->ds_x = nx; h->ds_y = ny; h->ds_xt = nxt;
+  h->ds_d = d; h->ds_cap = (long long)n_members * cap_rows; h->ds_rows = 0;
+  h->seg_E = n_members; h->seg_cap = cap_rows;
+  if (!same) h->seg_rows.assign(n_members, 0);
+  // growth: every member's rows move to the start of its new segment (X, Y and the transposed copy)
+  std::vector<long long> tab;
+  long long max_rows = 0;
+  for (int e = 0; same && e < n_members; e++) {
+    const long long r = h->seg_rows[e];
+    if (r == 0) continue;
+    tab.insert(tab.end(), {(long long)e * ocap * d, (long long)e * ocap * d, r, (long long)e * cap_rows});
+    max_rows = std::max(max_rows, r);
+  }
+  if (!tab.empty()) {
+    const long long* dtab = (const long long*)upload_table(h, 0, tab.data(), sizeof(long long) * tab.size(), nullptr);
+    if (!dtab) return nngp_fail(h, "seg_reserve: out of memory for the copy table");
+    if (int rc = append_seg_launch(h, ox, oy, nullptr, d, dtab, (int)(tab.size() / 4), max_rows, nullptr)) return rc;
+    NNGP_CUDA(h, cudaDeviceSynchronize());
+  }
+  if (ox) cudaFree(ox);
+  if (oy) cudaFree(oy);
+  if (oxt) cudaFree(oxt);
+  return 0;
+}
+
+int nngp_seg_reset(nngp_handle_t h) {
+  h->seg_rows.assign(h->seg_E, 0);
+  return 0;
+}
+
+long long nngp_seg_rows(nngp_handle_t h, int member) {
+  if (member < 0 || member >= h->seg_E) return -1;
+  return h->seg_rows[member];
+}
+
+long long nngp_seg_cap(nngp_handle_t h) { return h->seg_cap; }
+
+int nngp_seg_append_iteration(nngp_handle_t h, int n, const int* members, const int* I, const double* d_u_cur,
+                              const double* d_uF, const double* d_uG_cur, long long ld_state, int N, int d,
+                              void* stream) {
+  NNGP_USE_DEVICE(h);
+  if (n <= 0) return 0;
+  if (h->seg_E < 1) return nngp_fail(h, "seg_append_iteration: no segmented store (call nngp_seg_reserve)");
+  if (d != h->ds_d) return nngp_fail(h, "seg_append_iteration: d=%d but store d=%d", d, h->ds_d);
+  if (ld_state < (long long)(N + 1) * d) return nngp_fail(h, "seg_append_iteration: ld_state=%lld < (N+1) d", ld_state);
+  std::vector<long long> tab;
+  tab.reserve(4 * (size_t)n);
+  long long max_rows = 0;
+  for (int p = 0; p < n; p++) {
+    const int e = members[p];
+    if (e < 0 || e >= h->seg_E) return nngp_fail(h, "seg_append_iteration: member %d outside [0,%d)", e, h->seg_E);
+    if (I[p] < 1 || I[p] > N) return nngp_fail(h, "seg_append_iteration: I=%d outside [1,%d]", I[p], N);
+    const long long rows = (long long)N - I[p] + 1;
+    if (h->seg_rows[e] + rows > h->seg_cap)
+      return nngp_fail(h, "seg_append_iteration: member %d: %lld + %lld rows > capacity %lld", e, h->seg_rows[e], rows,
+                       h->seg_cap);
+    const long long so = (long long)p * ld_state;
+    tab.insert(tab.end(), {so + (long long)(I[p] - 1) * d, so + (long long)I[p] * d, rows,
+                           (long long)e * h->seg_cap + h->seg_rows[e]});
+    max_rows = std::max(max_rows, rows);
+  }
+  cudaStream_t st = as_stream(stream);
+  const long long* dtab = (const long long*)upload_table(h, 0, tab.data(), sizeof(long long) * tab.size(), st);
+  if (!dtab) return nngp_fail(h, "seg_append_iteration: out of memory for the row table");
+  if (int rc = append_seg_launch(h, d_u_cur, d_uF, d_uG_cur, d, dtab, n, max_rows, st)) return rc;
+  for (int p = 0; p < n; p++) h->seg_rows[members[p]] += (long long)N - I[p] + 1;
+  return 0;
+}
+
+int nngp_knn_segmented(nngp_handle_t h, const double* d_q, long long ld_q, int nq, int m, const long long* base,
+                       const long long* rows, long long* d_idx, double* d_dist, double* d_r2, void* stream) {
+  NNGP_USE_DEVICE(h);
+  if (nq <= 0) return 0;
+  if (!h->ds_x) return nngp_fail(h, "knn_segmented: no store");
+  if (ld_q < h->ds_d) return nngp_fail(h, "knn_segmented: ld_q=%lld < d=%d", ld_q, h->ds_d);
+  std::vector<long long> tab(2 * (size_t)nq);
+  long long n_max = 0;
+  for (int q = 0; q < nq; q++) {
+    if (rows[q] < m) return nngp_fail(h, "knn_segmented: query %d: segment of %lld rows, fewer than m=%d", q, rows[q], m);
+    if (base[q] < 0 || base[q] + rows[q] > h->ds_cap)
+      return nngp_fail(h, "knn_segmented: query %d: rows [%lld,%lld) outside the store (%lld)", q, base[q],
+                       base[q] + rows[q], h->ds_cap);
+    tab[q] = base[q];
+    tab[nq + q] = rows[q];
+    n_max = std::max(n_max, rows[q]);
+  }
+  cudaStream_t st = as_stream(stream);
+  void* ws = nngp_workspace(h, knn_seg_workspace_bytes(nq, n_max, m));
+  unsigned int* tickets = seg_tickets(h, nq);
+  if (!ws || !tickets) return nngp_fail(h, "knn_segmented: out of device memory");
+  const long long* dtab = (const long long*)upload_table(h, 1, tab.data(), sizeof(long long) * tab.size(), st);
+  if (!dtab) return nngp_fail(h, "knn_segmented: out of memory for the segment table");
+  return knn_seg_launch(h, d_q, ld_q, nq, m, dtab, dtab + nq, n_max, d_idx, d_dist, d_r2, tickets, ws, st);
+}
+
+int nngp_copy_rows(nngp_handle_t h, const double* d_src, const long long* d_src_idx, double* d_dst,
+                   const long long* d_dst_idx, long long rows, long long d, void* stream) {
+  NNGP_USE_DEVICE(h);
+  return copy_rows_launch(h, d_src, d_src_idx, d_dst, d_dst_idx, rows, d, as_stream(stream));
+}
+
+// t_rep[i, p] = t[i]: the per-slice time arrays of a launch over the members of one slice
+__global__ void repeat_t_kernel(const double* __restrict__ t, int n_t, int E, double* __restrict__ t_rep) {
+  const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e < (long long)n_t * E) t_rep[e] = t[e / E];
+}
+
+int nngp_ensemble_sweep(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g, const double* d_t, int N,
+                        int E, const int* members, const int* I, int m, int n_restarts, const signed char* d_starts,
+                        double fatol, double xatol, double* d_u_next, double* d_uG_next, int d, void* stream) {
+  NNGP_USE_DEVICE(h);
+  const SystemDesc* s;
+  if (int rc = get_sys(h, sys, &s)) return rc;
+  if (h->seg_E < 1) return nngp_fail(h, "ensemble_sweep: no segmented store (call nngp_seg_reserve)");
+  if (d != s->d || d != h->ds_d) return nngp_fail(h, "ensemble_sweep: d=%d, system d=%d, store d=%d", d, s->d, h->ds_d);
+  if (E < 1) return nngp_fail(h, "ensemble_sweep: E=%d < 1", E);
+  if (n_restarts < 1) return nngp_fail(h, "ensemble_sweep: n_restarts=%d < 1", n_restarts);
+  if (m < 1 || m > NNGP_MAX_NEIGHBOURS_BIG) return nngp_fail(h, "ensemble_sweep: m=%d outside [1,%d]", m, NNGP_MAX_NEIGHBOURS_BIG);
+  std::vector<long long> tab(2 * (size_t)E);
+  for (int p = 0; p < E; p++) {
+    const int e = members[p];
+    if (e < 0 || e >= h->seg_E) return nngp_fail(h, "ensemble_sweep: member %d outside [0,%d)", e, h->seg_E);
+    if (I[p] < 0 || I[p] > N || (p > 0 && I[p] < I[p - 1]))
+      return nngp_fail(h, "ensemble_sweep: I must be ascending in [0,%d] (position %d: %d)", N, p, I[p]);
+    if (I[p] < N && h->seg_rows[e] < m)
+      return nngp_fail(h, "ensemble_sweep: member %d holds %lld rows, fewer than m=%d", e, h->seg_rows[e], m);
+    tab[p] = (long long)e * h->seg_cap;
+    tab[E + p] = h->seg_rows[e];
+  }
+  if (I[0] >= N) return 0;
+  cudaStream_t st = as_stream(stream);
+  const long long ld = (long long)(N + 1) * d;
+  long long n_max_all = 0;
+  for (int p = 0; p < E; p++) n_max_all = std::max(n_max_all, tab[E + p]);
+  const int seg_len = d * NNGP_N_JITTER * n_restarts;
+  const size_t per_predict = (size_t)seg_len * 2;
+  const size_t bk = Carver::pad(knn_seg_workspace_bytes(E, n_max_all, m));
+  const size_t bf = Carver::pad(gp_fit_ws_bytes(E, d, m, n_restarts));
+  const size_t bi = Carver::pad(sizeof(long long) * (size_t)E * m), bd = Carver::pad(sizeof(double) * (size_t)E * m);
+  const size_t bo = Carver::pad(sizeof(int) * (size_t)E * seg_len);
+  const size_t bt = Carver::pad(sizeof(double) * (size_t)(N + 1) * E);
+  char* ws = (char*)nngp_workspace(h, bk + bf + bi + bd + bo + bt);
+  unsigned int* tickets = seg_tickets(h, E);
+  if (!ws || !tickets) return nngp_fail(h, "ensemble_sweep: out of device memory");
+  const long long* dtab = (const long long*)upload_table(h, 1, tab.data(), sizeof(long long) * tab.size(), st);
+  if (!dtab) return nngp_fail(h, "ensemble_sweep: out of memory for the segment table");
+  void* kws = ws;
+  void* fws = ws + bk;
+  long long* idx = (long long*)(ws + bk + bf);
+  double* dist = (double*)(ws + bk + bf + bi);
+  int* order = (int*)(ws + bk + bf + bi + bd);
+  double* t_rep = (double*)(ws + bk + bf + bi + bd + bo);
+  {
+    const long long tot = (long long)(N + 1) * E;
+    repeat_t_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(d_t, N + 1, E, t_rep);
+    h->launches++;
+    NNGP_CUDA(h, cudaGetLastError());
+  }
+  // The members active at slice i (I <= i) are a prefix of the positions: every launch below reaches them with the
+  // member stride (N+1) d of the state, and their predicts' starts are consecutive in d_starts (slice-major).
+  size_t done_predicts = 0;
+  int n_act = 0;
+  long long n_max = 0;
+  for (int i = I[0]; i < N; i++) {
+    while (n_act < E && I[n_act] <= i) n_max = std::max(n_max, tab[E + n_act++]);
+    const signed char* starts_i = d_starts + done_predicts * per_predict;
+    double* ui = d_u_next + (long long)i * d;
+    double* un = d_u_next + (long long)(i + 1) * d;
+    double* gn = d_uG_next + (long long)(i + 1) * d;
+    if (int rc = ensure_done_zero(h, fws, n_act, d, m, n_restarts, st)) return rc;
+    if (int rc = gp_order_launch(h, starts_i, n_act, seg_len, 1, order, st)) return rc;
+    // coarse step on the auxiliary stream beside the neighbour search (as in nngp_sweep)
+    NNGP_CUDA(h, cudaEventRecord(h->ev_fork, st));
+    NNGP_CUDA(h, cudaStreamWaitEvent(h->aux_stream, h->ev_fork, 0));
+    if (int rc = rk_launch(h, *s, method_g, h_mode, steps_g, n_act, t_rep + (size_t)i * E, t_rep + (size_t)(i + 1) * E,
+                           ui, ld, gn, ld, h->aux_stream))
+      return rc;
+    NNGP_CUDA(h, cudaEventRecord(h->ev_join, h->aux_stream));
+    if (int rc = knn_seg_launch(h, ui, ld, n_act, m, dtab, dtab + E, n_max, idx, dist, (double*)fws, tickets, kws, st))
+      return rc;
+    NNGP_CUDA(h, cudaStreamWaitEvent(st, h->ev_join, 0));
+    if (int rc = gp_fit_predict_launch(h, idx, dist, fws, next_queue(h, st), order, n_act, m, n_restarts, starts_i, fatol,
+                                       xatol, un, gn, ld, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, st))
+      return rc;
+    done_predicts += n_act;
   }
   return 0;
 }

@@ -79,6 +79,18 @@ struct nngp_handle_s {
   cudaStream_t queue_stream = nullptr;  // stream of the last fit that took a queue slot (next_queue)
   bool queue_stream_valid = false;
   bool attr_knn_tile = false;  // scan_select_tile_kernel's shared-memory attribute set on this device
+  bool attr_knn_tile_seg = false;
+  // segmented store (nngp_seg_reserve): seg_E members of seg_cap rows each in ds_x / ds_y / ds_xt (ds_cap = seg_E *
+  // seg_cap); seg_rows[e] rows held by member e.  0 members: the handle holds a plain dataset.
+  int seg_E = 0;
+  long long seg_cap = 0;
+  std::vector<long long> seg_rows;
+  unsigned int* seg_tickets = nullptr;  // one zeroed last-CTA counter per query of the segmented kNN
+  int seg_tickets_n = 0;
+  // small host->device tables of the segmented entry points: pinned staging, re-used once the copy that last read it
+  // has completed (event)
+  struct Upload { void* host = nullptr; void* dev = nullptr; size_t bytes = 0; cudaEvent_t done = nullptr; };
+  Upload up[2];
   // device counters: [0] Nelder-Mead runs, [1] objective (nll) evaluations
   unsigned long long* d_counters = nullptr;
   // task-queue heads of the persistent fit kernel: one zeroed counter per launch
@@ -136,6 +148,14 @@ int dataset_append_launch(nngp_handle_t h, const double* d_x, const double* d_y,
                           cudaStream_t st);
 int append_iteration_launch(nngp_handle_t h, const double* d_u_cur, const double* d_uF,
                             const double* d_uG_cur, int N, int I, int d, cudaStream_t st);
+size_t knn_seg_workspace_bytes(int nq, long long n_max, int m);
+int knn_seg_launch(nngp_handle_t h, const double* d_q, long long ld_q, int nq, int m, const long long* d_base,
+                   const long long* d_rows, long long n_max, long long* d_idx, double* d_dist, double* d_r2,
+                   unsigned int* tickets, void* ws, cudaStream_t st);
+int append_seg_launch(nngp_handle_t h, const double* xs, const double* ya, const double* yb, long long ld,
+                      const long long* d_tab, int nsrc, long long max_rows, cudaStream_t st);
+int copy_rows_launch(nngp_handle_t h, const double* src, const long long* si, double* dst, const long long* di,
+                     long long rows, long long d, cudaStream_t st);
 int rowwise_maxabs_launch(nngp_handle_t h, const double* a, const double* b, int rows, int d,
                           double* err, cudaStream_t st);
 

@@ -22,6 +22,7 @@
 // ranks the few keys below the m-th smallest list head instead of sorting.
 #include "common.cuh"
 
+#include <algorithm>
 #include <cfloat>
 #include <cstdlib>
 
@@ -814,6 +815,227 @@ scan_select_tile_kernel(const double* __restrict__ X, long long n, int d, const 
   }
 }
 
+// scan_select_tile_kernel for many queries, each over its own segment of rows (the kNN of an ensemble of runs that
+// share one store): query blockIdx.y searches the rows [base, base + n) of X and its candidate lists are read back from
+// the nl = ceil(n / SCAN_ROWS) first of the gridDim.x slots of the query; the CTAs past the end of a short segment only
+// take their ticket.  Indices are global (base + row).  The same operations in the same order as
+// scan_select_tile_kernel, so the same bits; a separate copy, because folding both into one template changed the
+// register allocation of the existing kernel.
+__device__ __forceinline__ void scan_select_tile_seg_body(const double* __restrict__ X, long long n, long long base, int d,
+                                                      const double* __restrict__ q, int m, int nl,
+                                                      double* __restrict__ cand_d, long long* __restrict__ cand_i,
+                                                      unsigned int* tickets, long long* __restrict__ idx_out,
+                                                      double* __restrict__ dist_out, double* __restrict__ r2) {
+  extern __shared__ double dyn[];  // [d] query | [TILE_ROWS][TILE_LD] tile
+  double* qs = dyn;
+  double* tile = dyn + ((d + 1) & ~1);
+  constexpr int NW = PRO_THREADS / 32;
+  static_assert(TILE_ROWS % NW == 0 && SCAN_ROWS % NW == 0 && SCAN_ROWS <= 32 && TILE_COLS == 8 * 32, "row / column mapping of the tile");
+  __shared__ bool last;
+  __shared__ int active[NNGP_MAX_NEIGHBOURS];
+  const double INF = __longlong_as_double(0x7ff0000000000000LL);
+  const long long IMAX = 0x7fffffffffffffffLL;
+  const int qi = blockIdx.y, tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+#pragma unroll 1
+  for (int e = tid; e < d; e += PRO_THREADS) qs[e] = q[e];
+  const long long lo = (long long)blockIdx.x * SCAN_ROWS;
+  const int rows = (int)min((long long)SCAN_ROWS, n - lo);
+  if (rows > 0) {
+  double acc = 0.0;
+  KNN_STAMP(0);
+  __syncthreads();
+#pragma unroll 1
+  for (int j0 = 0; j0 < d; j0 += TILE_COLS) {
+    const int jn = min(TILE_COLS, d - j0);
+    stage_rows<true, SCAN_ROWS / NW>(X, nullptr, base + lo, rows, d, j0, jn, qs, tile, wid, lane);
+    __syncthreads();
+    if (tid < rows) {
+      const double* tr = tile + tid * TILE_LD;
+#pragma unroll 32
+      for (int c = 0; c < jn; c++) acc = acc + tr[c];
+    }
+    __syncthreads();
+  }
+  KNN_STAMP(1);
+  // level 1: the CTA's rows sorted by (distance, index); the first m are its candidates
+  if (tid < 32) {
+    u64 kk = (lane < rows) ? ukey_of(acc) : UKEY_PAD;
+    long long ki = (lane < rows) ? base + lo + lane : IMAX;
+    warp_sort32_compact(kk, ki, lane);
+    if (lane < m) {
+      const long long cbase = ((long long)qi * gridDim.x + blockIdx.x) * m;
+      cand_i[cbase + lane] = ki;
+      reinterpret_cast<u64*>(cand_d)[cbase + lane] = kk;  // the integer key; level 2 converts back
+    }
+  }
+  }
+  KNN_STAMP(2);
+  __threadfence();
+  __syncthreads();
+  if (tid == 0) last = (atomicAdd(tickets + qi, 1u) == gridDim.x - 1);
+  __syncthreads();
+  KNN_STAMP(3);
+  if (!last) return;
+  __threadfence();
+  KNN_STAMP(4);
+  // level 2: the m smallest keys of the gridDim.x sorted candidate lists.  With at least m lists, T = the m-th smallest
+  // list head bounds the answer (m heads are <= T), every key <= T sits in one of the m lists whose heads are <= T
+  // ("active"), and the rank of such a key among the active lists is its rank among all candidates: each surviving
+  // key finds its output position by binary searches -- no sorting network, cost independent of the number of lists.
+  // With fewer than m lists all of them are active and nothing is bounded.
+  long long* io = idx_out + (long long)qi * m;
+  {
+    const u64* cdq = reinterpret_cast<const u64*>(cand_d) + (long long)qi * gridDim.x * m;
+    const long long* ciq = cand_i + (long long)qi * gridDim.x * m;
+    u64* hd = reinterpret_cast<u64*>(tile);                 // [nl] heads
+    long long* hi = reinterpret_cast<long long*>(tile + nl);
+    u64* ad = reinterpret_cast<u64*>(tile + 2 * nl);        // [na][m] active lists
+    long long* ai = reinterpret_cast<long long*>(tile + 2 * nl + NNGP_MAX_NEIGHBOURS * NNGP_MAX_NEIGHBOURS);
+#pragma unroll 1
+    for (int l = tid; l < nl; l += PRO_THREADS) {
+      hd[l] = __ldcg(cdq + (long long)l * m);
+      hi[l] = __ldcg(ciq + (long long)l * m);
+    }
+    __syncthreads();
+    KNN_STAMP(8);
+    const int na = min(nl, m);
+#pragma unroll 1
+    for (int l = tid; l < nl; l += PRO_THREADS) {
+      const u64 kk = hd[l];
+      const long long ki = hi[l];
+      int r = 0;
+#pragma unroll 4
+      for (int t = 0; t < nl; t++) r += ukey_less(hd[t], hi[t], kk, ki) ? 1 : 0;
+      if (r < na) active[r] = l;
+    }
+    __syncthreads();
+    KNN_STAMP(9);
+#pragma unroll 1
+    for (int e = tid; e < na * m; e += PRO_THREADS) {
+      const int a = e / m, pp = e - a * m;
+      ad[e] = __ldcg(cdq + (long long)active[a] * m + pp);
+      ai[e] = __ldcg(ciq + (long long)active[a] * m + pp);
+    }
+    __syncthreads();
+    KNN_STAMP(10);
+    const bool bounded = nl >= m;
+    const u64 tk = ad[(na - 1) * m];
+    const long long ti = ai[(na - 1) * m];
+    // surviving keys (not padding, not above the bound) are packed, then one thread per (survivor, active list) counts
+    // the list's keys below the survivor's (lower bound in a sorted list of m <= 32 entries) and adds it to the rank
+    int* surv = reinterpret_cast<int*>(tile + 2 * nl + 2 * NNGP_MAX_NEIGHBOURS * NNGP_MAX_NEIGHBOURS);
+    int* rankacc = surv + NNGP_MAX_NEIGHBOURS * NNGP_MAX_NEIGHBOURS;
+    __shared__ int n_surv;
+    if (tid == 0) n_surv = 0;
+    __syncthreads();
+#pragma unroll 1
+    for (int e = tid; e < na * m; e += PRO_THREADS) {
+      const u64 kk = ad[e];
+      const long long ki = ai[e];
+      if (ki == IMAX || (bounded && ukey_less(tk, ti, kk, ki))) continue;
+      const int pos = atomicAdd(&n_surv, 1);
+      surv[pos] = e;
+      rankacc[pos] = 0;
+    }
+    __syncthreads();
+    const int ns = n_surv;
+#pragma unroll 1
+    for (int t = tid; t < ns * na; t += PRO_THREADS) {
+      const int sidx = t / na, a = t - sidx * na;
+      const int e = surv[sidx];
+      const u64 kk = ad[e];
+      const long long ki = ai[e];
+      int base = 0, len = m;
+#pragma unroll 1
+      for (int step = 0; step < 6; step++) {
+        const int half = len >> 1;
+        const int at = a * m + min(base + half, m - 1);
+        const bool below = (len > 0) & ukey_less(ad[at], ai[at], kk, ki);
+        base = below ? base + half + 1 : base;
+        len = below ? len - half - 1 : half;
+      }
+      if (base) atomicAdd(&rankacc[sidx], base);
+    }
+    __syncthreads();
+#pragma unroll 1
+    for (int sidx = tid; sidx < ns; sidx += PRO_THREADS) {
+      const int rank = rankacc[sidx];
+      if (rank < m) {
+        const int e = surv[sidx];
+        io[rank] = ai[e];
+        dist_out[(long long)qi * m + rank] = ukey_to_double(ad[e]);
+      }
+    }
+  }
+  KNN_STAMP(11);
+  if (tid == 0) tickets[qi] = 0;  // ready for the next launch
+  if (r2 == nullptr) return;
+  __threadfence_block();
+  __syncthreads();  // idx_out written by this CTA
+  KNN_STAMP(5);
+  // neighbour matrix: pair (a, b), a >= b, per thread (m (m + 1) / 2 <= 528 pairs: up to three per thread)
+  double* r2q = r2 + (long long)qi * m * m;
+  const int npairs = m * (m + 1) / 2;
+  constexpr int PP = (NNGP_MAX_NEIGHBOURS * (NNGP_MAX_NEIGHBOURS + 1) / 2 + PRO_THREADS - 1) / PRO_THREADS;
+  int pa[PP], pb[PP];
+  double acc2[PP];
+#pragma unroll
+  for (int u = 0; u < PP; u++) {
+    const int pidx = tid + u * PRO_THREADS;
+    int a = 0, b = 0;
+    if (pidx < npairs) {
+      a = (int)((sqrtf(8.0f * (float)pidx + 1.0f) - 1.0f) * 0.5f);
+      while ((a + 1) * (a + 2) / 2 <= pidx) a++;
+      while (a * (a + 1) / 2 > pidx) a--;
+      b = pidx - a * (a + 1) / 2;
+    }
+    pa[u] = a;
+    pb[u] = b;
+    acc2[u] = 0.0;
+  }
+  KNN_STAMP(6);
+#pragma unroll 1
+  for (int j0 = 0; j0 < d; j0 += TILE_COLS) {
+    const int jn = min(TILE_COLS, d - j0);
+    __syncthreads();
+    stage_rows<false, TILE_ROWS / NW>(X, io, 0, m, d, j0, jn, nullptr, tile, wid, lane);
+    __syncthreads();
+#pragma unroll
+    for (int u = 0; u < PP; u++) {
+      if (tid + u * PRO_THREADS < npairs) {
+        const double *ta = tile + pa[u] * TILE_LD, *tb = tile + pb[u] * TILE_LD;
+        double sacc = acc2[u];
+#pragma unroll 16
+        for (int c = 0; c < jn; c++) {
+          const double diff = ta[c] - tb[c];
+          sacc = sacc + diff * diff;
+        }
+        acc2[u] = sacc;
+      }
+    }
+  }
+  KNN_STAMP(7);
+#pragma unroll
+  for (int u = 0; u < PP; u++) {
+    if (tid + u * PRO_THREADS < npairs) {
+      r2q[pa[u] * m + pb[u]] = acc2[u];
+      r2q[pb[u] * m + pa[u]] = acc2[u];
+    }
+  }
+}
+
+// query qi (row stride ld_q) searches rows [base[qi], base[qi] + rows[qi]); gridDim.x covers the longest segment
+__global__ void __launch_bounds__(PRO_THREADS)
+scan_select_tile_seg_kernel(const double* __restrict__ X, int d, const double* __restrict__ Q, long long ld_q,
+                            const long long* __restrict__ base, const long long* __restrict__ rows, int m,
+                            double* __restrict__ cand_d, long long* __restrict__ cand_i, unsigned int* tickets,
+                            long long* __restrict__ idx_out, double* __restrict__ dist_out, double* __restrict__ r2) {
+  const int qi = blockIdx.y;
+  const long long n = rows[qi];
+  scan_select_tile_seg_body(X, n, base[qi], d, Q + (long long)qi * ld_q, m, (int)((n + SCAN_ROWS - 1) / SCAN_ROWS),
+                              cand_d, cand_i, tickets, idx_out, dist_out, r2);
+}
+
 #ifdef NNGP_KNN_TIMING
 extern "C" void nngp_knn_stamps(long long* out) { cudaMemcpyFromSymbol(out, g_knn_stamps, sizeof(long long) * 16); }
 #endif
@@ -981,4 +1203,170 @@ int knn_prep_fused_launch(nngp_handle_t h, const double* d_q, int m, long long n
   (void)ticket;
   ProfScope prof(h, 1, st);
   return scan_select_launch(h, d_q, 1, m, n, d_idx, d_dist, d_r2, ws, st);
+}
+
+// ---------------------------------------------------------------------------------------
+// Segmented store (an ensemble of E runs in one handle): member e's rows live at [e cap, e cap + rows_e) of X, Y, XT
+// (cap_total = E cap), so every kernel that gathers rows by a global index (gp_prep_kernel, the fits) is unchanged.
+// ---------------------------------------------------------------------------------------
+
+// Rows of several sources, one per blockIdx.z, appended in one launch.  tab[z] = {x offset, y offset, rows, first
+// destination row}; offsets in doubles from xs / ya / yb, sources row-major with stride ld.  XT through a tile as in
+// append_kernel.
+__global__ void append_seg_kernel(const double* __restrict__ xs, const double* __restrict__ ya,
+                                  const double* __restrict__ yb, long long ld, const long long* __restrict__ tab, int d,
+                                  long long cap, double* __restrict__ X, double* __restrict__ Y,
+                                  double* __restrict__ XT) {
+  __shared__ double tile[32][33];
+  const long long* t = tab + 4 * (long long)blockIdx.z;
+  const long long xo = t[0], yo = t[1], rows = t[2], n0 = t[3];
+  const long long r0 = (long long)blockIdx.y * 32;
+  if (r0 >= rows) return;
+  const int j0 = blockIdx.x * 32;
+  for (int rr = threadIdx.y; rr < 32; rr += blockDim.y) {
+    const long long r = r0 + rr;
+    const int j = j0 + threadIdx.x;
+    if (r < rows && j < d) {
+      const double xv = xs[xo + r * ld + j];
+      X[(n0 + r) * d + j] = xv;
+      tile[rr][threadIdx.x] = xv;
+      double yv = ya[yo + r * ld + j];
+      if (yb != nullptr) yv = yv - yb[yo + r * ld + j];
+      Y[(n0 + r) * d + j] = yv;
+    }
+  }
+  __syncthreads();
+  for (int jj = threadIdx.y; jj < 32; jj += blockDim.y) {
+    const int j = j0 + jj;
+    const long long r = r0 + threadIdx.x;
+    if (r < rows && j < d) XT[(long long)j * cap + n0 + r] = tile[threadIdx.x][jj];
+  }
+}
+
+int append_seg_launch(nngp_handle_t h, const double* xs, const double* ya, const double* yb, long long ld,
+                      const long long* d_tab, int nsrc, long long max_rows, cudaStream_t st) {
+  if (nsrc <= 0 || max_rows <= 0) return 0;
+  const int d = h->ds_d;
+  ProfScope prof(h, 4, st);
+  dim3 block(32, 8);
+  dim3 grid((d + 31) / 32, (unsigned)((max_rows + 31) / 32), (unsigned)nsrc);
+  append_seg_kernel<<<grid, block, 0, st>>>(xs, ya, yb, ld, d_tab, d, h->ds_cap, h->ds_x, h->ds_y, h->ds_xt);
+  h->launches++;
+  NNGP_CUDA(h, cudaGetLastError());
+  return 0;
+}
+
+// dst[di[r]] = src[si[r]] for rows of d doubles (a null index list is the identity)
+__global__ void copy_rows_kernel(const double* __restrict__ src, const long long* __restrict__ si,
+                                 double* __restrict__ dst, const long long* __restrict__ di, long long rows, long long d) {
+  for (long long r = blockIdx.y; r < rows; r += gridDim.y) {
+    const double* s = src + (si ? si[r] : r) * d;
+    double* o = dst + (di ? di[r] : r) * d;
+    for (long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x; j < d; j += (long long)gridDim.x * blockDim.x)
+      o[j] = s[j];
+  }
+}
+
+int copy_rows_launch(nngp_handle_t h, const double* src, const long long* si, double* dst, const long long* di,
+                     long long rows, long long d, cudaStream_t st) {
+  if (rows <= 0 || d <= 0) return 0;
+  const unsigned gx = (unsigned)std::min<long long>((d + 255) / 256, 64);
+  copy_rows_kernel<<<dim3(gx, (unsigned)std::min<long long>(rows, 65535)), 256, 0, st>>>(src, si, dst, di, rows, d);
+  h->launches++;
+  NNGP_CUDA(h, cudaGetLastError());
+  return 0;
+}
+
+// Distances of query q (row stride ld_q) to the rows of its segment, written at dist[q, 0 .. rows[q]); the rest of the
+// row, up to n_max, is NaN.  select_kernel / select_big_kernel order keys by (isnan, distance, index), so a padding
+// entry sorts after every row of the segment, NaN distances included (its index is larger), and with m <= rows[q]
+// it is never selected.
+__global__ void __launch_bounds__(128)
+sqdist_seg_kernel(const double* __restrict__ XT, long long cap, int d, const double* __restrict__ Q, long long ld_q,
+                  const long long* __restrict__ base, const long long* __restrict__ rows, long long n_max,
+                  double* __restrict__ dist) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n_max) return;
+  const int qi = blockIdx.y;
+  double acc = __longlong_as_double(0x7ff8000000000000LL);
+  if (i < rows[qi]) {
+    const double* q = Q + (long long)qi * ld_q;
+    const double* xp = XT + base[qi] + i;
+    acc = 0.0;
+    for (int j = 0; j < d; j++) {
+      const double diff = __ldg(q + j) - xp[(long long)j * cap];
+      acc = acc + diff * diff;
+    }
+  }
+  dist[(long long)qi * n_max + i] = acc;
+}
+
+__global__ void add_base_kernel(long long* __restrict__ idx, const long long* __restrict__ base, int nq, int m) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e < nq * m) idx[e] += base[e / m];
+}
+
+// [distances nq*n_max | candidates]: both routes have at most ceil(n_max / SCAN_ROWS) candidate lists per query
+size_t knn_seg_workspace_bytes(int nq, long long n_max, int m) {
+  return knn_pad256(sizeof(double) * (size_t)nq * (size_t)n_max) +
+         2 * knn_pad256(sizeof(double) * (size_t)nq * (size_t)((n_max + SCAN_ROWS - 1) / SCAN_ROWS) * m);
+}
+
+bool knn_seg_tile_ok(nngp_handle_t h, long long n_max, int m) {
+  const size_t tile_smem = sizeof(double) * ((size_t)((h->ds_d + 1) & ~1) + (size_t)TILE_ROWS * TILE_LD);
+  return n_max <= KNN_TILE_MAX_ROWS && m <= NNGP_MAX_NEIGHBOURS && tile_smem <= 200 * 1024;
+}
+
+// kNN of nq queries, each in its own segment: d_base / d_rows device [nq], n_max = the largest rows[q] (host), every
+// rows[q] >= m.  Global indices ordered by (distance, index) and squared distances; r2 (optional, [nq, m, m]): the
+// neighbour matrix of gp_prep_kernel.  tickets: nq zeroed counters (left zero).
+int knn_seg_launch(nngp_handle_t h, const double* d_q, long long ld_q, int nq, int m, const long long* d_base,
+                   const long long* d_rows, long long n_max, long long* d_idx, double* d_dist, double* d_r2,
+                   unsigned int* tickets, void* ws, cudaStream_t st) {
+  if (nq <= 0) return 0;
+  if (m < 1 || m > NNGP_MAX_NEIGHBOURS_BIG) return nngp_fail(h, "knn_segmented: m=%d outside [1,%d]", m, NNGP_MAX_NEIGHBOURS_BIG);
+  const int d = h->ds_d;
+  ProfScope prof(h, 1, st);
+  if (knn_seg_tile_ok(h, n_max, m)) {
+    const unsigned tchunks = (unsigned)((n_max + SCAN_ROWS - 1) / SCAN_ROWS);
+    double* tcand_d = (double*)ws;
+    long long* tcand_i = (long long*)((char*)ws + knn_pad256(sizeof(double) * (size_t)nq * tchunks * m));
+    const size_t tile_smem = sizeof(double) * ((size_t)((d + 1) & ~1) + (size_t)TILE_ROWS * TILE_LD);
+    if (!h->attr_knn_tile_seg) {
+      NNGP_CUDA(h, cudaFuncSetAttribute(scan_select_tile_seg_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+      h->attr_knn_tile_seg = true;
+    }
+    scan_select_tile_seg_kernel<<<dim3(tchunks, nq), PRO_THREADS, tile_smem, st>>>(
+        h->ds_x, d, d_q, ld_q, d_base, d_rows, m, tcand_d, tcand_i, tickets, d_idx, d_dist, d_r2);
+    h->launches++;
+    NNGP_CUDA(h, cudaGetLastError());
+    return 0;
+  }
+  double* dist = (double*)ws;
+  sqdist_seg_kernel<<<dim3((unsigned)((n_max + 127) / 128), nq), 128, 0, st>>>(h->ds_xt, h->ds_cap, d, d_q, ld_q, d_base,
+                                                                             d_rows, n_max, dist);
+  h->launches++;
+  NNGP_CUDA(h, cudaGetLastError());
+  const long long chunk_rows = knn_chunk_rows(nq, n_max);
+  const long long chunks = (n_max + chunk_rows - 1) / chunk_rows;
+  if (m > NNGP_MAX_NEIGHBOURS) {
+    select_big_kernel<<<nq, 256, 0, st>>>(dist, n_max, m, d_idx, d_dist);
+    h->launches++;
+  } else if (chunks == 1) {
+    select_kernel<<<dim3(1, nq), KNN_SEL_THREADS, 0, st>>>(dist, nullptr, n_max, n_max, m, d_idx, d_dist);
+    h->launches++;
+  } else {
+    char* cb = (char*)ws + knn_pad256(sizeof(double) * (size_t)nq * (size_t)n_max);
+    double* cand_d = (double*)cb;
+    long long* cand_i = (long long*)(cb + knn_pad256(sizeof(double) * (size_t)nq * chunks * m));
+    select_kernel<<<dim3((unsigned)chunks, nq), KNN_SEL_THREADS, 0, st>>>(dist, nullptr, n_max, chunk_rows, m, cand_i, cand_d);
+    const long long nc = chunks * m;
+    select_kernel<<<dim3(1, nq), KNN_SEL_THREADS, 0, st>>>(cand_d, cand_i, nc, nc, m, d_idx, d_dist);
+    h->launches += 2;
+  }
+  add_base_kernel<<<(nq * m + 255) / 256, 256, 0, st>>>(d_idx, d_base, nq, m);
+  h->launches++;
+  NNGP_CUDA(h, cudaGetLastError());
+  if (d_r2 != nullptr) return gp_prep_launch(h, d_idx, nq, m, d_r2, st);
+  return 0;
 }

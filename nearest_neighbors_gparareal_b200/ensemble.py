@@ -1,0 +1,272 @@
+"""Many independent nnGParareal runs as one device-resident ensemble.
+
+`PararealEnsemble.run(seeds=[...])` runs E solves of the same system, solver, tspan, N, `nn`, `n_restarts`,
+`fatol` and `xatol` in lockstep; the runs may differ in seed, initial condition, epsilon and early_stop.  Every
+iteration makes the launches of one `PararealDevice` iteration, each over all runs at once: one fine-step launch, one
+dataset append, and per slice of the sweep one coarse step, one kNN (each run searches its own rows of a segmented
+store, csrc/knn.cu) and one fit over all the runs' predicts.  Run e's output dict equals, bit for bit, what
+`PararealDevice(...).run(model='nngp', seed=seeds[e], ...)` returns with its settings.
+
+Layout: the state is [E, N+1, d] per array.  At the start of every iteration the member axis is re-ordered by
+(finished, I), so the runs still going are a prefix, sorted by their first unconverged slice: at slice i of the sweep
+the runs with I <= i are a prefix too, and every launch of the sweep reaches them with the member stride (N+1) d --
+no gather or scatter per slice.  Only the fine step, whose slices I_e..N-1 differ per run, gathers its rows into one
+batch (nngp_copy_rows) once per iteration.
+"""
+import time
+
+import numpy as np
+
+from . import _lib
+from .models import CudaNNGP, N_JITTER
+from .solver import CudaSolverRK
+from .systems import ODE
+
+MAX_NEIGHBOURS = 160  # include/nngpara.h: NNGP_MAX_NEIGHBOURS_BIG
+
+
+def check_run_args(E_lists, model='nngp', store_int=False, nn='adaptive'):
+    """Validates the per-member lists of `PararealEnsemble.run` (dict name -> list or None); returns E."""
+    if not isinstance(model, str) or model.lower() != 'nngp':
+        raise ValueError(f"PararealEnsemble runs the 'nngp' model only (got {model!r})")
+    if store_int:
+        raise ValueError('PararealEnsemble does not write intermediate checkpoints (store_int=True)')
+    seeds = E_lists.get('seeds')
+    if seeds is None or len(seeds) == 0:
+        raise ValueError('PararealEnsemble.run needs a non-empty list of seeds')
+    E = len(seeds)
+    for name, v in E_lists.items():
+        if v is not None and len(v) != E:
+            raise ValueError(f'{name} has {len(v)} entries, seeds has {E}: give one per member')
+    if nn != 'adaptive' and not (1 <= int(nn) <= MAX_NEIGHBOURS):
+        raise ValueError(f'nn={nn}: 1 to {MAX_NEIGHBOURS} neighbours are supported')
+    return E
+
+
+def member_order(I, done):
+    """Members in state order for the next iteration: running ones first, by ascending I (stable)."""
+    I = np.asarray(I)
+    return np.lexsort((np.arange(I.size), I, np.asarray(done, dtype=bool)))
+
+
+def fine_rows(I_pos, N):
+    """(flat state row, slice) of every fine solve of the runs at positions 0..len(I_pos)-1: slices I_p..N-1 of each"""
+    rows, sl = [], []
+    for p, I in enumerate(I_pos):
+        s = np.arange(I, N)
+        rows.append(p * (N + 1) + s)
+        sl.append(s)
+    if not rows:
+        return np.zeros(0, np.int64), np.zeros(0, np.int64)
+    return np.concatenate(rows).astype(np.int64), np.concatenate(sl).astype(np.int64)
+
+
+def pack_starts(blocks, I_pos, N):
+    """The starts of the sweep in the order nngp_ensemble_sweep reads them: slice-major, and within slice i the blocks of
+    the positions with I_p <= i in position order.  blocks[p] = [N - I_p, d, 9, R, 2], the run's solo draw for this
+    sweep (its block j belongs to slice I_p + j).  I_pos ascending."""
+    out = []
+    for i in range(min(I_pos), N):
+        for p, I in enumerate(I_pos):
+            if I > i:
+                break
+            out.append(blocks[p][i - I])
+    return np.ascontiguousarray(np.stack(out))
+
+
+def advance(err_k, I, eps):
+    """parareal.py:402-416 for one run: err_k[I] = 0, then I moves over the slices whose error is below eps"""
+    err_k[I] = 0
+    N = err_k.shape[0] - 1
+    for p in range(I + 1, N + 1):
+        if err_k[p] < eps:
+            I += 1
+        else:
+            break
+    return I
+
+
+class PararealEnsemble:
+    """E independent device-resident nnGParareal runs in lockstep (see the module docstring).
+
+    The ensemble owns its own library handle, so its segmented dataset never meets the dataset of a solo run on the
+    default handle.  Per-member timings are the ensemble's shared wall times: F_time, G_time and sweep_time of every
+    member are the times of the launches that served all members together.
+    """
+
+    def __init__(self, ode, solver, tspan, N, epsilon=5e-7, verbose='v', device=None):
+        if not isinstance(ode, ODE):
+            raise Exception('ode must be an instance of the ODE class, see systems.py file.')
+        if not isinstance(solver, CudaSolverRK):
+            raise Exception('PararealEnsemble needs a CudaSolverRK')
+        self.ode, self.solver, self.tspan, self.N = ode, solver, tspan, N
+        self.epsilon = epsilon
+        self.verbose = verbose
+        self.n = ode.get_dim()
+        self.u0 = ode.get_init_cond()
+        self._device = device
+        self._h = None
+
+    def handle(self):
+        if self._h is None:
+            import os
+            dev = self._device if self._device is not None else int(os.environ.get("LOCAL_RANK", "0"))
+            self._h = _lib.Handle(dev)
+        return self._h
+
+    def run(self, model='nngp', seeds=None, nn='adaptive', n_restarts=1, fatol=None, xatol=None, epsilons=None,
+            early_stops=None, init_conds=None, max_rows=None, store_int=False):
+        """Returns one output dict per seed (the keys of PararealDevice.run, n_rows included)."""
+        E = check_run_args(dict(seeds=seeds, epsilons=epsilons, early_stops=early_stops, init_conds=init_conds),
+                           model=model, store_int=store_int, nn=nn)
+        solver = self.solver
+        if max(solver.Nf, solver.Ng) > solver.thresh:
+            raise Exception('steps > thresh (RK paging, solver.py:89-96) is only supported by the host driver')
+        eps = [self.epsilon if epsilons is None or epsilons[e] is None else epsilons[e] for e in range(E)]
+        stops = [None if early_stops is None else early_stops[e] for e in range(E)]
+        u0s = np.stack([self.u0 if init_conds is None or init_conds[e] is None else self.ode.get_init_cond(u0=init_conds[e])
+                        for e in range(E)])
+        h = self.handle()
+        models = [CudaNNGP(n=self.n, N=self.N, seed=s, nn=nn, n_restarts=n_restarts, fatol=fatol, xatol=xatol,
+                           handle=h) for s in seeds]
+        return self._run(h, models, eps, stops, u0s, max_rows)
+
+    def _run(self, h, models, eps, stops, u0s, max_rows):
+        import torch
+        N, n, solver = self.N, self.n, self.solver
+        E = len(models)
+        verbose = self.verbose
+        _, sysid = self.ode.device_system(h)
+        dev = torch.device('cuda', h.device)
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        mF, mG, hm = _lib.METHODS[solver.F], _lib.METHODS[solver.G], solver.h_mode
+        f64 = dict(dtype=torch.float64, device=dev)
+        ld = (N + 1) * n
+        tic = time.time()
+        t_host = np.linspace(self.tspan[0], self.tspan[1], num=N + 1)
+        t = torch.from_numpy(t_host).to(dev)
+        t_rep = t.repeat_interleave(E)  # t_rep[i E + p] = t_i
+        st = {key: torch.zeros((E, N + 1, n), **f64) for key in ('u_cur', 'uG_cur', 'uF')}
+        for a in st.values():
+            a[:, 0] = torch.from_numpy(u0s).to(dev)
+        for i in range(N):  # coarse initialisation: N dependent launches over all members
+            h.rk_batch(sysid, mG, hm, solver.Ng, E, t_rep[i * E:], t_rep[(i + 1) * E:], st['uG_cur'][:, i], ld,
+                       st['uG_cur'][:, i + 1], ld, stream)
+        st['u_cur'].copy_(st['uG_cur'])
+        st['u_next'] = st['u_cur'].clone()
+        st['uG_next'] = st['uG_cur'].clone()
+        scratch = torch.empty_like(st['u_cur'])
+        err_dev = torch.zeros(E * (N + 1), **f64)
+        cap = max_rows or min(N * (N + 3) // 2 + 1, N * 16)
+        h.seg_reset()
+        h.seg_reserve(E, cap, n)
+        cap = h.seg_cap()
+        torch.cuda.synchronize(dev)
+        G_time = time.time() - tic
+        F_time = sweep_time = 0.0
+
+        I = np.zeros(E, dtype=np.int64)
+        done = np.zeros(E, dtype=bool)
+        rows = np.zeros(E, dtype=np.int64)
+        last_k = np.zeros(E, dtype=np.int64)
+        conv_int = [[] for _ in range(E)]
+        err = [np.full((N + 1, N), np.nan) for _ in range(E)]
+        pos = np.arange(E)  # pos[p] = member at state position p
+        for k in range(N):
+            # state order: running members first, by ascending I
+            order = member_order(I[pos], done[pos])
+            if not np.array_equal(order, np.arange(E)):
+                perm = torch.from_numpy(order.astype(np.int64)).to(dev)
+                for key in ('u_cur', 'uG_cur', 'uF', 'u_next', 'uG_next'):
+                    h.copy_rows(st[key], perm, scratch, None, E, ld, stream)
+                    st[key], scratch = scratch, st[key]
+                pos = pos[order]
+            n_live = int(np.count_nonzero(~done[pos]))
+            if n_live == 0:
+                break
+            live = pos[:n_live]
+            if verbose == 'v':
+                print(f'{self.ode.name} ensemble of {E} iteration number (out of {N}): {k+1}, {n_live} running')
+            tic = time.time()
+            # fine solves of every running member's unconverged slices in one launch (parareal.py:309-334)
+            fr, fs = fine_rows(I[live], N)
+            idx = torch.from_numpy(np.concatenate([fr, fr + 1, np.arange(n_live) * (N + 1) + I[live] + 1])).to(dev)
+            tt = torch.from_numpy(np.concatenate([t_host[fs], t_host[fs + 1]])).to(dev)
+            nf = fr.size
+            buf = torch.empty((2, nf, n), **f64)
+            h.copy_rows(st['u_cur'], idx[:nf], buf[0], None, nf, n, stream)
+            h.rk_batch(sysid, mF, hm, solver.Nf, nf, tt[:nf], tt[nf:], buf[0], n, buf[1], n, stream)
+            h.copy_rows(buf[1], None, st['uF'], idx[nf:2 * nf], nf, n, stream)
+            exact = idx[2 * nf:]
+            h.copy_rows(st['uF'], exact, st['u_next'], exact, n_live, n, stream)
+            h.copy_rows(st['uG_cur'], exact, st['uG_next'], exact, n_live, n, stream)
+            torch.cuda.synchronize(dev)
+            F_time += time.time() - tic
+            I[live] += 1
+            tic = time.time()
+            # dataset append of every running member, before the early-stop check as in PararealDevice.device_sweep
+            need = rows[live] + (N - I[live] + 1)
+            if need.max() > cap:
+                while need.max() > cap:
+                    cap = 2 * cap + N
+                h.seg_reserve(E, cap, n)
+            h.seg_append_iteration(live, I[live], st['u_cur'], st['uF'], st['uG_cur'], ld, N, n, stream)
+            rows[live] = need
+            n_sweep = int(np.count_nonzero(I[live] < N))  # the members with I == N sort last among the running ones
+            if n_sweep > 0:
+                sw = live[:n_sweep]
+                mdl0 = models[sw[0]]
+                m = mdl0.neighbours(k)
+                if m > MAX_NEIGHBOURS:
+                    raise Exception('nn > 160 neighbours is not supported (include/nngpara.h: NNGP_MAX_NEIGHBOURS_BIG)')
+                short = [e for e in sw if rows[e] < m]
+                if short:
+                    raise Exception(f'members {short} hold fewer dataset rows ({rows[short].min()}) than the common m={m}: '
+                                    'an ensemble needs one m per launch')
+                blocks = []
+                for e in sw:
+                    mdl = models[e]
+                    mdl.k = mdl.time_k = k
+                    blocks.append(mdl.draw_starts(N - I[e]))
+                    mdl.train_count += (N - I[e]) * n * N_JITTER * mdl.n_restarts
+                starts = torch.from_numpy(pack_starts(blocks, I[sw], N)).to(dev)
+                h.ensemble_sweep(sysid, mG, hm, solver.Ng, t, N, sw, I[sw], m, mdl0.n_restarts, starts, mdl0.fatol,
+                                 mdl0.xatol, st['u_next'], st['uG_next'], n, stream)
+            # parareal.py:402: one error launch over the running members and ONE device->host read
+            h.rowwise_maxabs_diff(st['u_next'], st['u_cur'], n_live * (N + 1), n, err_dev, stream)
+            errs = err_dev[:n_live * (N + 1)].cpu().numpy().reshape(n_live, N + 1)
+            dt_sweep = time.time() - tic
+            sweep_time += dt_sweep
+            for p, e in enumerate(live):
+                err[e][:, k] = errs[p]
+                last_k[e] = k
+                if I[e] == N:  # early stopping (parareal.py:341-347)
+                    err[e][-1, k] = np.nextafter(eps[e], 0)
+                    done[e] = True
+                    continue
+                mdl = models[e]
+                mdl.pred_time += dt_sweep
+                mdl.pred_times[k] += dt_sweep
+                mdl.tot_train_t += dt_sweep
+                if np.any(np.isnan(err[e][:, k])) and bool(torch.isnan(st['uG_next'][p]).any()):
+                    raise Exception("NaN values in initial coarse solve - increase Ng!")
+                I[e] = advance(err[e][:, k], I[e], eps[e])
+                conv_int[e].append(int(I[e]))
+                if I[e] == N or (stops[e] is not None and k == stops[e] - 1):
+                    done[e] = True
+            st['u_cur'].copy_(st['u_next'])
+            st['uG_cur'].copy_(st['uG_next'])
+        u_all = st['u_cur'].cpu().numpy()
+        where = np.empty(E, dtype=np.int64)
+        where[pos] = np.arange(E)
+        outs = []
+        for e in range(E):
+            timings = {'F_time': F_time, 'G_time': G_time, 'F_time_serial_avg': F_time / max(N, 1),
+                       'sweep_time': sweep_time}
+            timings.update(models[e].get_times())
+            u = u_all[where[e]].copy()
+            kk = int(last_k[e])
+            outs.append({'t': t_host, 'u': u, 'u_last': u, 'err': err[e][:, :kk + 1], 'k': kk + 1, 'timings': timings,
+                         'debug_dict': {}, 'converged': bool(I[e] == N), 'conv_int': conv_int[e],
+                         'n_rows': int(h.seg_rows(e))})
+        return outs

@@ -556,11 +556,20 @@ rk_fhn_tile_kernel(SysArgs A, int h_mode, long long steps, int n_slices, long lo
   const int oup = ((iy0 == 0 ? dx : iy0) - 1) * dx + ix0;        // row iy0-1, columns ix0, ix0+1
   const int odn = ((iy0 + TY == dx) ? 0 : iy0 + TY) * dx + ix0;  // row iy0+TY
   const int xl = (ix0 == 0 ? dx : ix0) - 1, xr = (ix0 + 2 == dx) ? 0 : ix0 + 2;
-  const int ol0 = iy0 * dx + xl, or0 = iy0 * dx + xr;
+  // Column loads: a left neighbour sits in an odd column, a right one in an even column, and a 128-byte line holds
+  // 16 doubles, so if every thread fetched its left (or right) neighbour in the same instruction, the 16 threads of a
+  // half-warp would share 8 eight-byte bank pairs: 2 wavefronts per 64-bit load instead of 1 (16 of the 64 shared-memory
+  // wavefronts per warp and stage at d_x = 16, profiles/r01/rk_tile_r1.summary.csv).  Instead, threads with flip set
+  // fetch the right neighbour first.  flip alternates between the block rows of a half-warp at d_x = 16 (and between
+  // the two halves of a row at d_x = 32), so each half-warp reads 8 odd and 8 even columns: conflict-free, 48 wavefronts
+  // (scripts/rk_shared_wavefronts.py).  The two loaded values trade places in registers: 16 FSEL per thread and stage,
+  // 222 registers for <11, 2, 64>.  Same values, same arithmetic: the same bits.  (A swizzled buffer -- the pairs of
+  // alternate block rows stored swapped -- is conflict-free too, but has to undo the swap for the own and the upper and
+  // lower pairs: 32 FSEL per stage and 226 registers with 128-bit accesses, or 239 registers with 64-bit ones.)
+  const bool flip = (((iy0 / TY) ^ (ix0 >> 4)) & 1) != 0;
+  const int oc0 = iy0 * dx + (flip ? xr : xl), oc1 = iy0 * dx + (flip ? xl : xr);
   // shx: the left / right neighbour columns come from the neighbouring lanes of the same block row by shuffle instead
-  // of shared memory (the threads of a block row are hx consecutive lanes; hx a power of two <= 32).  The column loads
-  // they replace touch only every other 8-byte bank pair and alias across the four block rows of a warp: 16 of the 64
-  // shared-memory wavefronts per warp and stage were bank conflicts (profiles/r01/rk_tile_r1.summary.csv).
+  // of shared memory (the threads of a block row are hx consecutive lanes; hx a power of two <= 32).
   const int lane = threadIdx.x & 31;
   const int lsrc = (lane & ~(hx - 1)) | ((lane - 1) & (hx - 1)), rsrc = (lane & ~(hx - 1)) | ((lane + 1) & (hx - 1));
   double u[2][NV], k[2][NV][S];
@@ -637,8 +646,9 @@ rk_fhn_tile_kernel(SysArgs A, int h_mode, long long steps, int n_slices, long lo
         if (!SHX) {
 #pragma unroll
           for (int r = 0; r < TY; r++) {
-            lf[c][r] = b[ol0 + r * dx];
-            rt[c][r] = b[or0 + r * dx];
+            const double c0 = b[oc0 + r * dx], c1 = b[oc1 + r * dx];
+            lf[c][r] = flip ? c1 : c0;
+            rt[c][r] = flip ? c0 : c1;
           }
         }
       }
@@ -698,14 +708,15 @@ rk_fhn_tile_kernel(SysArgs A, int h_mode, long long steps, int n_slices, long lo
   }
 }
 
-// Time-chunked launch.  Measured (profiles/r01/rk_sweep.log): an SM reaches its full fine-step throughput
-// with TWO resident slices (one warp per sub-partition, each saturating its FP64 issue); 3 slices per SM are
-// slower than 2 (two sub-partitions hold two warps), 4 gain nothing, and 512 slices on 148 SMs leave 80 SMs
-// a slice short.  So when a GPU holds more than 2 slices per SM the step range is cut into chunks and the
-// (chunk, slice) tasks are executed chunk-major by a sequence of launches of exactly 2 CTAs per SM (forced by
-// the shared-memory request): every launch is perfectly balanced, a slice's state passes from chunk to chunk
-// through u1, and task (c, s) always falls into a later launch than (c-1, s) because a launch is smaller than
-// the number of slices.  Results are bit-identical to the single launch.
+// Time-chunked launch.  Measured (profiles/r01/rk_sweep.log; again with conflict-free column loads,
+// profiles/r04/rk_layout_sweep.log): an SM reaches nearly its full fine-step throughput with TWO resident slices (one
+// warp per sub-partition); 3 slices per SM are slower than 2 (two sub-partitions hold two warps: 3 per SM chunked,
+// 512 slices, 625 ms against 507), 4 gain 4 % per slice (one launch of 592 slices: 560 ms against 2 x 291), and 512
+// slices in one launch leave 80 SMs a slice short (560 ms).  So when a GPU holds more than 2 slices per SM the step
+// range is cut into chunks and the (chunk, slice) tasks are executed chunk-major by a sequence of launches of
+// exactly 2 CTAs per SM (forced by the shared-memory request): every launch is perfectly balanced, a slice's state
+// passes from chunk to chunk through u1, and task (c, s) always falls into a later launch than (c-1, s) because a
+// launch is smaller than the number of slices.  Results are bit-identical to the single launch.
 template <int S, int TY, int TB, bool SHX>
 static int launch_fhn_tile_x(const SysArgs& A, int npts, int h_mode, long long steps, int n, int sms,
                              const double* t0, const double* t1, const double* u0, long long ld0, double* u1,
@@ -753,6 +764,8 @@ static int launch_fhn_tile_s(const SysArgs& A, int npts, int h_mode, long long s
   // (2x2 blocks) to 11 % (1x2) faster -- the shuffles leave before the barrier and shorten the per-stage dependency chain --
   // while with several slices per SM the 16 shuffles per thread and stage cost more shared-pipe cycles than the 8 column
   // loads they replace (512 slices on one GPU: 627 vs 562 ms).  So: shuffle only when the GPU holds at most one slice per SM.
+  // Re-measured with conflict-free column loads (profiles/r04/rk_layout_sweep.log, 64 and 148 slices): the shuffle form
+  // still wins, 1x2 257.0 against 268.7 ms, 2x2 278.0 against 288.8 ms.
   const bool shx = getenv("NNGP_RK_NO_SHFL") == nullptr && hx_ >= 1 && hx_ <= 32 && (hx_ & (hx_ - 1)) == 0 &&
                    (npts / (2 * TY)) % 32 == 0 && n <= sms;
   if (shx) return launch_fhn_tile_x<S, TY, TB, true>(A, npts, h_mode, steps, n, sms, t0, t1, u0, ld0, u1, ld1, st);

@@ -210,7 +210,6 @@ int nngp_create(int device, nngp_handle_t* out) {
   h->device = device;
   h->sm_count = prop.multiProcessorCount;
   if (const char* fm = getenv("NNGP_FIT_MODE")) h->fit_mode = (strcmp(fm, "warp") == 0) ? 1 : (strcmp(fm, "grouped") == 0) ? 2 : (strcmp(fm, "quad") == 0) ? 3 : 0;
-  if (getenv("NNGP_FIT_LEGACY")) h->fit_mode = 1;
   if (const char* b = getenv("NNGP_FIT_BUDGET")) h->fit_budget = atoi(b);
   if (cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking) != cudaSuccess) {
     delete h;
@@ -762,21 +761,17 @@ int nngp_predict_host_block(nngp_handle_t h, const double* q, int nq, int m, lon
 static int sweep_slice_prologue(nngp_handle_t h, const SystemDesc& s, int method_g, int h_mode, long long steps_g,
                                 const double* d_ti, double* ui, double* gn, int d, int m, long long n, long long* idx,
                                 double* dist, void* kws, void* fws, cudaStream_t st) {
-  const bool fork = getenv("NNGP_SWEEP_NO_FORK") == nullptr;
-  cudaStream_t sg = fork ? h->aux_stream : st;
-  if (fork) {
-    NNGP_CUDA(h, cudaEventRecord(h->ev_fork, st));
-    NNGP_CUDA(h, cudaStreamWaitEvent(sg, h->ev_fork, 0));
-  }
-  if (int rc = rk_launch(h, s, method_g, h_mode, steps_g, 1, d_ti, d_ti + 1, ui, d, gn, d, sg)) return rc;
-  if (fork) NNGP_CUDA(h, cudaEventRecord(h->ev_join, sg));
-  if (knn_prep_fused_ok(h, n, m) && getenv("NNGP_SWEEP_NO_FUSED_PROLOGUE") == nullptr) {
+  NNGP_CUDA(h, cudaEventRecord(h->ev_fork, st));
+  NNGP_CUDA(h, cudaStreamWaitEvent(h->aux_stream, h->ev_fork, 0));
+  if (int rc = rk_launch(h, s, method_g, h_mode, steps_g, 1, d_ti, d_ti + 1, ui, d, gn, d, h->aux_stream)) return rc;
+  NNGP_CUDA(h, cudaEventRecord(h->ev_join, h->aux_stream));
+  if (knn_prep_fused_ok(h, n, m)) {
     if (int rc = knn_prep_fused_launch(h, ui, m, n, idx, dist, (double*)fws, kws, h->d_ticket, st)) return rc;
   } else {
     if (int rc = knn_launch(h, ui, 1, m, n, idx, dist, kws, st)) return rc;
     if (int rc = gp_prep_launch(h, idx, 1, m, (double*)fws, st)) return rc;
   }
-  if (fork) NNGP_CUDA(h, cudaStreamWaitEvent(st, h->ev_join, 0));
+  NNGP_CUDA(h, cudaStreamWaitEvent(st, h->ev_join, 0));
   return 0;
 }
 

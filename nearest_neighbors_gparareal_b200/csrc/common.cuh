@@ -72,9 +72,11 @@ struct nngp_handle_s {
   // evaluations after which a search is handed to the four-warp continuation kernel (0: never, the default: measured
   // slower than the sequential search at 1 and at 8 GPUs, profiles/r02/fit_kernel_variants.log); NNGP_FIT_BUDGET
   int fit_budget = 0;
-  // which search kernel a fit launches: 0 auto (several searches per warp for batched queries with m <= 20, where it
-  // is 1.4-4x faster; one search per warp for the serial sweep, whose searches fail early and cheaply 45 % of the
-  // time -- DESIGN.md section 4.5), 1 always one search per warp, 2 always grouped.  NNGP_FIT_MODE=auto|warp|grouped
+  // which search kernel a fit launches: 0 auto (several searches per warp for batched queries, nq >= 4 and m <= 20,
+  // where it is 1.4-4x faster; otherwise one search per warp, as in the serial sweep, whose searches fail early and
+  // cheaply 45 % of the time -- DESIGN.md section 4.5 -- or four warps per search when such a launch has at most 3
+  // searches per resident CTA), 1 always one search per warp, 2 always grouped, 3 always four warps per search.
+  // NNGP_FIT_MODE=auto|warp|grouped|quad
   int fit_mode = 0;
   cudaStream_t queue_stream = nullptr;  // stream of the last fit that took a queue slot (next_queue)
   bool queue_stream_valid = false;

@@ -36,10 +36,6 @@
 #include <cmath>
 #include <cstdlib>
 
-#ifndef NNGP_PIVOT_AHEAD
-#define NNGP_PIVOT_AHEAD 0  // see gp_core
-#endif
-
 static constexpr int GP_WARPS = 4;  // warps per CTA of the persistent fit kernel
 static constexpr unsigned FULL = 0xffffffffu;
 
@@ -497,15 +493,7 @@ __device__ __forceinline__ GpOut gp_core(double th0, double th1, double jit10, c
   double inv_own = 1.0, w_own = 0.0;  // ALPHA: 1/d_r and (L'^-1 y)_r of the own row
   bool ok = true;
   double u[M];
-  // NNGP_PIVOT_AHEAD (compile-time variant, off): the next pivot is formed redundantly in every lane from row
-  // k+1's diagonal (pn) and its column-k entry (bn), both broadcast one step ahead, with the very operations row
-  // k+1 applies to itself (bit-identical): the shuffle leaves the reciprocal -> scale -> update chain that
-  // serialises the M steps.  Measured (profiles/r02/fit_kernel_variants.log): slower where the sweep is
-  // throughput-bound (1 GPU, 357 -> 376 ms per iteration).
   double p = dd0, zk = shfl(z, 0);
-#if NNGP_PIVOT_AHEAD
-  double pn = dd0, bn = (M > 1) ? shfl(a[0], 1) : 0.0;
-#endif
   if (lane > 0 && lane < M) Kt[lane] = a[0];
   __syncwarp();
   load_col(0, u);
@@ -540,15 +528,7 @@ __device__ __forceinline__ GpOut gp_core(double th0, double th1, double jit10, c
     z = fma(-w, zk, z);
     if (k + 1 < M) {
       a[k + 1] = fma(-w, u[k + 1], a[k + 1]);
-#if NNGP_PIVOT_AHEAD
-      p = fma(-(bn * ip), bn, pn);  // == row k+1's dd after this step, bit for bit
-      if (k + 2 < M) {
-        pn = shfl(dd, k + 2);
-        bn = shfl(a[k + 1], k + 2);
-      }
-#else
       p = shfl(dd, k + 1);
-#endif
       zk = shfl(z, k + 1);
       if (k + 2 < M) {
         if (lane > k + 1 && lane < M) Kt[(k + 1) * LD + lane] = a[k + 1];
@@ -914,15 +894,11 @@ __device__ __forceinline__ void finish_search(const FitArgs& A, int task, double
   }
 }
 
-// registers per thread: 4-warp CTAs, K CTAs per SM
-#ifndef FIT_OCC20
-#define FIT_OCC20 3
-#endif
-static inline int FitOccRuntime(int m) { return (m <= 12) ? 4 : ((m <= 20) ? FIT_OCC20 : 2); }
-template <int M> struct FitOcc { static constexpr int value = (M <= 12) ? 4 : ((M <= 20) ? FIT_OCC20 : 2); };
+// registers per thread: 4-warp CTAs, fit_occ(m) CTAs per SM
+static constexpr int fit_occ(int m) { return (m <= 12) ? 4 : ((m <= 20) ? 3 : 2); }
 
 template <int M>
-__global__ void __launch_bounds__(GP_WARPS * 32, FitOcc<M>::value)
+__global__ void __launch_bounds__(GP_WARPS * 32, fit_occ(M))
 gp_fit_predict_kernel(FitArgs A) {
   extern __shared__ double sm[];
   const int m = A.m, d = A.d, R = A.R, nruns = NNGP_N_JITTER * R;
@@ -985,7 +961,7 @@ gp_fit_predict_kernel(FitArgs A) {
 // to the sequential search; an iteration costs one evaluation latency instead of two (four when it shrinks).
 // ---------------------------------------------------------------------------------------
 template <int M>
-__global__ void __launch_bounds__(GP_WARPS * 32, FitOcc<M>::value)
+__global__ void __launch_bounds__(GP_WARPS * 32, fit_occ(M))
 gp_fit_spec_kernel(FitArgs A) {
   static_assert(GP_WARPS == 4, "four candidate points per iteration");
   extern __shared__ double sm[];
@@ -1449,7 +1425,7 @@ int gp_fit_predict_launch(nngp_handle_t h, const long long* d_idx, const double*
     // Few searches per launch (a rank's share of the dimension-sharded sweep): the launch lasts as long as its
     // longest search, most warp slots idle -> four warps per search.  Measured per predict at the FHN target
     // (profiles/r02/fit_kernel_variants.log): 576 searches 388 -> 266 us, 1152: 429 -> 375 us, 2304: 504 -> 654 us.
-    const long long quad_limit = 3LL * h->sm_count * FitOccRuntime(m);
+    const long long quad_limit = 3LL * h->sm_count * fit_occ(m);
     if (h->fit_mode == 3 || (h->fit_mode == 0 && ntasks <= quad_limit)) {
       A.quad_all = 1;
     } else if (h->fit_budget >= 3) {

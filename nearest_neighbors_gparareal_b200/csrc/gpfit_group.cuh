@@ -323,10 +323,7 @@ __device__ __forceinline__ bool nm_step(NMState& S, double f, double fatol, doub
   return false;
 }
 
-#ifndef GRP_OCC20
-#define GRP_OCC20 2
-#endif
-template <int M> struct GrpOcc { static constexpr int value = (M <= 12) ? 4 : ((M <= 20) ? GRP_OCC20 : 2); };
+template <int M> struct GrpOcc { static constexpr int value = (M <= 12) ? 4 : 2; };
 
 // searches only: res[task] = (fval, theta0, theta1); selection and mean follow in gp_select_mean_kernel
 template <int M>

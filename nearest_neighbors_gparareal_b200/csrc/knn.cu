@@ -1115,9 +1115,8 @@ static int scan_select_launch(nngp_handle_t h, const double* d_q, int nq, int m,
   const int d = h->ds_d;
   double* dist = (double*)ws;
   char* base = (char*)ws + knn_pad256(sizeof(double) * (size_t)nq * (size_t)n);
-  static const bool no_tile = getenv("NNGP_KNN_NO_TILE") != nullptr;
   const size_t tile_smem = sizeof(double) * ((size_t)((d + 1) & ~1) + (size_t)TILE_ROWS * TILE_LD);
-  if (n <= KNN_TILE_MAX_ROWS && !no_tile && tile_smem <= 200 * 1024) {
+  if (n <= KNN_TILE_MAX_ROWS && tile_smem <= 200 * 1024) {
     const unsigned tchunks = (unsigned)((n + SCAN_ROWS - 1) / SCAN_ROWS);
     double* tcand_d = (double*)base;
     long long* tcand_i = (long long*)(base + knn_pad256(sizeof(double) * (size_t)nq * tchunks * m));
@@ -1152,8 +1151,7 @@ int knn_launch(nngp_handle_t h, const double* d_q, int nq, int m, long long n_ro
   const int d = h->ds_d;
   double* dist = (double*)ws;
   ProfScope prof(h, 1, st);
-  if (nq <= KNN_FUSED_MAX_Q && m <= NNGP_MAX_NEIGHBOURS && (size_t)d * sizeof(double) <= 48 * 1024 &&
-      getenv("NNGP_KNN_NO_FUSED") == nullptr)
+  if (nq <= KNN_FUSED_MAX_Q && m <= NNGP_MAX_NEIGHBOURS && (size_t)d * sizeof(double) <= 48 * 1024)
     return scan_select_launch(h, d_q, nq, m, n, d_idx, d_dist, nullptr, ws, st);
   const int tb = 128;
   const unsigned gx = (unsigned)((n + tb - 1) / tb);

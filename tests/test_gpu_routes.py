@@ -55,8 +55,7 @@ rk_small_kernel<SYS, S>                            the ODE systems              
                                                                                            tests/test_gpu_kernels.py
 
 S (stages) is chosen by the RK method alone; every RK case runs RK1, RK2, RK4 and RK8.  The environment switches used
-here (NNGP_RK_TILE, NNGP_RK_NO_SHFL, NNGP_RK_CHUNKS) are read on every call; NNGP_KNN_NO_TILE is read once per process
-and is not used: n > 8192 reaches scan_select_kernel instead.
+here (NNGP_RK_TILE, NNGP_RK_NO_SHFL, NNGP_RK_CHUNKS) are read on every call.
 """
 import os
 

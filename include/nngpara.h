@@ -166,7 +166,8 @@ int nngp_set_fit_budget(nngp_handle_t h, int evaluations);
 /* ---- fused on-device sweep: parareal.py:359-382 for slices i = I..N-1 -------------------
  * per slice: uG_next[i+1] = G(t_i, t_{i+1}, u_next[i]); kNN of u_next[i]; fit+predict;
  * u_next[i+1] = pred + uG_next[i+1].  No host round trip inside; d_starts holds the starts of
- * all N-I predicts in call order [(N-I), d, 9, R, 2].  d_t[N+1] slice boundaries.        */
+ * all N-I predicts in call order [(N-I), d, 9, R, 2].  d_t[N+1] slice boundaries.
+ * The whole-range, all-dimension case of nngp_sweep_shard (i_first = I, i_count = N-I, j0 = 0, dl = d). */
 int nngp_sweep(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g,
                const double* d_t, int N, int I, int m, int n_restarts,
                const signed char* d_starts, double fatol, double xatol, double* d_u_next,
@@ -174,7 +175,8 @@ int nngp_sweep(nngp_handle_t h, int sys, int method_g, int h_mode, long long ste
 /* One rank's share of the same sweep (SURVEY.md section 8e, optional sharding of the d*9*R fits of a predict by
  * output dimension): slices i_first .. i_first+i_count-1 of the sweep that starts at slice I; G and kNN in full,
  * fits and u_next[i+1] only for dimensions [j0, j0+dl).  The caller all-gathers row i+1 of u_next over the ranks
- * (d/W doubles each) before the next slice; results are bit-identical to nngp_sweep.                          */
+ * (d/W doubles each) before the next slice; results are bit-identical to nngp_sweep.  So a block dl < d takes
+ * i_count = 1 (rejected otherwise); with dl = d any range of slices is swept in one call.                     */
 int nngp_sweep_shard(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g,
                      const double* d_t, int N, int I, int i_first, int i_count, int m, int n_restarts,
                      const signed char* d_starts, double fatol, double xatol, double* d_u_next,

@@ -187,6 +187,31 @@ static unsigned int* seg_tickets(nngp_handle_t h, int nq) {
   return h->seg_tickets;
 }
 
+// kNN + neighbour matrix of nq queries: one launch (scan + top-m + neighbour matrix) for a single query when the
+// shape allows it, otherwise the general kNN followed by gp_prep_kernel
+static int knn_prep_launch(nngp_handle_t h, const double* d_q, int nq, int m, long long n, long long* idx, double* dist,
+                           void* kws, void* fws, cudaStream_t st) {
+  if (nq == 1 && knn_prep_fused_ok(h, n, m)) return knn_prep_fused_launch(h, d_q, m, n, idx, dist, (double*)fws, kws, st);
+  if (int rc = knn_launch(h, d_q, nq, m, n, idx, dist, kws, st)) return rc;
+  return gp_prep_launch(h, idx, nq, m, (double*)fws, st);
+}
+
+// Everything of a slice that precedes the fits: the coarse step gn = G(u) of nq rows (row stride ld) on the auxiliary
+// stream, beside it the neighbour search `knn` on the caller's stream, which then joins the auxiliary one before the
+// fit, whose epilogue adds gn to the prediction.
+template <class Knn>
+static int sweep_slice_prologue(nngp_handle_t h, const SystemDesc& s, int method_g, int h_mode, long long steps_g, int nq,
+                                const double* t0, const double* t1, const double* u, long long ld, double* gn,
+                                cudaStream_t st, Knn knn) {
+  NNGP_CUDA(h, cudaEventRecord(h->ev_fork, st));
+  NNGP_CUDA(h, cudaStreamWaitEvent(h->aux_stream, h->ev_fork, 0));
+  if (int rc = rk_launch(h, s, method_g, h_mode, steps_g, nq, t0, t1, u, ld, gn, ld, h->aux_stream)) return rc;
+  NNGP_CUDA(h, cudaEventRecord(h->ev_join, h->aux_stream));
+  if (int rc = knn()) return rc;
+  NNGP_CUDA(h, cudaStreamWaitEvent(st, h->ev_join, 0));
+  return 0;
+}
+
 extern "C" {
 
 int nngp_abi_version(void) { return NNGP_ABI_VERSION; }
@@ -721,12 +746,7 @@ int nngp_predict_host_block(nngp_handle_t h, const double* q, int nq, int m, lon
   int* order;
   if (int rc = fit_workspace(h, nq, n, m, R, &kws, &fws, &order)) return rc;
   if (int rc = ensure_done_zero(h, fws, nq, d, m, R, st)) return rc;
-  if (nq == 1 && n >= m && knn_prep_fused_ok(h, n, m)) {  // the sweep's shape: scan + top-m + neighbour matrix in one launch
-    if (int rc = knn_prep_fused_launch(h, gq, m, n, gidx, gdist, (double*)fws, kws, h->d_ticket, st)) return rc;
-  } else {
-    if (int rc = knn_launch(h, gq, nq, m, n, gidx, gdist, kws, st)) return rc;
-    if (int rc = gp_prep_launch(h, gidx, nq, m, (double*)fws, st)) return rc;
-  }
+  if (int rc = knn_prep_launch(h, gq, nq, m, n, gidx, gdist, kws, fws, st)) return rc;
   if (dl == d) {
     if (int rc = gp_order_launch(h, gst, nq, d * NNGP_N_JITTER * R, 1, order, st)) return rc;
   } else {  // the searches of the block are a contiguous range of the (single) query's task list
@@ -755,72 +775,19 @@ int nngp_predict_host_block(nngp_handle_t h, const double* q, int nq, int m, lon
   return 0;
 }
 
-// Everything of a slice that precedes the fits: the coarse step uG_next[i+1] = G(u_next[i]) on the auxiliary stream,
-// beside it ONE launch for distance scan + top-m + neighbour matrix (general shapes: three launches); the caller's
-// stream joins the auxiliary one before the fit, whose epilogue adds uG_next[i+1] to the prediction.
-static int sweep_slice_prologue(nngp_handle_t h, const SystemDesc& s, int method_g, int h_mode, long long steps_g,
-                                const double* d_ti, double* ui, double* gn, int d, int m, long long n, long long* idx,
-                                double* dist, void* kws, void* fws, cudaStream_t st) {
-  NNGP_CUDA(h, cudaEventRecord(h->ev_fork, st));
-  NNGP_CUDA(h, cudaStreamWaitEvent(h->aux_stream, h->ev_fork, 0));
-  if (int rc = rk_launch(h, s, method_g, h_mode, steps_g, 1, d_ti, d_ti + 1, ui, d, gn, d, h->aux_stream)) return rc;
-  NNGP_CUDA(h, cudaEventRecord(h->ev_join, h->aux_stream));
-  if (knn_prep_fused_ok(h, n, m)) {
-    if (int rc = knn_prep_fused_launch(h, ui, m, n, idx, dist, (double*)fws, kws, h->d_ticket, st)) return rc;
-  } else {
-    if (int rc = knn_launch(h, ui, 1, m, n, idx, dist, kws, st)) return rc;
-    if (int rc = gp_prep_launch(h, idx, 1, m, (double*)fws, st)) return rc;
-  }
-  NNGP_CUDA(h, cudaStreamWaitEvent(st, h->ev_join, 0));
-  return 0;
-}
-
 // ---- fused on-device sweep (parareal.py:359-382) --------------------------------------
 int nngp_sweep(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g,
                const double* d_t, int N, int I, int m, int n_restarts,
                const signed char* d_starts, double fatol, double xatol, double* d_u_next,
                double* d_uG_next, int d, void* stream) {
-  NNGP_USE_DEVICE(h);
-  const SystemDesc* s;
-  if (int rc = get_sys(h, sys, &s)) return rc;
-  if (d != s->d || d != h->ds_d) return nngp_fail(h, "sweep: d=%d, system d=%d, dataset d=%d", d, s->d, h->ds_d);
-  if (I < 0 || I > N) return nngp_fail(h, "sweep: I=%d outside [0,%d]", I, N);
-  cudaStream_t st = as_stream(stream);
-  if (n_restarts < 1) return nngp_fail(h, "sweep: n_restarts=%d < 1", n_restarts);
-  const long long n = h->ds_rows;
-  const size_t bk = Carver::pad(knn_workspace_bytes(1, n, m));
-  const size_t bf = Carver::pad(gp_fit_ws_bytes(1, d, m, n_restarts));
-  const size_t bi = Carver::pad(sizeof(long long) * m), bd = Carver::pad(sizeof(double) * m);
-  const int seg_len = d * NNGP_N_JITTER * n_restarts;
-  const size_t bo = Carver::pad(sizeof(int) * (size_t)seg_len * (size_t)(N - I));
-  char* ws = (char*)nngp_workspace(h, bk + bf + bi + bd + bo);
-  if (!ws) return nngp_fail(h, "sweep: out of device memory");
-  void* kws = ws;
-  void* fws = ws + bk;
-  long long* idx = (long long*)(ws + bk + bf);
-  double* dist = (double*)(ws + bk + bf + bi);
-  int* order = (int*)(ws + bk + bf + bi + bd);
-  if (int rc = ensure_done_zero(h, fws, 1, d, m, n_restarts, st)) return rc;
-  // queue order of every predict of the sweep in one launch (the starts are all known up front)
-  if (int rc = gp_order_launch(h, d_starts, N - I, seg_len, 0, order, st)) return rc;
-  const size_t per_predict = (size_t)d * NNGP_N_JITTER * n_restarts * 2;
-  for (int i = I; i < N; i++) {
-    double* ui = d_u_next + (long long)i * d;
-    double* un = d_u_next + (long long)(i + 1) * d;
-    double* gn = d_uG_next + (long long)(i + 1) * d;
-    if (int rc = sweep_slice_prologue(h, *s, method_g, h_mode, steps_g, d_t + i, ui, gn, d, m, n, idx, dist, kws, fws, st)) return rc;
-    if (int rc = gp_fit_predict_launch(h, idx, dist, fws, next_queue(h, st), order + (size_t)(i - I) * seg_len, 1, m,
-                                       n_restarts, d_starts + (size_t)(i - I) * per_predict, fatol, xatol, un, gn, d,
-                                       nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, st))
-      return rc;
-  }
-  return 0;
+  return nngp_sweep_shard(h, sys, method_g, h_mode, steps_g, d_t, N, I, I, N - I, m, n_restarts, d_starts, fatol, xatol,
+                          d_u_next, d_uG_next, d, 0, d, stream);
 }
 
-// One rank's share of the sweep for slices i_first .. i_first+i_count-1 (I = first slice of the whole
-// sweep: d_starts holds the starts of predicts I, I+1, ... in order): G and the neighbour search are done
-// in full (replicated, cheap), the d*9*R searches only for the output dimensions [j0, j0+dl); u_next[i+1]
-// is written for those dimensions only -- the caller all-gathers the row before the next slice.
+// Slices i_first .. i_first+i_count-1 of the sweep that starts at slice I (d_starts holds the starts of predicts I,
+// I+1, ... in order): G and the neighbour search in full, the d*9*R searches only for the output dimensions
+// [j0, j0+dl), and u_next[i+1] written for those dimensions only.  A block dl < d sweeps one slice per call: the
+// caller all-gathers row i+1 before the neighbour search of slice i+1 reads it.
 int nngp_sweep_shard(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g,
                      const double* d_t, int N, int I, int i_first, int i_count, int m, int n_restarts,
                      const signed char* d_starts, double fatol, double xatol, double* d_u_next,
@@ -829,18 +796,23 @@ int nngp_sweep_shard(nngp_handle_t h, int sys, int method_g, int h_mode, long lo
   const SystemDesc* s;
   if (int rc = get_sys(h, sys, &s)) return rc;
   if (d != s->d || d != h->ds_d) return nngp_fail(h, "sweep: d=%d, system d=%d, dataset d=%d", d, s->d, h->ds_d);
-  if (I < 0 || I > N || i_first < I || i_count < 0 || i_first + i_count > N)
-    return nngp_fail(h, "sweep_shard: slices [%d,%d) outside [%d,%d)", i_first, i_first + i_count, I, N);
-  if (j0 < 0 || dl < 1 || j0 + dl > d) return nngp_fail(h, "sweep_shard: dimensions [%d,%d) outside [0,%d)", j0, j0 + dl, d);
+  if (I < 0 || I > N) return nngp_fail(h, "sweep: I=%d outside [0,%d]", I, N);
+  if (i_first < I || i_count < 0 || i_first + i_count > N)
+    return nngp_fail(h, "sweep: slices [%d,%d) outside [%d,%d)", i_first, i_first + i_count, I, N);
+  if (j0 < 0 || dl < 1 || j0 + dl > d) return nngp_fail(h, "sweep: dimensions [%d,%d) outside [0,%d)", j0, j0 + dl, d);
+  if (dl < d && i_count > 1)
+    return nngp_fail(h, "sweep: a dimension block sweeps one slice per call (i_count=%d): row i+1 must be all-gathered "
+                     "before the neighbour search of slice i+1", i_count);
   if (n_restarts < 1) return nngp_fail(h, "sweep: n_restarts=%d < 1", n_restarts);
   cudaStream_t st = as_stream(stream);
   const long long n = h->ds_rows;
+  const int nruns = NNGP_N_JITTER * n_restarts;
+  const int seg_len = dl * nruns;
+  const size_t per_predict = (size_t)d * nruns * 2;
   const size_t bk = Carver::pad(knn_workspace_bytes(1, n, m));
   const size_t bf = Carver::pad(gp_fit_ws_bytes(1, d, m, n_restarts));
   const size_t bi = Carver::pad(sizeof(long long) * m), bd = Carver::pad(sizeof(double) * m);
-  const int nruns = NNGP_N_JITTER * n_restarts;
-  const int seg_len = dl * nruns;
-  const size_t bo = Carver::pad(sizeof(int) * (size_t)seg_len);
+  const size_t bo = Carver::pad(sizeof(int) * (size_t)seg_len * (size_t)i_count);
   char* ws = (char*)nngp_workspace(h, bk + bf + bi + bd + bo);
   if (!ws) return nngp_fail(h, "sweep: out of device memory");
   void* kws = ws;
@@ -849,16 +821,21 @@ int nngp_sweep_shard(nngp_handle_t h, int sys, int method_g, int h_mode, long lo
   double* dist = (double*)(ws + bk + bf + bi);
   int* order = (int*)(ws + bk + bf + bi + bd);
   if (int rc = ensure_done_zero(h, fws, 1, d, m, n_restarts, st)) return rc;
-  const size_t per_predict = (size_t)d * nruns * 2;
+  // queue order of every predict of the call in one launch (the starts are all known up front); with dl = d the
+  // blocks of consecutive predicts are contiguous, with dl < d there is one
+  const signed char* starts_first = d_starts + (size_t)(i_first - I) * per_predict;
+  if (int rc = gp_order_launch(h, starts_first + (size_t)j0 * nruns * 2, i_count, seg_len, 0, order, st)) return rc;
   for (int i = i_first; i < i_first + i_count; i++) {
     double* ui = d_u_next + (long long)i * d;
     double* un = d_u_next + (long long)(i + 1) * d;
     double* gn = d_uG_next + (long long)(i + 1) * d;
-    const signed char* starts_i = d_starts + (size_t)(i - I) * per_predict;
-    if (int rc = sweep_slice_prologue(h, *s, method_g, h_mode, steps_g, d_t + i, ui, gn, d, m, n, idx, dist, kws, fws, st)) return rc;
-    if (int rc = gp_order_launch(h, starts_i + (size_t)j0 * nruns * 2, 1, seg_len, 0, order, st)) return rc;
-    if (int rc = gp_fit_predict_launch(h, idx, dist, fws, next_queue(h, st), order, 1, m, n_restarts, starts_i, fatol,
-                                       xatol, un, gn, d, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, st, j0, dl))
+    if (int rc = sweep_slice_prologue(h, *s, method_g, h_mode, steps_g, 1, d_t + i, d_t + i + 1, ui, d, gn, st, [&] {
+          return knn_prep_launch(h, ui, 1, m, n, idx, dist, kws, fws, st);
+        }))
+      return rc;
+    if (int rc = gp_fit_predict_launch(h, idx, dist, fws, next_queue(h, st), order + (size_t)(i - i_first) * seg_len, 1, m,
+                                       n_restarts, starts_first + (size_t)(i - i_first) * per_predict, fatol, xatol, un,
+                                       gn, d, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, st, j0, dl))
       return rc;
   }
   return 0;
@@ -1053,16 +1030,11 @@ int nngp_ensemble_sweep(nngp_handle_t h, int sys, int method_g, int h_mode, long
     double* gn = d_uG_next + (long long)(i + 1) * d;
     if (int rc = ensure_done_zero(h, fws, n_act, d, m, n_restarts, st)) return rc;
     if (int rc = gp_order_launch(h, starts_i, n_act, seg_len, 1, order, st)) return rc;
-    // coarse step on the auxiliary stream beside the neighbour search (as in nngp_sweep)
-    NNGP_CUDA(h, cudaEventRecord(h->ev_fork, st));
-    NNGP_CUDA(h, cudaStreamWaitEvent(h->aux_stream, h->ev_fork, 0));
-    if (int rc = rk_launch(h, *s, method_g, h_mode, steps_g, n_act, t_rep + (size_t)i * E, t_rep + (size_t)(i + 1) * E,
-                           ui, ld, gn, ld, h->aux_stream))
+    if (int rc = sweep_slice_prologue(h, *s, method_g, h_mode, steps_g, n_act, t_rep + (size_t)i * E,
+                                      t_rep + (size_t)(i + 1) * E, ui, ld, gn, st, [&] {
+          return knn_seg_launch(h, ui, ld, n_act, m, dtab, dtab + E, n_max, idx, dist, (double*)fws, tickets, kws, st);
+        }))
       return rc;
-    NNGP_CUDA(h, cudaEventRecord(h->ev_join, h->aux_stream));
-    if (int rc = knn_seg_launch(h, ui, ld, n_act, m, dtab, dtab + E, n_max, idx, dist, (double*)fws, tickets, kws, st))
-      return rc;
-    NNGP_CUDA(h, cudaStreamWaitEvent(st, h->ev_join, 0));
     if (int rc = gp_fit_predict_launch(h, idx, dist, fws, next_queue(h, st), order, n_act, m, n_restarts, starts_i, fatol,
                                        xatol, un, gn, ld, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, st))
       return rc;

@@ -145,7 +145,7 @@ int knn_launch(nngp_handle_t h, const double* d_q, int nq, int m, long long n_ro
                long long* d_idx, double* d_dist, void* ws, cudaStream_t st);
 bool knn_prep_fused_ok(nngp_handle_t h, long long n, int m);
 int knn_prep_fused_launch(nngp_handle_t h, const double* d_q, int m, long long n, long long* d_idx, double* d_dist,
-                          double* d_r2, void* ws, unsigned int* ticket, cudaStream_t st);
+                          double* d_r2, void* ws, cudaStream_t st);
 int dataset_append_launch(nngp_handle_t h, const double* d_x, const double* d_y, long long rows,
                           cudaStream_t st);
 int append_iteration_launch(nngp_handle_t h, const double* d_u_cur, const double* d_uF,

@@ -1197,8 +1197,7 @@ bool knn_prep_fused_ok(nngp_handle_t h, long long n, int m) {
 }
 
 int knn_prep_fused_launch(nngp_handle_t h, const double* d_q, int m, long long n, long long* d_idx, double* d_dist,
-                          double* d_r2, void* ws, unsigned int* ticket, cudaStream_t st) {
-  (void)ticket;
+                          double* d_r2, void* ws, cudaStream_t st) {
   ProfScope prof(h, 1, st);
   return scan_select_launch(h, d_q, 1, m, n, d_idx, d_dist, d_r2, ws, st);
 }

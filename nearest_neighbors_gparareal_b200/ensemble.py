@@ -19,6 +19,7 @@ import numpy as np
 
 from . import _lib
 from .models import CudaNNGP, N_JITTER
+from .parareal import advance
 from .solver import CudaSolverRK
 from .systems import ODE
 
@@ -72,18 +73,6 @@ def pack_starts(blocks, I_pos, N):
                 break
             out.append(blocks[p][i - I])
     return np.ascontiguousarray(np.stack(out))
-
-
-def advance(err_k, I, eps):
-    """parareal.py:402-416 for one run: err_k[I] = 0, then I moves over the slices whose error is below eps"""
-    err_k[I] = 0
-    N = err_k.shape[0] - 1
-    for p in range(I + 1, N + 1):
-        if err_k[p] < eps:
-            I += 1
-        else:
-            break
-    return I
 
 
 class PararealEnsemble:

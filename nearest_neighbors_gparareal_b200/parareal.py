@@ -45,6 +45,18 @@ def gather_fine_rows(uF, I, chunk, rank, world, group=None):
     dist.all_gather_into_tensor(view, mine, group=group)
 
 
+def advance(err_k, I, eps):
+    """parareal.py:402-416 for one run: err_k[I] = 0, then I moves over the slices whose error is below eps"""
+    err_k[I] = 0
+    N = err_k.shape[0] - 1
+    for p in range(I + 1, N + 1):
+        if err_k[p] < eps:
+            I += 1
+        else:
+            break
+    return I
+
+
 class Parareal():
     def __init__(self, ode, solver, tspan, N, epsilon=5e-7, verbose='v', **kwargs):
         if not isinstance(ode, ODE):
@@ -492,17 +504,10 @@ class PararealDevice(Parareal):
     def device_advance(self, st, err_k):
         """parareal.py:402-416 after a sweep: the new iterate becomes the current one, `I` moves over the slices whose
         error is below epsilon.  err_k = the per-slice errors of this iteration (host array); returns the new I."""
-        I = st['I']
-        err_k[I] = 0
         st['u_cur'].copy_(st['u_next'])
         st['uG_cur'].copy_(st['uG_next'])
-        for p in range(I + 1, self.N + 1):
-            if err_k[p] < self.epsilon:
-                I += 1
-            else:
-                break
-        st['I'] = I
-        return I
+        st['I'] = advance(err_k, st['I'], self.epsilon)
+        return st['I']
 
     def _parareal(self, model, early_stop=None, parall='Serial', store_int=False, max_rows=None,
                   iteration_hook=None, **kwargs):

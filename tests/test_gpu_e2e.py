@@ -138,7 +138,8 @@ def test_full_size_fhn_target_against_published_run():
 
 def test_dimension_sharded_sweep_equals_replicated_sweep_bitwise():
     """nngp_sweep_shard (one rank's share of the fits of every predict, by output dimension) emulated on one
-    GPU: running the W blocks one after the other for every slice fills u_next exactly as nngp_sweep does"""
+    GPU: running the W blocks one after the other for every slice fills u_next exactly as nngp_sweep does, and so
+    does one nngp_sweep_shard call over all slices and dimensions"""
     import torch
     from nearest_neighbors_gparareal_b200 import _lib
     z, cfg, mkw, p = build("fhn_d32_N32_m12", nn.PararealDevice)
@@ -149,21 +150,35 @@ def test_dimension_sharded_sweep_equals_replicated_sweep_bitwise():
     h.append_iteration(st['u_cur'], st['uF'], st['uG_cur'], N, I, n, st['stream'])
     m = 12
     starts = torch.from_numpy(model.draw_starts(N - I)).to(st['dev'])
+
+    def shard(u, g, i_first, i_count, j0, dl):
+        h.sweep_shard(st['sys'], st['mG'], p.solver.h_mode, p.solver.Ng, st['t'], N, I, i_first, i_count, m, 1, starts,
+                      0.1, 0.1, u, g, n, j0, dl, st['stream'])
+
     ref_u, ref_g = st['u_next'].clone(), st['uG_next'].clone()
+    c0 = h.launch_count()
     h.sweep(st['sys'], st['mG'], p.solver.h_mode, p.solver.Ng, st['t'], N, I, m, 1, starts, 0.1, 0.1, ref_u, ref_g, n,
             st['stream'])
+    # per slice: the coarse step, the fused kNN and one fit; one queue-order launch for the whole sweep
+    assert h.launch_count() - c0 == 1 + 3 * (N - I)
     for world in (2, 4):
         u, g = st['u_next'].clone(), st['uG_next'].clone()
         for i in range(I, N):
             for rank in range(world):
                 j0, dl = nn.parareal.dim_block(n, rank, world)
-                h.sweep_shard(st['sys'], st['mG'], p.solver.h_mode, p.solver.Ng, st['t'], N, I, i, 1, m, 1, starts,
-                              0.1, 0.1, u, g, n, j0, dl, st['stream'])
+                c0 = h.launch_count()
+                shard(u, g, i, 1, j0, dl)
+                assert h.launch_count() - c0 == 4
         torch.cuda.synchronize()
         assert torch.equal(u, ref_u) and torch.equal(g, ref_g), world
+    u, g = st['u_next'].clone(), st['uG_next'].clone()
+    shard(u, g, I, N - I, 0, n)
+    torch.cuda.synchronize()
+    assert torch.equal(u, ref_u) and torch.equal(g, ref_g)
     with pytest.raises(_lib.NNGPError, match="outside"):
-        h.sweep_shard(st['sys'], st['mG'], p.solver.h_mode, p.solver.Ng, st['t'], N, I, I, 1, m, 1, starts, 0.1, 0.1,
-                      ref_u, ref_g, n, 24, 16, st['stream'])
+        shard(ref_u, ref_g, I, 1, 24, 16)
+    with pytest.raises(_lib.NNGPError, match="one slice per call"):
+        shard(u, g, I, 2, 0, n // 2)
 
 
 def test_checkpoint_and_resume_nngp_host_driver(tmp_path):

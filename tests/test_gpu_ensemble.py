@@ -182,7 +182,21 @@ def test_members_that_stop_at_different_iterations():
     epsilons = [eps, 1e-3, eps, 5e-6]
     stops = [None, None, 3, None]
     ics = [None, [-14.0, -15.0, 21.0], None, [-15.5, -14.0, 19.0]]
-    outs = _ensemble(key, kw, cfg, eps, mkw, seeds, epsilons=epsilons, early_stops=stops, init_conds=ics)
+    ode = device_system(key, **kw)
+    ens = nn.PararealEnsemble(ode, _solver(ode, cfg), tspan=cfg["tspan"], N=cfg["N"], epsilon=eps, verbose='')
+    h = ens.handle()
+    sweep, launches = h.ensemble_sweep, []
+
+    def counted_sweep(*args):
+        c0 = h.launch_count()
+        sweep(*args)
+        launches.append(h.launch_count() - c0)
+
+    h.ensemble_sweep = counted_sweep
+    outs = ens.run(model='nngp', seeds=seeds, epsilons=epsilons, early_stops=stops, init_conds=ics, **mkw)
+    # the first sweep, all four members at I = 1: the time table, then per slice the queue order, the coarse step,
+    # the segmented kNN and the grouped fit (searches, then selection and mean)
+    assert launches[0] == 1 + 5 * (cfg["N"] - 1), launches
     ks = set()
     for e, s in enumerate(seeds):
         ref = _solo(key, kw, cfg, epsilons[e], mkw, s, init_cond=ics[e], early_stop=stops[e])

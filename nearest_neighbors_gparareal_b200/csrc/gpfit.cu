@@ -343,9 +343,43 @@ __device__ __forceinline__ GpHead gp_head(double th0, double th1, double jit10, 
   return g;
 }
 
+// Pivots 1..4 of the leading 5 x 5 block  b_ij = K'_ij (i > j, diagonal dd0)  with exactly the operations the
+// factorisation in gp_core performs on these entries: true if one of them is not above pmin.  ip: the reciprocals
+// of pivots 0..3, which the factorisation reuses.  Called warp-wide by gp_core and per lane by nm_screen_fails, so the
+// two decide every point alike.
+__device__ __forceinline__ bool block5_fails(double b10, double b20, double b30, double b40, double b21, double b31,
+                                             double b32, double b41, double b42, double b43, double dd0, double pmin,
+                                             double (&ip)[4]) {
+  const double ip0 = rcp_pos(dd0);
+  double w1 = b10 * ip0, w2 = b20 * ip0, w3 = b30 * ip0, w4 = b40 * ip0;
+  const double d1 = fma(-w1, b10, dd0);
+  double d2 = fma(-w2, b20, dd0), d3 = fma(-w3, b30, dd0), d4 = fma(-w4, b40, dd0);
+  b21 = fma(-w2, b10, b21); b31 = fma(-w3, b10, b31); b41 = fma(-w4, b10, b41);
+  b32 = fma(-w3, b20, b32); b42 = fma(-w4, b20, b42);
+  b43 = fma(-w4, b30, b43);
+  const double ip1 = rcp_pos(d1);
+  w2 = b21 * ip1; w3 = b31 * ip1; w4 = b41 * ip1;
+  d2 = fma(-w2, b21, d2); d3 = fma(-w3, b31, d3); d4 = fma(-w4, b41, d4);
+  b32 = fma(-w3, b21, b32); b42 = fma(-w4, b21, b42);
+  b43 = fma(-w4, b31, b43);
+  const double ip2 = rcp_pos(d2);
+  w3 = b32 * ip2; w4 = b42 * ip2;
+  d3 = fma(-w3, b32, d3); d4 = fma(-w4, b42, d4);
+  b43 = fma(-w4, b32, b43);
+  const double ip3 = rcp_pos(d3);
+  w4 = b43 * ip3;
+  d4 = fma(-w4, b43, d4);
+  ip[0] = ip0; ip[1] = ip1; ip[2] = ip2; ip[3] = ip3;
+  // a failed pivot makes the later ones meaningless, exactly as in the factorisation (ok stays false)
+  return !(d1 > pmin) || !(d2 > pmin) || !(d3 > pmin) || !(d4 > pmin);
+}
+
 struct GpOut {
   double val, amp, c;
   bool ok;
+#ifdef NNGP_FIT_STATS
+  int stage;  // 1: failed at pivots 0 / 1 (head), 2: at pivots 2..4 (leading block), 3: factorised further
+#endif
 };
 
 template <int M, bool ALPHA>
@@ -369,6 +403,9 @@ __device__ __forceinline__ GpOut gp_core(double th0, double th1, double jit10, c
       bad.c = c;
       bad.ok = false;
       bad.val = dinf();
+#ifdef NNGP_FIT_STATS
+      bad.stage = 1;
+#endif
       return bad;
     }
   }
@@ -386,31 +423,8 @@ __device__ __forceinline__ GpOut gp_core(double th0, double th1, double jit10, c
     // one exponential and a 5 x 5 elimination instead of the whole kernel matrix, and the searches that run to
     // SciPy's 400-evaluation limit on failing points -- the chain that ends a launch -- shrink by 3-4x.
     const double k0 = P.pad[0] ? 0.0 : amp_s * v[0];
-    const double b10 = shfl(k0, 0), b20 = shfl(k0, 1), b30 = shfl(k0, 3), b40 = shfl(k0, 6);
-    double b21 = shfl(k0, 2), b31 = shfl(k0, 4), b32 = shfl(k0, 5), b41 = shfl(k0, 7), b42 = shfl(k0, 8),
-           b43 = shfl(k0, 9);
-    const double ip0 = rcp_pos(dd0);
-    double w1 = b10 * ip0, w2 = b20 * ip0, w3 = b30 * ip0, w4 = b40 * ip0;
-    const double d1 = fma(-w1, b10, dd0);
-    double d2 = fma(-w2, b20, dd0), d3 = fma(-w3, b30, dd0), d4 = fma(-w4, b40, dd0);
-    b21 = fma(-w2, b10, b21); b31 = fma(-w3, b10, b31); b41 = fma(-w4, b10, b41);
-    b32 = fma(-w3, b20, b32); b42 = fma(-w4, b20, b42);
-    b43 = fma(-w4, b30, b43);
-    const double ip1 = rcp_pos(d1);
-    w2 = b21 * ip1; w3 = b31 * ip1; w4 = b41 * ip1;
-    d2 = fma(-w2, b21, d2); d3 = fma(-w3, b31, d3); d4 = fma(-w4, b41, d4);
-    b32 = fma(-w3, b21, b32); b42 = fma(-w4, b21, b42);
-    b43 = fma(-w4, b31, b43);
-    const double ip2 = rcp_pos(d2);
-    w3 = b32 * ip2; w4 = b42 * ip2;
-    d3 = fma(-w3, b32, d3); d4 = fma(-w4, b42, d4);
-    b43 = fma(-w4, b32, b43);
-    const double ip3 = rcp_pos(d3);
-    w4 = b43 * ip3;
-    d4 = fma(-w4, b43, d4);
-    // a failed pivot makes the later ones meaningless, exactly as in the loop below (ok stays false)
-    fail5 = !(d1 > pmin) || !(d2 > pmin) || !(d3 > pmin) || !(d4 > pmin);
-    ipb[0] = ip0; ipb[1] = ip1; ipb[2] = ip2; ipb[3] = ip3;
+    fail5 = block5_fails(shfl(k0, 0), shfl(k0, 1), shfl(k0, 3), shfl(k0, 6), shfl(k0, 2), shfl(k0, 4), shfl(k0, 5),
+                         shfl(k0, 7), shfl(k0, 8), shfl(k0, 9), dd0, pmin, ipb);
   }
   if constexpr (NP > 1) {
     constexpr int NV = NP - 1;
@@ -445,6 +459,9 @@ __device__ __forceinline__ GpOut gp_core(double th0, double th1, double jit10, c
       bad.c = c;
       bad.ok = false;
       bad.val = dinf();
+#ifdef NNGP_FIT_STATS
+      bad.stage = 2;
+#endif
       return bad;
     }
   }
@@ -512,6 +529,9 @@ __device__ __forceinline__ GpOut gp_core(double th0, double th1, double jit10, c
         bad.c = c;
         bad.ok = false;
         bad.val = dinf();
+#ifdef NNGP_FIT_STATS
+        bad.stage = 3;
+#endif
         __syncwarp();  // the next evaluation overwrites the tile
         return bad;
       }
@@ -554,6 +574,9 @@ __device__ __forceinline__ GpOut gp_core(double th0, double th1, double jit10, c
   o.amp = amp;
   o.c = c;
   o.ok = ok;
+#ifdef NNGP_FIT_STATS
+  o.stage = 3;
+#endif
   if (!ALPHA) {
     __syncwarp();  // the next evaluation overwrites the tile
     // -(-0.5*y@alpha - sum(log(diag L)) - (N/2) log(2 pi)),  sum log L_rr = 0.5 log det K,
@@ -623,6 +646,94 @@ __device__ __forceinline__ double shrink_to(double x0, double xj) {
   return __dadd_rn(x0, __dmul_rn(0.5, __dsub_rn(xj, x0)));
 }
 
+// Look-ahead of a search whose sorted simplex is all +inf.  While every value stays +inf, every comparison of the state
+// machine is false: an iteration evaluates the reflection, the inside contraction and the two shrunk vertices, then
+// keeps the best vertex, moves the other two halfway towards it, and the sort leaves the order as it is.  So the next
+// 8 iterations' 32 points are known in advance; lane l computes point l (iteration l / 4, in SciPy's order) with the
+// state machine's own operations.
+__device__ __forceinline__ void nm_lookahead_point(const double (&sx)[3][2], int lane, double& t0, double& t1) {
+  const int k = lane >> 2, s = lane & 3;
+  double a0 = sx[1][0], a1 = sx[1][1], b0 = sx[2][0], b1 = sx[2][1];
+#pragma unroll
+  for (int i = 0; i < 7; i++) {
+    if (i < k) {
+      a0 = shrink_to(sx[0][0], a0); a1 = shrink_to(sx[0][1], a1);
+      b0 = shrink_to(sx[0][0], b0); b1 = shrink_to(sx[0][1], b1);
+    }
+  }
+  const double xb0 = __dmul_rn(__dadd_rn(sx[0][0], a0), 0.5), xb1 = __dmul_rn(__dadd_rn(sx[0][1], a1), 0.5);
+  if (s == 0) {  // reflection
+    t0 = __dsub_rn(__dmul_rn(2.0, xb0), b0); t1 = __dsub_rn(__dmul_rn(2.0, xb1), b1);
+  } else if (s == 1) {  // inside contraction
+    t0 = __dadd_rn(__dmul_rn(0.5, xb0), __dmul_rn(0.5, b0)); t1 = __dadd_rn(__dmul_rn(0.5, xb1), __dmul_rn(0.5, b1));
+  } else if (s == 2) {  // shrunk second vertex
+    t0 = shrink_to(sx[0][0], a0); t1 = shrink_to(sx[0][1], a1);
+  } else {  // shrunk worst vertex
+    t0 = shrink_to(sx[0][0], b0); t1 = shrink_to(sx[0][1], b1);
+  }
+}
+
+// The leading whole iterations of a window whose four points all fail the screen, skipped in one step: each ends with
+// the two shrunk vertices (points 4k-2 and 4k-1 of the window) and +inf values, so after k of them the simplex is
+// (sx[0], point 4k-2, point 4k-1), fcalls has grown by 4k and it by k.  k stops before maxfun / maxiter would end
+// the search, so the state machine applies those ends itself.  Returns k; the caller forms the next reflection.
+__device__ __forceinline__ int nm_skip_iterations(unsigned fails, double t0, double t1, double (&sx)[3][2], int& fcalls,
+                                                  int& it, int maxfun, int maxiter) {
+  int k = (fails == FULL) ? 8 : (__ffs(~fails) - 1) >> 2;
+  k = min(k, min((maxfun - 1 - fcalls) >> 2, maxiter - 1 - it));
+  if (k > 0) {
+    sx[1][0] = shfl(t0, 4 * k - 2); sx[1][1] = shfl(t1, 4 * k - 2);
+    sx[2][0] = shfl(t0, 4 * k - 1); sx[2][1] = shfl(t1, 4 * k - 1);
+    fcalls += 4 * k;
+    it += k;
+  }
+  return k;
+}
+
+// Does the objective at this lane's point fail at pivots 0..4?  gp_head and the leading-block check of gp_core, with
+// the lane's own arguments: the ten block entries, which gp_core gathers by shuffle from lanes 0..9, are computed
+// here from their squared distances (slot 0 of lanes 0..9) with the same operations, so both decide alike.
+template <int M>
+__device__ __noinline__ bool nm_screen_fails(double th0, double th1, double jit10, const PairSlots<M>& P, int m,
+                                             double guard) {
+  const GpHead hd = gp_head(th0, th1, jit10, P.r2_10, m, guard);
+  double x[10], v[10];
+  bool pad[10];
+#pragma unroll
+  for (int e = 0; e < 10; e++) {
+    x[e] = hd.c * shfl(P.r2[0], e);
+    pad[e] = __shfl_sync(FULL, (int)P.pad[0], e) != 0;
+  }
+  {
+    double xa[5], oa[5];
+#pragma unroll
+    for (int e = 0; e < 5; e++) xa[e] = x[e];
+    exp_neg_vec<5>(xa, oa);
+#pragma unroll
+    for (int e = 0; e < 5; e++) v[e] = oa[e];
+#pragma unroll
+    for (int e = 0; e < 5; e++) xa[e] = x[5 + e];
+    exp_neg_vec<5>(xa, oa);
+#pragma unroll
+    for (int e = 0; e < 5; e++) v[5 + e] = oa[e];
+  }
+  double k[10];
+#pragma unroll
+  for (int e = 0; e < 10; e++) k[e] = pad[e] ? 0.0 : hd.amp_s * v[e];
+  double ip[4];
+  const bool fail5 = block5_fails(k[0], k[1], k[3], k[6], k[2], k[4], k[5], k[7], k[8], k[9], hd.dd0, hd.pmin, ip);
+  return hd.fail01 || fail5;
+}
+
+#ifdef NNGP_FIT_STATS
+// statistics build only (scripts/fit_inf_share_probe.py): evaluations of nelder_mead by where they were decided,
+// [0..3] in iterations that start with every vertex +inf, [4..7] in the others (and the three initial ones):
+// not evaluated (look-ahead), failed at pivots 0 / 1, failed at pivots 2..4, factorised further;
+// [8] / [9] warp cycles spent in the two kinds of iteration; [10] searches, [11] searches with an all-inf iteration,
+// [12] their warp cycles, [13] the longest search in cycles
+__device__ unsigned long long g_nm_stats[16];
+#endif
+
 template <int M>
 __device__ __forceinline__ NMOut nelder_mead(double s0, double s1, double jit10, double fatol, double xatol,
                                              const PairSlots<M>& P, double y, int m, int lane,
@@ -638,19 +749,50 @@ __device__ __forceinline__ NMOut nelder_mead(double s0, double s1, double jit10,
   int fcalls = 0, it = 1, phase = PH_INIT0;
   double p0 = s0, p1 = s1;
   double xb0 = 0, xb1 = 0, xr0 = 0, xr1 = 0, fxr = 0;
-  // When every vertex is +inf an iteration evaluates the reflection, the inside contraction and the two shrunk
-  // vertices -- four points known in advance.  Their heads (gp_head: do pivots 0 / 1 fail?) are computed at
-  // once in four lanes; an evaluation whose point is in this list with a failing head returns +inf without
-  // being repeated.  Same arithmetic, same decisions, a quarter of the work for the searches that run to maxfev.
-  double cx0[4], cx1[4];
-  unsigned cmask = 0;
+  // When every vertex is +inf (head_batch), the next 32 points are screened at once, one per lane (nm_lookahead_point,
+  // nm_screen_fails).  The leading whole iterations whose points all fail are skipped in one step (nm_skip_iterations);
+  // for the other screened-out points the state machine consumes +inf without evaluating them, so the decisions and
+  // the maxfun / aborted rules of a partial iteration are its own.  A point that passes the screen is evaluated; while
+  // its value is +inf the rest of the window still applies, a finite one ends it.
+  double la0 = 0.0, la1 = 0.0;  // this lane's point of the window
+  unsigned lfail = 0;           // bit l: point l fails at pivots 0..4
+  int lpos = 32;                // position of the next evaluation in the window; 32: no window
+#ifdef NNGP_FIT_STATS
+  unsigned long long st_n[8] = {0, 0, 0, 0, 0, 0, 0, 0}, st_cyc[2] = {0, 0};
+  const long long st_begin = clock64();
+  long long st_last = st_begin;
+  int st_inf = 0, st_any_inf = 0;
+#endif
   for (;;) {
-    bool hit = false;
-    if (cmask) {
-#pragma unroll
-      for (int j = 0; j < 4; j++) hit = hit || (((cmask >> j) & 1u) && p0 == cx0[j] && p1 == cx1[j]);
+#ifdef NNGP_FIT_STATS
+    {
+      const long long now = clock64();
+      st_cyc[st_inf] += (unsigned long long)(now - st_last);
+      st_last = now;
     }
+#endif
+    bool hit = false;
+    if (lpos < 32) {
+      if (p0 == shfl(la0, lpos) && p1 == shfl(la1, lpos)) {
+        hit = (lfail >> lpos) & 1u;
+        lpos++;
+      } else {
+        lpos = 32;
+      }
+    }
+#ifdef NNGP_FIT_STATS
+    double f = dinf();
+    if (hit) {
+      st_n[st_inf ? 0 : 4]++;
+    } else {
+      const GpOut g = gp_core<M, false>(p0, p1, jit10, P, y, m, lane, Lt, hml, guard);
+      f = g.val;
+      st_n[(st_inf ? 0 : 4) + g.stage]++;
+    }
+#else
     const double f = hit ? dinf() : gp_core<M, false>(p0, p1, jit10, P, y, m, lane, Lt, hml, guard).val;
+#endif
+    if (f != dinf()) lpos = 32;  // a finite value changes the trajectory
     fcalls++;
     bool aborted = false, do_shrink = false;
     if (phase == PH_INIT0) {
@@ -741,25 +883,49 @@ __device__ __forceinline__ NMOut nelder_mead(double s0, double s1, double jit10,
     xr0 = __dsub_rn(__dmul_rn(2.0, xb0), sx[2][0]);
     xr1 = __dsub_rn(__dmul_rn(2.0, xb1), sx[2][1]);
     phase = PH_REFLECT; p0 = xr0; p1 = xr1;
-    cmask = 0;
+#ifdef NNGP_FIT_STATS
+    st_inf = (sf[0] == dinf()) ? 1 : 0;
+    st_any_inf |= st_inf;
+#endif
     // iteration boundary: sorted simplex, nothing pending.  Searches whose vertices are all +inf stay here: their
-    // iterations cost four head checks in four lanes (below), cheaper than a CTA round of the continuation kernel
+    // iterations are screened 32 points at a time (below), cheaper than a CTA round of the continuation kernel
     if (budget > 0 && fcalls >= budget && sf[0] != dinf()) {
       unfinished = true;
       break;
     }
-    if (head_batch && sf[0] == dinf()) {  // sorted: the best vertex is +inf, so all are
-      cx0[0] = xr0; cx1[0] = xr1;
-      cx0[1] = __dadd_rn(__dmul_rn(0.5, xb0), __dmul_rn(0.5, sx[2][0]));  // inside contraction
-      cx1[1] = __dadd_rn(__dmul_rn(0.5, xb1), __dmul_rn(0.5, sx[2][1]));
-      cx0[2] = shrink_to(sx[0][0], sx[1][0]); cx1[2] = shrink_to(sx[0][1], sx[1][1]);
-      cx0[3] = shrink_to(sx[0][0], sx[2][0]); cx1[3] = shrink_to(sx[0][1], sx[2][1]);
-      const int jl = lane & 3;
-      const double t0 = (jl == 0) ? cx0[0] : (jl == 1) ? cx0[1] : (jl == 2) ? cx0[2] : cx0[3];
-      const double t1 = (jl == 0) ? cx1[0] : (jl == 1) ? cx1[1] : (jl == 2) ? cx1[2] : cx1[3];
-      cmask = __ballot_sync(FULL, gp_head(t0, t1, jit10, P.r2_10, m, guard).fail01) & 0xFu;
+    // sorted: the best vertex is +inf, so all are.  An unfinished window still holds this iteration's points.
+    if (head_batch && sf[0] == dinf() && lpos >= 32) {
+      nm_lookahead_point(sx, lane, la0, la1);
+      lfail = __ballot_sync(FULL, nm_screen_fails<M>(la0, la1, jit10, P, m, guard));
+      const int k = nm_skip_iterations(lfail, la0, la1, sx, fcalls, it, maxfun, maxiter);
+      if (k > 0) {
+        xb0 = __dmul_rn(__dadd_rn(sx[0][0], sx[1][0]), 0.5);
+        xb1 = __dmul_rn(__dadd_rn(sx[0][1], sx[1][1]), 0.5);
+        xr0 = __dsub_rn(__dmul_rn(2.0, xb0), sx[2][0]);
+        xr1 = __dsub_rn(__dmul_rn(2.0, xb1), sx[2][1]);
+        p0 = xr0; p1 = xr1;
+#ifdef NNGP_FIT_STATS
+        st_n[0] += 4 * k;
+#endif
+      }
+      lpos = 4 * k;
     }
   }
+#ifdef NNGP_FIT_STATS
+  {
+    const long long now = clock64();
+    st_cyc[st_inf] += (unsigned long long)(now - st_last);
+    if (lane == 0) {
+      for (int i = 0; i < 8; i++) atomicAdd(g_nm_stats + i, st_n[i]);
+      atomicAdd(g_nm_stats + 8, st_cyc[1]);
+      atomicAdd(g_nm_stats + 9, st_cyc[0]);
+      atomicAdd(g_nm_stats + 10, 1ULL);
+      atomicAdd(g_nm_stats + 11, (unsigned long long)st_any_inf);
+      if (st_any_inf) atomicAdd(g_nm_stats + 12, (unsigned long long)(now - st_begin));
+      atomicMax(g_nm_stats + 13, (unsigned long long)(now - st_begin));
+    }
+  }
+#endif
   NMOut o;
   o.x0 = sx[0][0];
   o.x1 = sx[0][1];
@@ -799,7 +965,7 @@ struct FitArgs {
   unsigned int* queue;    // next task to hand out; zero on entry
   const int* order;       // optional [ntasks]: queue position -> task (longest searches first)
   int d, m, R, ntasks;
-  int head_batch;         // 1: pre-decide the four points of an all-inf Nelder-Mead iteration at once (0: tests)
+  int head_batch;         // 1: screen the points of all-inf Nelder-Mead iterations ahead, in lanes (0: one by one, tests)
   int j0, dl;             // output dimensions [j0, j0+dl) handled by this launch (a rank's share; dl = d: all)
   long long ld_pred;      // row stride of pred / add
   double fatol, xatol;
@@ -1505,5 +1671,12 @@ extern "C" void nngp_fit_stats_dump(void) {
   fprintf(stderr, " | head fail01 %llu of wanted %llu\n", hst[16], hst[17]);
   unsigned long long z[18] = {0};
   cudaMemcpyToSymbol(g_fail_hist, z, sizeof(z));
+  unsigned long long s[16];
+  cudaMemcpyFromSymbol(s, g_nm_stats, sizeof(s));
+  fprintf(stderr, "nelder_mead evaluations, all-inf iterations: look-ahead %llu head %llu block %llu further %llu | "
+          "other: look-ahead %llu head %llu block %llu further %llu | cycles all-inf %llu other %llu | searches %llu "
+          "with all-inf iterations %llu (cycles %llu) | longest search %llu cycles\n",
+          s[0], s[1], s[2], s[3], s[4], s[5], s[6], s[7], s[8], s[9], s[10], s[11], s[12], s[13]);
+  cudaMemcpyToSymbol(g_nm_stats, z, sizeof(s));
 }
 #endif

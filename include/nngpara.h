@@ -225,6 +225,21 @@ int nngp_copy_rows(nngp_handle_t h, const double* d_src, const long long* d_src_
 int nngp_ensemble_sweep(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g, const double* d_t, int N,
                         int E, const int* members, const int* I, int m, int n_restarts, const signed char* d_starts,
                         double fatol, double xatol, double* d_u_next, double* d_uG_next, int d, void* stream);
+/* nngp_ensemble_sweep for runs that differ in neighbour count and time grid: m[E] (host) the neighbour count of each
+ * position, d_t_pos (device [E, N+1]) the slice boundaries of each position.  Per slice one segmented kNN at the
+ * largest m of the active runs (the first m_p neighbours of a top-m_max list are the top-m_p), then one fit per
+ * distinct m over the runs that use it, each seeing exactly the neighbour set and matrix of its nngp_sweep.  A slice
+ * in which an active run holds fewer rows than the slice's largest m is refused before anything is enqueued. */
+int nngp_ensemble_sweep_mixed(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g,
+                              const double* d_t_pos, int N, int E, const int* members, const int* I, const int* m,
+                              int n_restarts, const signed char* d_starts, double fatol, double xatol,
+                              double* d_u_next, double* d_uG_next, int d, void* stream);
+/* nngp_fit_predict with one neighbour count per predict: m[nq] (host); d_idx / d_dist rows ld = max m apart, the
+ * first m[q] entries of row q used; the neighbour matrix is formed at ld.  Outputs as nngp_fit_predict. */
+int nngp_fit_predict_mixed(nngp_handle_t h, const double* d_q, const long long* d_idx, const double* d_dist, int nq,
+                           const int* m, int n_restarts, const signed char* d_starts, double fatol, double xatol,
+                           double* d_pred, double* d_theta_opt, double* d_jitter_opt, double* d_fval_opt, int* d_nfev,
+                           double* d_fvals, double* d_thetas, void* stream);
 
 /* test hook: the device exp(-|x|), 1/|x| and -- when d_exp10 (2n doubles) is not NULL -- [10**x | log|x| + 3 ln 2]
  * used inside the GP kernels */

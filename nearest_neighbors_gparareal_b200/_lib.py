@@ -72,6 +72,8 @@ SIGNATURES = {
     "nngp_knn_segmented": (ci, [vp, vp, cll, ci, ci, vp, vp, vp, vp, vp, vp]),
     "nngp_copy_rows": (ci, [vp, vp, vp, vp, vp, cll, cll, vp]),
     "nngp_ensemble_sweep": (ci, [vp, ci, ci, ci, cll, vp, ci, ci, vp, vp, ci, ci, vp, cd, cd, vp, vp, ci, vp]),
+    "nngp_ensemble_sweep_mixed": (ci, [vp, ci, ci, ci, cll, vp, ci, ci, vp, vp, vp, ci, vp, cd, cd, vp, vp, ci, vp]),
+    "nngp_fit_predict_mixed": (ci, [vp, vp, vp, vp, ci, vp, ci, vp, cd, cd, vp, vp, vp, vp, vp, vp, vp, vp]),
 }
 
 SYSTEM_IDS = {"FHN_ODE": 0, "Rossler": 1, "Hopf": 2, "DblPend": 3, "Brusselator": 4, "Lorenz": 5,
@@ -268,6 +270,15 @@ class Handle:
                                              _ptr(d_pred), _ptr(d_theta), _ptr(d_jit), _ptr(d_fval),
                                              _ptr(d_nfev), _ptr(d_fvals), _ptr(d_thetas), stream))
 
+    def fit_predict_mixed(self, d_q, d_idx, d_dist, m, n_restarts, d_starts, fatol, xatol, d_pred, d_theta=None,
+                          d_jit=None, d_fval=None, d_nfev=None, d_fvals=None, d_thetas=None, stream=None):
+        """fit_predict with one neighbour count m[q] per predict; idx / dist rows max(m) apart"""
+        m = np.ascontiguousarray(m, dtype=np.int32)
+        self.check(self.lib.nngp_fit_predict_mixed(self.h, _ptr(d_q), _ptr(d_idx), _ptr(d_dist), m.size, _ptr(m),
+                                                   int(n_restarts), _ptr(d_starts), float(fatol), float(xatol),
+                                                   _ptr(d_pred), _ptr(d_theta), _ptr(d_jit), _ptr(d_fval),
+                                                   _ptr(d_nfev), _ptr(d_fvals), _ptr(d_thetas), stream))
+
     def gp_nll(self, d_idx, nq, m, nt, d_theta, d_jitter10, d_nll, stream=None):
         self.check(self.lib.nngp_gp_nll(self.h, _ptr(d_idx), int(nq), int(m), int(nt), _ptr(d_theta),
                                         _ptr(d_jitter10), _ptr(d_nll), stream))
@@ -331,6 +342,17 @@ class Handle:
                                                 members.size, _ptr(members), _ptr(I), int(m), int(n_restarts),
                                                 _ptr(d_starts), float(fatol), float(xatol), _ptr(d_u_next),
                                                 _ptr(d_uG_next), int(d), stream))
+
+    def ensemble_sweep_mixed(self, sys, method_g, h_mode, steps_g, d_t_pos, N, members, I, m, n_restarts, d_starts,
+                             fatol, xatol, d_u_next, d_uG_next, d, stream=None):
+        """ensemble_sweep with one neighbour count m[p] and one time grid d_t_pos[p] (device [E, N+1]) per position"""
+        members, I = np.ascontiguousarray(members, dtype=np.int32), np.ascontiguousarray(I, dtype=np.int32)
+        m = np.ascontiguousarray(m, dtype=np.int32)
+        assert m.size == members.size
+        self.check(self.lib.nngp_ensemble_sweep_mixed(self.h, sys, method_g, h_mode, int(steps_g), _ptr(d_t_pos), int(N),
+                                                      members.size, _ptr(members), _ptr(I), _ptr(m), int(n_restarts),
+                                                      _ptr(d_starts), float(fatol), float(xatol), _ptr(d_u_next),
+                                                      _ptr(d_uG_next), int(d), stream))
 
     def selftest_math(self, d_x, n, d_exp, d_rcp, d_exp10=None, stream=None):
         self.check(self.lib.nngp_selftest_math(self.h, _ptr(d_x), int(n), _ptr(d_exp), _ptr(d_rcp),

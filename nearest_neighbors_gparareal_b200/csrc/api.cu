@@ -966,9 +966,215 @@ __global__ void repeat_t_kernel(const double* __restrict__ t, int n_t, int E, do
   if (e < (long long)n_t * E) t_rep[e] = t[e / E];
 }
 
-int nngp_ensemble_sweep(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g, const double* d_t, int N,
-                        int E, const int* members, const int* I, int m, int n_restarts, const signed char* d_starts,
-                        double fatol, double xatol, double* d_u_next, double* d_uG_next, int d, void* stream) {
+// t_rep[i, p] = t_pos[p, i]: per-position time grids in the layout of repeat_t_kernel
+__global__ void transpose_t_kernel(const double* __restrict__ t_pos, int n_t, int E, double* __restrict__ t_rep) {
+  const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e < (long long)n_t * E) {
+    const long long i = e / E, p = e - i * E;
+    t_rep[e] = t_pos[p * n_t + i];
+  }
+}
+
+// `rows` rows of `bytes` bytes, row r from src + r src_ld to dst + r dst_ld (strides in bytes)
+struct CopySpan {
+  const char* src;
+  char* dst;
+  long long src_ld, dst_ld;
+  int bytes, rows;
+};
+
+// one warp per span; 8-byte words when every address and stride allows it
+__global__ void __launch_bounds__(256) copy_spans_kernel(const CopySpan* __restrict__ sp, int n) {
+  const int s = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (s >= n) return;
+  const CopySpan x = sp[s];
+  const bool w8 = ((((unsigned long long)x.src | (unsigned long long)x.dst | (unsigned long long)x.src_ld |
+                     (unsigned long long)x.dst_ld | (unsigned long long)x.bytes) & 7ull) == 0);
+  for (int r = 0; r < x.rows; r++) {
+    const char* a = x.src + r * x.src_ld;
+    char* b = x.dst + r * x.dst_ld;
+    if (w8) {
+      for (int k = lane; k < x.bytes / 8; k += 32) ((long long*)b)[k] = ((const long long*)a)[k];
+    } else {
+      for (int k = lane; k < x.bytes; k += 32) b[k] = a[k];
+    }
+  }
+}
+
+static int copy_spans_launch(nngp_handle_t h, const CopySpan* d_sp, int n, cudaStream_t st) {
+  if (n <= 0) return 0;
+  ProfScope prof(h, 4, st);
+  copy_spans_kernel<<<(unsigned)((n + 7) / 8), 256, 0, st>>>(d_sp, n);
+  h->launches++;
+  NNGP_CUDA(h, cudaGetLastError());
+  return 0;
+}
+
+static CopySpan copy_span(const void* src, void* dst, size_t bytes, int rows = 1, long long src_ld = 0, long long dst_ld = 0) {
+  return CopySpan{(const char*)src, (char*)dst, src_ld, dst_ld, (int)bytes, rows};
+}
+
+// The predicts of a fit with one neighbour count per predict, grouped by count: group g holds the positions pos[g]
+// (ascending) whose count is m[g].  Each group gets compact inputs (neighbour rows, matrix, starts, the added term)
+// and its own fit workspace, so its fit is an ordinary launch at m[g] over exactly what a solo fit at m[g] reads.
+// One fit per distinct m, not one per template size: the objective's determinant product is split at M/2 and
+// the padding rows' pivots enter it, so the bits of a search depend on the template size M as well as on m.
+struct MixedGroups {
+  std::vector<int> m;
+  std::vector<std::vector<int>> pos;
+  std::vector<int> grp, rank;  // position -> group, rank in its group
+  struct Dev {
+    char* fws;
+    int* order;
+    long long* idx;
+    double *dist, *add, *pred, *theta_opt, *jitter_opt, *fval_opt, *fvals, *thetas;
+    int* nfev;
+    signed char* starts;
+    const char* done_ptr = nullptr;  // the fit leaves its completion counters zero; clear them when they move
+    size_t done_bytes = 0;
+  };
+  std::vector<Dev> dev;
+
+  MixedGroups(const int* m_pos, int n) : grp(n), rank(n) {
+    std::vector<int> ms(m_pos, m_pos + n);
+    std::sort(ms.begin(), ms.end());
+    ms.erase(std::unique(ms.begin(), ms.end()), ms.end());
+    m = ms;
+    pos.resize(m.size());
+    for (int p = 0; p < n; p++) {
+      const int g = (int)(std::lower_bound(m.begin(), m.end(), m_pos[p]) - m.begin());
+      grp[p] = g;
+      rank[p] = (int)pos[g].size();
+      pos[g].push_back(p);
+    }
+    dev.resize(m.size());
+  }
+  // device bytes of every group's block (details: the per-search outputs of nngp_fit_predict too)
+  size_t bytes(int d, int R, bool details) const {
+    size_t t = 0;
+    for (size_t g = 0; g < m.size(); g++) t += group_bytes((int)g, d, R, details, nullptr);
+    return t;
+  }
+  void carve(char* base, int d, int R, bool details) {
+    for (size_t g = 0; g < m.size(); g++) {
+      dev[g].fws = base;
+      base += group_bytes((int)g, d, R, details, &dev[g]);
+    }
+  }
+  size_t group_bytes(int g, int d, int R, bool details, Dev* out) const {
+    const size_t n = pos[g].size(), mg = m[g], nt = n * d * NNGP_N_JITTER * R;
+    size_t off = 0;
+    auto take = [&](size_t b) { const size_t o = off; off += Carver::pad(b); return o; };
+    const size_t o_f = take(gp_fit_ws_bytes((int)n, d, (int)mg, R)), o_o = take(sizeof(int) * nt),
+                 o_i = take(sizeof(long long) * n * mg), o_d = take(sizeof(double) * n * mg), o_s = take(2 * nt),
+                 o_a = take(sizeof(double) * n * d), o_p = take(sizeof(double) * n * d);
+    size_t o_th = 0, o_j = 0, o_fv = 0, o_nf = 0, o_fs = 0, o_ts = 0;
+    if (details) {
+      o_th = take(sizeof(double) * n * d * 2); o_j = take(sizeof(double) * n * d); o_fv = take(sizeof(double) * n * d);
+      o_nf = take(sizeof(int) * nt); o_fs = take(sizeof(double) * nt); o_ts = take(sizeof(double) * nt * 2);
+    }
+    if (out) {
+      char* b = out->fws;  // the group's base (carve)
+      out->order = (int*)(b + o_o); out->idx = (long long*)(b + o_i); out->dist = (double*)(b + o_d);
+      out->starts = (signed char*)(b + o_s); out->add = (double*)(b + o_a); out->pred = (double*)(b + o_p);
+      out->theta_opt = details ? (double*)(b + o_th) : nullptr;
+      out->jitter_opt = details ? (double*)(b + o_j) : nullptr;
+      out->fval_opt = details ? (double*)(b + o_fv) : nullptr;
+      out->nfev = details ? (int*)(b + o_nf) : nullptr;
+      out->fvals = details ? (double*)(b + o_fs) : nullptr;
+      out->thetas = details ? (double*)(b + o_ts) : nullptr;
+      out->fws = b + o_f;
+      out->done_ptr = nullptr;
+    }
+    return off;
+  }
+};
+// order + fit of the first n active predicts of group g (compact inputs already gathered); pred += add when add_on
+static int mixed_fit_group(nngp_handle_t h, MixedGroups& G, int g, int n, int d, int R, double fatol, double xatol,
+                           bool add_on, cudaStream_t st) {
+  MixedGroups::Dev& D = G.dev[g];
+  const int mg = G.m[g], seg_len = d * NNGP_N_JITTER * R;
+  const char* done = D.fws + gp_fit_done_offset(n, d, mg, R);
+  const size_t done_bytes = sizeof(unsigned int) * (size_t)n * d;
+  if (D.done_ptr != done || D.done_bytes != done_bytes) {
+    NNGP_CUDA(h, cudaMemsetAsync((void*)done, 0, done_bytes, st));
+    D.done_ptr = done;
+    D.done_bytes = done_bytes;
+  }
+  if (int rc = gp_order_launch(h, D.starts, n, seg_len, 1, D.order, st)) return rc;
+  return gp_fit_predict_launch(h, D.idx, D.dist, D.fws, next_queue(h, st), D.order, n, mg, R, D.starts, fatol, xatol,
+                               D.pred, add_on ? D.add : nullptr, d, D.theta_opt, D.jitter_opt, D.fval_opt, D.nfev,
+                               D.fvals, D.thetas, st);
+}
+
+// The copies that hand predict p (rank r of group g) its inputs: the first m_g neighbours of its row of the kNN at
+// row stride mm, the leading m_g x m_g block of its mm x mm neighbour matrix, its starts and (optional) added term.
+static void mixed_gather_spans(std::vector<CopySpan>& sp, MixedGroups& G, int p, const long long* idx,
+                               const double* dist, const double* r2, int mm, const signed char* starts, size_t per_predict,
+                               const double* add, long long ld_add, int d) {
+  const int g = G.grp[p], r = G.rank[p], mg = G.m[g];
+  const MixedGroups::Dev& D = G.dev[g];
+  sp.push_back(copy_span(idx + (size_t)p * mm, D.idx + (size_t)r * mg, sizeof(long long) * mg));
+  sp.push_back(copy_span(dist + (size_t)p * mm, D.dist + (size_t)r * mg, sizeof(double) * mg));
+  sp.push_back(copy_span(r2 + (size_t)p * mm * mm, D.fws + sizeof(double) * (size_t)r * mg * mg, sizeof(double) * mg, mg,
+                    (long long)sizeof(double) * mm, (long long)sizeof(double) * mg));
+  sp.push_back(copy_span(starts + (size_t)p * per_predict, D.starts + (size_t)r * per_predict, per_predict));
+  if (add) sp.push_back(copy_span(add + (size_t)p * ld_add, D.add + (size_t)r * d, sizeof(double) * d));
+}
+
+int nngp_fit_predict_mixed(nngp_handle_t h, const double* d_q, const long long* d_idx, const double* d_dist, int nq,
+                           const int* m, int n_restarts, const signed char* d_starts, double fatol, double xatol,
+                           double* d_pred, double* d_theta_opt, double* d_jitter_opt, double* d_fval_opt, int* d_nfev,
+                           double* d_fvals, double* d_thetas, void* stream) {
+  NNGP_USE_DEVICE(h);
+  (void)d_q;
+  if (nq <= 0) return 0;
+  if (n_restarts < 1) return nngp_fail(h, "fit_mixed: n_restarts=%d < 1", n_restarts);
+  int ld = 0;
+  for (int q = 0; q < nq; q++) {
+    if (m[q] < 1 || m[q] > NNGP_MAX_NEIGHBOURS_BIG)
+      return nngp_fail(h, "fit_mixed: predict %d: m=%d outside [1,%d]", q, m[q], NNGP_MAX_NEIGHBOURS_BIG);
+    ld = std::max(ld, m[q]);
+  }
+  const int d = h->ds_d, R = n_restarts, seg_len = d * NNGP_N_JITTER * R;
+  const size_t per_predict = (size_t)seg_len * 2;
+  MixedGroups G(m, nq);
+  const size_t br = Carver::pad(gp_prep_bytes(nq, ld));
+  char* ws = (char*)nngp_workspace(h, br + G.bytes(d, R, true));
+  if (!ws) return nngp_fail(h, "fit_mixed: out of device memory");
+  G.carve(ws + br, d, R, true);
+  double* r2 = (double*)ws;
+  std::vector<CopySpan> sp;
+  for (int q = 0; q < nq; q++) mixed_gather_spans(sp, G, q, d_idx, d_dist, r2, ld, d_starts, per_predict, nullptr, 0, d);
+  const size_t n_gather = sp.size();
+  const size_t nd = sizeof(double) * d, nt = (size_t)seg_len;
+  for (int q = 0; q < nq; q++) {
+    const int r = G.rank[q];
+    const MixedGroups::Dev& D = G.dev[G.grp[q]];
+    sp.push_back(copy_span(D.pred + (size_t)r * d, d_pred + (size_t)q * d, nd));
+    if (d_theta_opt) sp.push_back(copy_span(D.theta_opt + (size_t)r * 2 * d, d_theta_opt + (size_t)q * 2 * d, 2 * nd));
+    if (d_jitter_opt) sp.push_back(copy_span(D.jitter_opt + (size_t)r * d, d_jitter_opt + (size_t)q * d, nd));
+    if (d_fval_opt) sp.push_back(copy_span(D.fval_opt + (size_t)r * d, d_fval_opt + (size_t)q * d, nd));
+    if (d_nfev) sp.push_back(copy_span(D.nfev + r * nt, d_nfev + q * nt, sizeof(int) * nt));
+    if (d_fvals) sp.push_back(copy_span(D.fvals + r * nt, d_fvals + q * nt, sizeof(double) * nt));
+    if (d_thetas) sp.push_back(copy_span(D.thetas + r * nt * 2, d_thetas + q * nt * 2, sizeof(double) * nt * 2));
+  }
+  cudaStream_t st = as_stream(stream);
+  const CopySpan* dsp = (const CopySpan*)upload_table(h, 2, sp.data(), sizeof(CopySpan) * sp.size(), st);
+  if (!dsp) return nngp_fail(h, "fit_mixed: out of memory for the copy table");
+  if (int rc = gp_prep_launch(h, d_idx, nq, ld, r2, st)) return rc;
+  if (int rc = copy_spans_launch(h, dsp, (int)n_gather, st)) return rc;
+  for (size_t g = 0; g < G.m.size(); g++)
+    if (int rc = mixed_fit_group(h, G, (int)g, (int)G.pos[g].size(), d, R, fatol, xatol, false, st)) return rc;
+  return copy_spans_launch(h, dsp + n_gather, (int)(sp.size() - n_gather), st);
+}
+
+// nngp_ensemble_sweep (m_pos == nullptr: one m and the shared grid d_t) and nngp_ensemble_sweep_mixed (m_pos[E] and
+// the per-position grids d_t_pos[E, N+1]).
+static int ensemble_sweep_impl(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g, const double* d_t,
+                               const double* d_t_pos, int N, int E, const int* members, const int* I, int m,
+                               const int* m_pos, int n_restarts, const signed char* d_starts, double fatol,
+                               double xatol, double* d_u_next, double* d_uG_next, int d, void* stream) {
   NNGP_USE_DEVICE(h);
   const SystemDesc* s;
   if (int rc = get_sys(h, sys, &s)) return rc;
@@ -976,27 +1182,57 @@ int nngp_ensemble_sweep(nngp_handle_t h, int sys, int method_g, int h_mode, long
   if (d != s->d || d != h->ds_d) return nngp_fail(h, "ensemble_sweep: d=%d, system d=%d, store d=%d", d, s->d, h->ds_d);
   if (E < 1) return nngp_fail(h, "ensemble_sweep: E=%d < 1", E);
   if (n_restarts < 1) return nngp_fail(h, "ensemble_sweep: n_restarts=%d < 1", n_restarts);
-  if (m < 1 || m > NNGP_MAX_NEIGHBOURS_BIG) return nngp_fail(h, "ensemble_sweep: m=%d outside [1,%d]", m, NNGP_MAX_NEIGHBOURS_BIG);
+  const bool mixed = m_pos != nullptr;
+  if (mixed) {
+    m = 0;
+    for (int p = 0; p < E; p++) {
+      if (m_pos[p] < 1 || m_pos[p] > NNGP_MAX_NEIGHBOURS_BIG)
+        return nngp_fail(h, "ensemble_sweep: position %d: m=%d outside [1,%d]", p, m_pos[p], NNGP_MAX_NEIGHBOURS_BIG);
+      if (I[p] < N) m = std::max(m, m_pos[p]);
+    }
+  } else if (m < 1 || m > NNGP_MAX_NEIGHBOURS_BIG) {
+    return nngp_fail(h, "ensemble_sweep: m=%d outside [1,%d]", m, NNGP_MAX_NEIGHBOURS_BIG);
+  }
   std::vector<long long> tab(2 * (size_t)E);
   for (int p = 0; p < E; p++) {
     const int e = members[p];
     if (e < 0 || e >= h->seg_E) return nngp_fail(h, "ensemble_sweep: member %d outside [0,%d)", e, h->seg_E);
     if (I[p] < 0 || I[p] > N || (p > 0 && I[p] < I[p - 1]))
       return nngp_fail(h, "ensemble_sweep: I must be ascending in [0,%d] (position %d: %d)", N, p, I[p]);
-    if (I[p] < N && h->seg_rows[e] < m)
+    if (!mixed && I[p] < N && h->seg_rows[e] < m)
       return nngp_fail(h, "ensemble_sweep: member %d holds %lld rows, fewer than m=%d", e, h->seg_rows[e], m);
     tab[p] = (long long)e * h->seg_cap;
     tab[E + p] = h->seg_rows[e];
   }
   if (I[0] >= N) return 0;
+  if (mixed) {
+    // each slice searches its runs' neighbours at the largest m among them: a run whose segment is shorter would
+    // read padding indices as rows.  Refused before anything is enqueued.
+    int n_act = 0, mm = 0, short_p = -1;
+    for (int i = I[0]; i < N; i++) {
+      while (n_act < E && I[n_act] <= i) {
+        mm = std::max(mm, m_pos[n_act]);
+        if (short_p < 0 || tab[E + n_act] < tab[E + short_p]) short_p = n_act;
+        n_act++;
+      }
+      if (tab[E + short_p] < mm)
+        return nngp_fail(h, "ensemble_sweep: member %d holds %lld rows, fewer than m=%d, the largest m of slice %d",
+                         members[short_p], tab[E + short_p], mm, i);
+    }
+  }
   cudaStream_t st = as_stream(stream);
   const long long ld = (long long)(N + 1) * d;
   long long n_max_all = 0;
   for (int p = 0; p < E; p++) n_max_all = std::max(n_max_all, tab[E + p]);
   const int seg_len = d * NNGP_N_JITTER * n_restarts;
   const size_t per_predict = (size_t)seg_len * 2;
+  int n_sw = 0;  // positions that sweep at least one slice
+  while (n_sw < E && I[n_sw] < N) n_sw++;
   const size_t bk = Carver::pad(knn_seg_workspace_bytes(E, n_max_all, m));
-  const size_t bf = Carver::pad(gp_fit_ws_bytes(E, d, m, n_restarts));
+  // mixed: the kNN's neighbour matrices get their own block; the fits work in the groups' blocks
+  MixedGroups G(m_pos, mixed ? n_sw : 0);
+  const size_t bf = mixed ? Carver::pad(gp_prep_bytes(E, m)) + G.bytes(d, n_restarts, false)
+                          : Carver::pad(gp_fit_ws_bytes(E, d, m, n_restarts));
   const size_t bi = Carver::pad(sizeof(long long) * (size_t)E * m), bd = Carver::pad(sizeof(double) * (size_t)E * m);
   const size_t bo = Carver::pad(sizeof(int) * (size_t)E * seg_len);
   const size_t bt = Carver::pad(sizeof(double) * (size_t)(N + 1) * E);
@@ -1013,21 +1249,69 @@ int nngp_ensemble_sweep(nngp_handle_t h, int sys, int method_g, int h_mode, long
   double* t_rep = (double*)(ws + bk + bf + bi + bd + bo);
   {
     const long long tot = (long long)(N + 1) * E;
-    repeat_t_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(d_t, N + 1, E, t_rep);
+    if (d_t_pos)
+      transpose_t_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(d_t_pos, N + 1, E, t_rep);
+    else
+      repeat_t_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(d_t, N + 1, E, t_rep);
     h->launches++;
     NNGP_CUDA(h, cudaGetLastError());
   }
+  // mixed: every slice's gather and scatter copies, in one table for the whole sweep
+  std::vector<CopySpan> sp;
+  std::vector<size_t> sp_at;  // per slice: start of its gather spans, start of its scatter spans
+  if (mixed) {
+    G.carve((char*)fws + Carver::pad(gp_prep_bytes(E, m)), d, n_restarts, false);
+    size_t done_predicts = 0;
+    int n_act = 0, mm = 0;
+    for (int i = I[0]; i < N; i++) {
+      while (n_act < E && I[n_act] <= i) mm = std::max(mm, m_pos[n_act++]);
+      const signed char* starts_i = d_starts + done_predicts * per_predict;
+      const double* gn = d_uG_next + (long long)(i + 1) * d;
+      double* un = d_u_next + (long long)(i + 1) * d;
+      sp_at.push_back(sp.size());
+      for (int p = 0; p < n_act; p++)
+        mixed_gather_spans(sp, G, p, idx, dist, (const double*)fws, mm, starts_i, per_predict, gn, ld, d);
+      sp_at.push_back(sp.size());
+      for (int p = 0; p < n_act; p++)
+        sp.push_back(copy_span(G.dev[G.grp[p]].pred + (size_t)G.rank[p] * d, un + (size_t)p * ld, sizeof(double) * d));
+      done_predicts += n_act;
+    }
+    sp_at.push_back(sp.size());
+  }
+  const CopySpan* dsp = nullptr;
+  if (mixed && !(dsp = (const CopySpan*)upload_table(h, 2, sp.data(), sizeof(CopySpan) * sp.size(), st)))
+    return nngp_fail(h, "ensemble_sweep: out of memory for the copy table");
   // The members active at slice i (I <= i) are a prefix of the positions: every launch below reaches them with the
   // member stride (N+1) d of the state, and their predicts' starts are consecutive in d_starts (slice-major).
   size_t done_predicts = 0;
-  int n_act = 0;
+  int n_act = 0, mm = 0;
   long long n_max = 0;
   for (int i = I[0]; i < N; i++) {
-    while (n_act < E && I[n_act] <= i) n_max = std::max(n_max, tab[E + n_act++]);
+    while (n_act < E && I[n_act] <= i) {
+      if (mixed) mm = std::max(mm, m_pos[n_act]);
+      n_max = std::max(n_max, tab[E + n_act++]);
+    }
     const signed char* starts_i = d_starts + done_predicts * per_predict;
     double* ui = d_u_next + (long long)i * d;
     double* un = d_u_next + (long long)(i + 1) * d;
     double* gn = d_uG_next + (long long)(i + 1) * d;
+    if (mixed) {
+      const size_t* at = sp_at.data() + 2 * (size_t)(i - I[0]);
+      if (int rc = sweep_slice_prologue(h, *s, method_g, h_mode, steps_g, n_act, t_rep + (size_t)i * E,
+                                        t_rep + (size_t)(i + 1) * E, ui, ld, gn, st, [&] {
+            return knn_seg_launch(h, ui, ld, n_act, mm, dtab, dtab + E, n_max, idx, dist, (double*)fws, tickets, kws, st);
+          }))
+        return rc;
+      if (int rc = copy_spans_launch(h, dsp + at[0], (int)(at[1] - at[0]), st)) return rc;
+      for (size_t g = 0; g < G.m.size(); g++) {
+        const int n_g = (int)(std::lower_bound(G.pos[g].begin(), G.pos[g].end(), n_act) - G.pos[g].begin());
+        if (n_g > 0)
+          if (int rc = mixed_fit_group(h, G, (int)g, n_g, d, n_restarts, fatol, xatol, true, st)) return rc;
+      }
+      if (int rc = copy_spans_launch(h, dsp + at[1], (int)(at[2] - at[1]), st)) return rc;
+      done_predicts += n_act;
+      continue;
+    }
     if (int rc = ensure_done_zero(h, fws, n_act, d, m, n_restarts, st)) return rc;
     if (int rc = gp_order_launch(h, starts_i, n_act, seg_len, 1, order, st)) return rc;
     if (int rc = sweep_slice_prologue(h, *s, method_g, h_mode, steps_g, n_act, t_rep + (size_t)i * E,
@@ -1041,6 +1325,22 @@ int nngp_ensemble_sweep(nngp_handle_t h, int sys, int method_g, int h_mode, long
     done_predicts += n_act;
   }
   return 0;
+}
+
+int nngp_ensemble_sweep(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g, const double* d_t, int N,
+                        int E, const int* members, const int* I, int m, int n_restarts, const signed char* d_starts,
+                        double fatol, double xatol, double* d_u_next, double* d_uG_next, int d, void* stream) {
+  return ensemble_sweep_impl(h, sys, method_g, h_mode, steps_g, d_t, nullptr, N, E, members, I, m, nullptr, n_restarts,
+                             d_starts, fatol, xatol, d_u_next, d_uG_next, d, stream);
+}
+
+int nngp_ensemble_sweep_mixed(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g,
+                              const double* d_t_pos, int N, int E, const int* members, const int* I, const int* m,
+                              int n_restarts, const signed char* d_starts, double fatol, double xatol,
+                              double* d_u_next, double* d_uG_next, int d, void* stream) {
+  if (m == nullptr || d_t_pos == nullptr) return nngp_fail(h, "ensemble_sweep_mixed: m and d_t_pos are required");
+  return ensemble_sweep_impl(h, sys, method_g, h_mode, steps_g, nullptr, d_t_pos, N, E, members, I, 0, m, n_restarts,
+                             d_starts, fatol, xatol, d_u_next, d_uG_next, d, stream);
 }
 
 int nngp_selftest_math(nngp_handle_t h, const double* d_x, int n, double* d_exp_neg, double* d_rcp,

@@ -92,7 +92,7 @@ struct nngp_handle_s {
   // small host->device tables of the segmented entry points: pinned staging, re-used once the copy that last read it
   // has completed (event)
   struct Upload { void* host = nullptr; void* dev = nullptr; size_t bytes = 0; cudaEvent_t done = nullptr; };
-  Upload up[2];
+  Upload up[3];  // 0 row tables, 1 segment tables, 2 copy spans of the mixed ensemble sweep
   // device counters: [0] Nelder-Mead runs, [1] objective (nll) evaluations
   unsigned long long* d_counters = nullptr;
   // task-queue heads of the persistent fit kernel: one zeroed counter per launch

@@ -1,10 +1,11 @@
 """Many independent nnGParareal runs as one device-resident ensemble.
 
-`PararealEnsemble.run(seeds=[...])` runs E solves of the same system, solver, tspan, N, `nn`, `n_restarts`,
-`fatol` and `xatol` in lockstep; the runs may differ in seed, initial condition, epsilon and early_stop.  Every
+`PararealEnsemble.run(seeds=[...])` runs E solves of the same system, solver, N, `n_restarts`, `fatol` and `xatol` in
+lockstep; the runs may differ in seed, initial condition, epsilon, early_stop, neighbour count `nn` and time span.  Every
 iteration makes the launches of one `PararealDevice` iteration, each over all runs at once: one fine-step launch, one
 dataset append, and per slice of the sweep one coarse step, one kNN (each run searches its own rows of a segmented
-store, csrc/knn.cu) and one fit over all the runs' predicts.  Run e's output dict equals, bit for bit, what
+store, csrc/knn.cu) and one fit over all the runs' predicts -- one fit per distinct neighbour count when the runs'
+counts differ (nngp_ensemble_sweep_mixed).  Run e's output dict equals, bit for bit, what
 `PararealDevice(...).run(model='nngp', seed=seeds[e], ...)` returns with its settings.
 
 Layout: the state is [E, N+1, d] per array.  At the start of every iteration the member axis is re-ordered by
@@ -26,8 +27,18 @@ from .systems import ODE
 MAX_NEIGHBOURS = 160  # include/nngpara.h: NNGP_MAX_NEIGHBOURS_BIG
 
 
+def _check_nn(nn):
+    if isinstance(nn, str):
+        if nn != 'adaptive':
+            raise ValueError(f"nn={nn!r}: 'adaptive' or 1 to {MAX_NEIGHBOURS} neighbours")
+        return
+    if isinstance(nn, bool) or int(nn) != nn or not (1 <= int(nn) <= MAX_NEIGHBOURS):
+        raise ValueError(f'nn={nn}: 1 to {MAX_NEIGHBOURS} neighbours are supported')
+
+
 def check_run_args(E_lists, model='nngp', store_int=False, nn='adaptive'):
-    """Validates the per-member lists of `PararealEnsemble.run` (dict name -> list or None); returns E."""
+    """Validates the per-member lists of `PararealEnsemble.run` (dict name -> list or None); returns E.
+    `nn` is one value for every member or a list with one per member; E_lists['tspans'] entries are [t0, t1] or None."""
     if not isinstance(model, str) or model.lower() != 'nngp':
         raise ValueError(f"PararealEnsemble runs the 'nngp' model only (got {model!r})")
     if store_int:
@@ -36,12 +47,37 @@ def check_run_args(E_lists, model='nngp', store_int=False, nn='adaptive'):
     if seeds is None or len(seeds) == 0:
         raise ValueError('PararealEnsemble.run needs a non-empty list of seeds')
     E = len(seeds)
-    for name, v in E_lists.items():
+    lists = dict(E_lists)
+    if isinstance(nn, (list, tuple, np.ndarray)):
+        lists['nn'] = nn
+    for name, v in lists.items():
         if v is not None and len(v) != E:
             raise ValueError(f'{name} has {len(v)} entries, seeds has {E}: give one per member')
-    if nn != 'adaptive' and not (1 <= int(nn) <= MAX_NEIGHBOURS):
-        raise ValueError(f'nn={nn}: 1 to {MAX_NEIGHBOURS} neighbours are supported')
+    for v in (nn if isinstance(nn, (list, tuple, np.ndarray)) else [nn]):
+        _check_nn(v)
+    for ts in E_lists.get('tspans') or []:
+        if ts is not None and not (len(ts) == 2 and float(ts[1]) > float(ts[0])):
+            raise ValueError(f'tspan {list(ts)}: give [t0, t1] with t1 > t0')
     return E
+
+
+def sweep_tables(m_members, t_members, sw):
+    """Per-position neighbour counts and time grids of a sweep over the members sw (state order)."""
+    sw = np.asarray(sw, dtype=np.int64)
+    return np.asarray(m_members, dtype=np.int32)[sw], np.ascontiguousarray(np.asarray(t_members)[sw])
+
+
+def launch_sweep(h, t_dev, sysid, mG, hm, steps, N, sw, I_sw, m_pos, t_pos, mdl0, starts, u_next, uG_next, n, stream):
+    """nngp_ensemble_sweep when every position has the same m and grid, otherwise nngp_ensemble_sweep_mixed.
+    t_dev: the members' grids [E, N+1], uploaded once per run; rows are selected on the device."""
+    import torch
+    if np.all(m_pos == m_pos[0]) and np.all(t_pos == t_pos[0]):
+        h.ensemble_sweep(sysid, mG, hm, steps, t_dev[int(sw[0])], N, sw, I_sw, int(m_pos[0]), mdl0.n_restarts, starts,
+                         mdl0.fatol, mdl0.xatol, u_next, uG_next, n, stream)
+    else:
+        rows = torch.from_numpy(np.asarray(sw, dtype=np.int64)).to(t_dev.device)
+        h.ensemble_sweep_mixed(sysid, mG, hm, steps, t_dev.index_select(0, rows), N, sw, I_sw, m_pos,
+                               mdl0.n_restarts, starts, mdl0.fatol, mdl0.xatol, u_next, uG_next, n, stream)
 
 
 def member_order(I, done):
@@ -104,10 +140,14 @@ class PararealEnsemble:
         return self._h
 
     def run(self, model='nngp', seeds=None, nn='adaptive', n_restarts=1, fatol=None, xatol=None, epsilons=None,
-            early_stops=None, init_conds=None, max_rows=None, store_int=False):
-        """Returns one output dict per seed (the keys of PararealDevice.run, n_rows included)."""
-        E = check_run_args(dict(seeds=seeds, epsilons=epsilons, early_stops=early_stops, init_conds=init_conds),
-                           model=model, store_int=store_int, nn=nn)
+            early_stops=None, init_conds=None, tspans=None, max_rows=None, store_int=False):
+        """Returns one output dict per seed (the keys of PararealDevice.run, n_rows included).
+
+        nn: 'adaptive', an int in 1..160, or a list with one of those per member.  tspans: None or a list with one
+        [t0, t1] (or None: the ensemble's tspan) per member; member e's output 't' is its own grid.  n_restarts,
+        fatol and xatol are common to all members."""
+        E = check_run_args(dict(seeds=seeds, epsilons=epsilons, early_stops=early_stops, init_conds=init_conds,
+                                tspans=tspans), model=model, store_int=store_int, nn=nn)
         solver = self.solver
         if max(solver.Nf, solver.Ng) > solver.thresh:
             raise Exception('steps > thresh (RK paging, solver.py:89-96) is only supported by the host driver')
@@ -115,12 +155,15 @@ class PararealEnsemble:
         stops = [None if early_stops is None else early_stops[e] for e in range(E)]
         u0s = np.stack([self.u0 if init_conds is None or init_conds[e] is None else self.ode.get_init_cond(u0=init_conds[e])
                         for e in range(E)])
+        nns = list(nn) if isinstance(nn, (list, tuple, np.ndarray)) else [nn] * E
+        spans = [self.tspan if tspans is None or tspans[e] is None else tspans[e] for e in range(E)]
+        t_members = np.stack([np.linspace(ts[0], ts[1], num=self.N + 1) for ts in spans])
         h = self.handle()
-        models = [CudaNNGP(n=self.n, N=self.N, seed=s, nn=nn, n_restarts=n_restarts, fatol=fatol, xatol=xatol,
-                           handle=h) for s in seeds]
-        return self._run(h, models, eps, stops, u0s, max_rows)
+        models = [CudaNNGP(n=self.n, N=self.N, seed=s, nn=v if v == 'adaptive' else int(v), n_restarts=n_restarts,
+                           fatol=fatol, xatol=xatol, handle=h) for s, v in zip(seeds, nns)]
+        return self._run(h, models, eps, stops, u0s, max_rows, t_members)
 
-    def _run(self, h, models, eps, stops, u0s, max_rows):
+    def _run(self, h, models, eps, stops, u0s, max_rows, t_members):
         import torch
         N, n, solver = self.N, self.n, self.solver
         E = len(models)
@@ -132,9 +175,8 @@ class PararealEnsemble:
         f64 = dict(dtype=torch.float64, device=dev)
         ld = (N + 1) * n
         tic = time.time()
-        t_host = np.linspace(self.tspan[0], self.tspan[1], num=N + 1)
-        t = torch.from_numpy(t_host).to(dev)
-        t_rep = t.repeat_interleave(E)  # t_rep[i E + p] = t_i
+        t_dev = torch.from_numpy(t_members).to(dev)  # [E, N+1], member order
+        t_rep = t_dev.t().contiguous().view(-1)  # t_rep[i E + p] = t_p[i]
         st = {key: torch.zeros((E, N + 1, n), **f64) for key in ('u_cur', 'uG_cur', 'uF')}
         for a in st.values():
             a[:, 0] = torch.from_numpy(u0s).to(dev)
@@ -180,7 +222,8 @@ class PararealEnsemble:
             # fine solves of every running member's unconverged slices in one launch (parareal.py:309-334)
             fr, fs = fine_rows(I[live], N)
             idx = torch.from_numpy(np.concatenate([fr, fr + 1, np.arange(n_live) * (N + 1) + I[live] + 1])).to(dev)
-            tt = torch.from_numpy(np.concatenate([t_host[fs], t_host[fs + 1]])).to(dev)
+            fm = np.repeat(live, N - I[live])  # member of every fine solve
+            tt = torch.from_numpy(np.concatenate([t_members[fm, fs], t_members[fm, fs + 1]])).to(dev)
             nf = fr.size
             buf = torch.empty((2, nf, n), **f64)
             h.copy_rows(st['u_cur'], idx[:nf], buf[0], None, nf, n, stream)
@@ -205,11 +248,12 @@ class PararealEnsemble:
             if n_sweep > 0:
                 sw = live[:n_sweep]
                 mdl0 = models[sw[0]]
-                m = mdl0.neighbours(k)
-                if m > MAX_NEIGHBOURS:
+                m_pos, t_pos = sweep_tables([mdl.neighbours(k) for mdl in models], t_members, sw)
+                if m_pos.max() > MAX_NEIGHBOURS:
                     raise Exception('nn > 160 neighbours is not supported (include/nngpara.h: NNGP_MAX_NEIGHBOURS_BIG)')
+                m = int(m_pos[0])
                 short = [e for e in sw if rows[e] < m]
-                if short:
+                if short and np.all(m_pos == m):
                     raise Exception(f'members {short} hold fewer dataset rows ({rows[short].min()}) than the common m={m}: '
                                     'an ensemble needs one m per launch')
                 blocks = []
@@ -219,8 +263,8 @@ class PararealEnsemble:
                     blocks.append(mdl.draw_starts(N - I[e]))
                     mdl.train_count += (N - I[e]) * n * N_JITTER * mdl.n_restarts
                 starts = torch.from_numpy(pack_starts(blocks, I[sw], N)).to(dev)
-                h.ensemble_sweep(sysid, mG, hm, solver.Ng, t, N, sw, I[sw], m, mdl0.n_restarts, starts, mdl0.fatol,
-                                 mdl0.xatol, st['u_next'], st['uG_next'], n, stream)
+                launch_sweep(h, t_dev, sysid, mG, hm, solver.Ng, N, sw, I[sw], m_pos, t_pos, mdl0, starts, st['u_next'],
+                             st['uG_next'], n, stream)
             # parareal.py:402: one error launch over the running members and ONE device->host read
             h.rowwise_maxabs_diff(st['u_next'], st['u_cur'], n_live * (N + 1), n, err_dev, stream)
             errs = err_dev[:n_live * (N + 1)].cpu().numpy().reshape(n_live, N + 1)
@@ -255,7 +299,7 @@ class PararealEnsemble:
             timings.update(models[e].get_times())
             u = u_all[where[e]].copy()
             kk = int(last_k[e])
-            outs.append({'t': t_host, 'u': u, 'u_last': u, 'err': err[e][:, :kk + 1], 'k': kk + 1, 'timings': timings,
+            outs.append({'t': t_members[e], 'u': u, 'u_last': u, 'err': err[e][:, :kk + 1], 'k': kk + 1, 'timings': timings,
                          'debug_dict': {}, 'converged': bool(I[e] == N), 'conv_int': conv_int[e],
                          'n_rows': int(h.seg_rows(e))})
         return outs

@@ -136,6 +136,12 @@ int nngp_predict_host_block(nngp_handle_t h, const double* q, int nq, int m, lon
                             int n_restarts, const signed char* starts, double fatol, double xatol, int j0, int dl,
                             double* pred, long long* idx, double* theta_opt, double* jitter_opt,
                             double* fval_opt, int* nfev, double* fvals, double* thetas);
+/* GP inputs of host-chosen neighbour lists (the listed prep of the listed sweeps, one launch): for query q (row stride
+ * ld_q) and the m dataset rows d_rows[q, 0..m) (rows ld >= m apart; any order, repeats allowed),
+ * dist[q, a] = ||x_rows[a] - q||^2 and r2[q, a, b] = ||x_rows[a] - x_rows[b]||^2 (rows ld apart, matrices ld x ld,
+ * leading m x m block written), summed strictly left to right without FMA like nngp_knn and the fit's matrix. */
+int nngp_listed_prep(nngp_handle_t h, const double* d_q, long long ld_q, int nq, int m, const long long* d_rows, int ld,
+                     double* d_dist, double* d_r2, void* stream);
 /* objective only: nll[nq,d,nt] at theta[nq,d,nt,2], jitter10[nq,d,nt] (= 10**jitter), the
  * `log_lik` of models.py:240-252 (+inf where the reference returns inf). */
 int nngp_gp_nll(nngp_handle_t h, const long long* d_idx, int nq, int m, int nt,
@@ -181,6 +187,16 @@ int nngp_sweep_shard(nngp_handle_t h, int sys, int method_g, int h_mode, long lo
                      const double* d_t, int N, int I, int i_first, int i_count, int m, int n_restarts,
                      const signed char* d_starts, double fatol, double xatol, double* d_u_next,
                      double* d_uG_next, int d, int j0, int dl, void* stream);
+/* nngp_sweep_shard for the position-based neighbour rules of the time-aware study (nnGPara_with_time.py:27-184,
+ * models_alt.py): the m neighbours of the predict at slice i are the dataset rows rows[(i - I) m .. + m) that the host
+ * chose, not the m nearest.  rows[(N-I), m] (host, int64, every row in [0, dataset rows), 1 <= m <= 160) covers the
+ * whole sweep; a call reads the lists of its slices i_first .. i_first+i_count-1 and uploads them.  Per slice one
+ * listed-prep launch forms the distances to the query and the neighbour matrix (the bits of the strict left-to-right
+ * sums of the kNN path), then the same order and fit launches as nngp_sweep_shard. */
+int nngp_sweep_listed_shard(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g,
+                            const double* d_t, int N, int I, int i_first, int i_count, int m, const long long* rows,
+                            int n_restarts, const signed char* d_starts, double fatol, double xatol,
+                            double* d_u_next, double* d_uG_next, int d, int j0, int dl, void* stream);
 /* parareal.py:336-339: x <- u_cur[I-1:N], D <- uF[I:N+1] - uG_cur[I:N+1] appended on device. */
 int nngp_append_iteration(nngp_handle_t h, const double* d_u_cur, const double* d_uF,
                           const double* d_uG_cur, int N, int I, int d, void* stream);
@@ -234,6 +250,17 @@ int nngp_ensemble_sweep_mixed(nngp_handle_t h, int sys, int method_g, int h_mode
                               const double* d_t_pos, int N, int E, const int* members, const int* I, const int* m,
                               int n_restarts, const signed char* d_starts, double fatol, double xatol,
                               double* d_u_next, double* d_uG_next, int d, void* stream);
+/* nngp_ensemble_sweep_mixed where each position has its own neighbour rule: listed[p] != 0 (host) marks the positions
+ * whose neighbours the host chose (nngp_sweep_listed_shard); the others take the m_p nearest rows of their segment.
+ * rows (host, int64): for every listed position in position order, its lists of slices I_p .. N-1, [(N - I_p), m_p],
+ * as global rows of the store (members[p] cap + the member's row, inside its held rows).  Per slice at most one
+ * listed-prep launch (which also gathers the queries of the kNN positions when the slice has both kinds) and one
+ * segmented kNN over the kNN positions; the "fewer rows than the slice's largest m" refusal applies to those only.
+ * Everything is validated before anything is enqueued; each run's results equal its solo listed or kNN sweep. */
+int nngp_ensemble_sweep_listed(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g,
+                               const double* d_t_pos, int N, int E, const int* members, const int* I, const int* m,
+                               const int* listed, const long long* rows, int n_restarts, const signed char* d_starts,
+                               double fatol, double xatol, double* d_u_next, double* d_uG_next, int d, void* stream);
 /* nngp_fit_predict with one neighbour count per predict: m[nq] (host); d_idx / d_dist rows ld = max m apart, the
  * first m[q] entries of row q used; the neighbour matrix is formed at ld.  Outputs as nngp_fit_predict. */
 int nngp_fit_predict_mixed(nngp_handle_t h, const double* d_q, const long long* d_idx, const double* d_dist, int nq,

@@ -74,6 +74,11 @@ SIGNATURES = {
     "nngp_ensemble_sweep": (ci, [vp, ci, ci, ci, cll, vp, ci, ci, vp, vp, ci, ci, vp, cd, cd, vp, vp, ci, vp]),
     "nngp_ensemble_sweep_mixed": (ci, [vp, ci, ci, ci, cll, vp, ci, ci, vp, vp, vp, ci, vp, cd, cd, vp, vp, ci, vp]),
     "nngp_fit_predict_mixed": (ci, [vp, vp, vp, vp, ci, vp, ci, vp, cd, cd, vp, vp, vp, vp, vp, vp, vp, vp]),
+    "nngp_listed_prep": (ci, [vp, vp, cll, ci, ci, vp, ci, vp, vp, vp]),
+    "nngp_sweep_listed_shard": (ci, [vp, ci, ci, ci, cll, vp, ci, ci, ci, ci, ci, vp, ci, vp, cd, cd, vp, vp, ci, ci, ci,
+                                     vp]),
+    "nngp_ensemble_sweep_listed": (ci, [vp, ci, ci, ci, cll, vp, ci, ci, vp, vp, vp, vp, vp, ci, vp, cd, cd, vp, vp, ci,
+                                        vp]),
 }
 
 SYSTEM_IDS = {"FHN_ODE": 0, "Rossler": 1, "Hopf": 2, "DblPend": 3, "Brusselator": 4, "Lorenz": 5,
@@ -279,6 +284,10 @@ class Handle:
                                                    _ptr(d_pred), _ptr(d_theta), _ptr(d_jit), _ptr(d_fval),
                                                    _ptr(d_nfev), _ptr(d_fvals), _ptr(d_thetas), stream))
 
+    def listed_prep(self, d_q, ld_q, nq, m, d_rows, ld, d_dist, d_r2, stream=None):
+        self.check(self.lib.nngp_listed_prep(self.h, _ptr(d_q), int(ld_q), int(nq), int(m), _ptr(d_rows), int(ld),
+                                             _ptr(d_dist), _ptr(d_r2), stream))
+
     def gp_nll(self, d_idx, nq, m, nt, d_theta, d_jitter10, d_nll, stream=None):
         self.check(self.lib.nngp_gp_nll(self.h, _ptr(d_idx), int(nq), int(m), int(nt), _ptr(d_theta),
                                         _ptr(d_jitter10), _ptr(d_nll), stream))
@@ -299,6 +308,16 @@ class Handle:
                                              int(i_first), int(i_count), int(m), int(n_restarts), _ptr(d_starts),
                                              float(fatol), float(xatol), _ptr(d_u_next), _ptr(d_uG_next), int(d),
                                              int(j0), int(dl), stream))
+
+    def sweep_listed_shard(self, sys, method_g, h_mode, steps_g, d_t, N, I, i_first, i_count, rows, n_restarts, d_starts,
+                           fatol, xatol, d_u_next, d_uG_next, d, j0, dl, stream=None):
+        """sweep_shard with host-chosen neighbours: rows [(N-I), m] (host int64) lists the dataset rows of each slice"""
+        rows = np.ascontiguousarray(rows, dtype=np.int64)
+        assert rows.ndim == 2 and rows.shape[0] == N - I, "rows must be [(N-I), m]"
+        self.check(self.lib.nngp_sweep_listed_shard(self.h, sys, method_g, h_mode, int(steps_g), _ptr(d_t), int(N),
+                                                    int(I), int(i_first), int(i_count), rows.shape[1], _ptr(rows),
+                                                    int(n_restarts), _ptr(d_starts), float(fatol), float(xatol),
+                                                    _ptr(d_u_next), _ptr(d_uG_next), int(d), int(j0), int(dl), stream))
 
     def append_iteration(self, d_u_cur, d_uF, d_uG_cur, N, I, d, stream=None):
         self.check(self.lib.nngp_append_iteration(self.h, _ptr(d_u_cur), _ptr(d_uF), _ptr(d_uG_cur), int(N),
@@ -353,6 +372,25 @@ class Handle:
                                                       members.size, _ptr(members), _ptr(I), _ptr(m), int(n_restarts),
                                                       _ptr(d_starts), float(fatol), float(xatol), _ptr(d_u_next),
                                                       _ptr(d_uG_next), int(d), stream))
+
+    def ensemble_sweep_listed(self, sys, method_g, h_mode, steps_g, d_t_pos, N, members, I, m, listed, rows, n_restarts,
+                              d_starts, fatol, xatol, d_u_next, d_uG_next, d, stream=None):
+        """ensemble_sweep_mixed where the positions with listed[p] take the host lists rows[p] ([N - I[p], m[p]] global
+        store rows; None for the others) instead of the segmented kNN"""
+        members, I = np.ascontiguousarray(members, dtype=np.int32), np.ascontiguousarray(I, dtype=np.int32)
+        m, listed = np.ascontiguousarray(m, dtype=np.int32), np.ascontiguousarray(listed, dtype=np.int32)
+        assert m.size == members.size and listed.size == members.size and len(rows) == members.size
+        blocks = []
+        for p in range(members.size):
+            if listed[p]:
+                b = np.asarray(rows[p], dtype=np.int64).reshape(-1, int(m[p]))
+                assert b.shape[0] == N - I[p], "the lists of position p must be [N - I[p], m[p]]"
+                blocks.append(b.ravel())
+        flat = np.ascontiguousarray(np.concatenate(blocks) if blocks else np.zeros(0, np.int64))
+        self.check(self.lib.nngp_ensemble_sweep_listed(self.h, sys, method_g, h_mode, int(steps_g), _ptr(d_t_pos), int(N),
+                                                       members.size, _ptr(members), _ptr(I), _ptr(m), _ptr(listed),
+                                                       _ptr(flat), int(n_restarts), _ptr(d_starts), float(fatol),
+                                                       float(xatol), _ptr(d_u_next), _ptr(d_uG_next), int(d), stream))
 
     def selftest_math(self, d_x, n, d_exp, d_rcp, d_exp10=None, stream=None):
         self.check(self.lib.nngp_selftest_math(self.h, _ptr(d_x), int(n), _ptr(d_exp), _ptr(d_rcp),

@@ -668,6 +668,24 @@ int nngp_fit_predict(nngp_handle_t h, const double* d_q, const long long* d_idx,
                                d_fvals, d_thetas, st);
 }
 
+int nngp_listed_prep(nngp_handle_t h, const double* d_q, long long ld_q, int nq, int m, const long long* d_rows, int ld,
+                     double* d_dist, double* d_r2, void* stream) {
+  NNGP_USE_DEVICE(h);
+  if (nq <= 0) return 0;
+  if (!h->ds_x) return nngp_fail(h, "listed_prep: dataset is empty");
+  if (m < 1 || m > NNGP_MAX_NEIGHBOURS_BIG || ld < m)
+    return nngp_fail(h, "listed_prep: m=%d outside [1,%d] or ld=%d < m", m, NNGP_MAX_NEIGHBOURS_BIG, ld);
+  if (ld_q < h->ds_d) return nngp_fail(h, "listed_prep: ld_q=%lld < d=%d", ld_q, h->ds_d);
+  std::vector<ListedQuery> lq(nq);
+  for (int q = 0; q < nq; q++)
+    lq[q] = ListedQuery{d_q + q * ld_q, d_rows + (size_t)q * ld, nullptr, d_dist + (size_t)q * ld,
+                        d_r2 + (size_t)q * ld * ld, nullptr, m, ld};
+  cudaStream_t st = as_stream(stream);
+  const ListedQuery* dlq = (const ListedQuery*)upload_table(h, 4, lq.data(), sizeof(ListedQuery) * lq.size(), st);
+  if (!dlq) return nngp_fail(h, "listed_prep: out of memory for the query table");
+  return listed_prep_launch(h, dlq, nq, st);
+}
+
 int nngp_gp_nll(nngp_handle_t h, const long long* d_idx, int nq, int m, int nt,
                 const double* d_theta, const double* d_jitter10, double* d_nll, void* stream) {
   NNGP_USE_DEVICE(h);
@@ -788,10 +806,12 @@ int nngp_sweep(nngp_handle_t h, int sys, int method_g, int h_mode, long long ste
 // I+1, ... in order): G and the neighbour search in full, the d*9*R searches only for the output dimensions
 // [j0, j0+dl), and u_next[i+1] written for those dimensions only.  A block dl < d sweeps one slice per call: the
 // caller all-gathers row i+1 before the neighbour search of slice i+1 reads it.
-int nngp_sweep_shard(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g,
-                     const double* d_t, int N, int I, int i_first, int i_count, int m, int n_restarts,
-                     const signed char* d_starts, double fatol, double xatol, double* d_u_next,
-                     double* d_uG_next, int d, int j0, int dl, void* stream) {
+// rows == nullptr: the neighbours are the m nearest dataset rows (nngp_sweep_shard); otherwise rows[(N-I), m] (host)
+// lists them per slice and one listed-prep launch replaces the kNN (nngp_sweep_listed_shard).
+static int sweep_shard_impl(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g, const double* d_t,
+                            int N, int I, int i_first, int i_count, int m, const long long* rows, int n_restarts,
+                            const signed char* d_starts, double fatol, double xatol, double* d_u_next,
+                            double* d_uG_next, int d, int j0, int dl, void* stream) {
   NNGP_USE_DEVICE(h);
   const SystemDesc* s;
   if (int rc = get_sys(h, sys, &s)) return rc;
@@ -806,10 +826,24 @@ int nngp_sweep_shard(nngp_handle_t h, int sys, int method_g, int h_mode, long lo
   if (n_restarts < 1) return nngp_fail(h, "sweep: n_restarts=%d < 1", n_restarts);
   cudaStream_t st = as_stream(stream);
   const long long n = h->ds_rows;
+  const ListedQuery* dlq = nullptr;
+  const long long* drows = nullptr;
+  if (rows) {
+    if (m < 1 || m > NNGP_MAX_NEIGHBOURS_BIG)
+      return nngp_fail(h, "sweep_listed: m=%d outside [1,%d]", m, NNGP_MAX_NEIGHBOURS_BIG);
+    const long long* used = rows + (size_t)(i_first - I) * m;
+    for (size_t a = 0; a < (size_t)i_count * m; a++)
+      if (used[a] < 0 || used[a] >= n)
+        return nngp_fail(h, "sweep_listed: slice %d lists row %lld, outside the dataset's %lld rows",
+                         i_first + (int)(a / m), used[a], n);
+    if (i_count > 0 &&
+        !(drows = (const long long*)upload_table(h, 3, used, sizeof(long long) * (size_t)i_count * m, st)))
+      return nngp_fail(h, "sweep_listed: out of memory for the neighbour lists");
+  }
   const int nruns = NNGP_N_JITTER * n_restarts;
   const int seg_len = dl * nruns;
   const size_t per_predict = (size_t)d * nruns * 2;
-  const size_t bk = Carver::pad(knn_workspace_bytes(1, n, m));
+  const size_t bk = rows ? 0 : Carver::pad(knn_workspace_bytes(1, n, m));
   const size_t bf = Carver::pad(gp_fit_ws_bytes(1, d, m, n_restarts));
   const size_t bi = Carver::pad(sizeof(long long) * m), bd = Carver::pad(sizeof(double) * m);
   const size_t bo = Carver::pad(sizeof(int) * (size_t)seg_len * (size_t)i_count);
@@ -820,6 +854,14 @@ int nngp_sweep_shard(nngp_handle_t h, int sys, int method_g, int h_mode, long lo
   long long* idx = (long long*)(ws + bk + bf);
   double* dist = (double*)(ws + bk + bf + bi);
   int* order = (int*)(ws + bk + bf + bi + bd);
+  if (drows) {
+    std::vector<ListedQuery> lq(i_count);
+    for (int c = 0; c < i_count; c++)
+      lq[c] = ListedQuery{d_u_next + (long long)(i_first + c) * d, drows + (size_t)c * m, nullptr, dist, (double*)fws,
+                          nullptr, m, m};
+    if (!(dlq = (const ListedQuery*)upload_table(h, 4, lq.data(), sizeof(ListedQuery) * lq.size(), st)))
+      return nngp_fail(h, "sweep_listed: out of memory for the query table");
+  }
   if (int rc = ensure_done_zero(h, fws, 1, d, m, n_restarts, st)) return rc;
   // queue order of every predict of the call in one launch (the starts are all known up front); with dl = d the
   // blocks of consecutive predicts are contiguous, with dl < d there is one
@@ -830,15 +872,34 @@ int nngp_sweep_shard(nngp_handle_t h, int sys, int method_g, int h_mode, long lo
     double* un = d_u_next + (long long)(i + 1) * d;
     double* gn = d_uG_next + (long long)(i + 1) * d;
     if (int rc = sweep_slice_prologue(h, *s, method_g, h_mode, steps_g, 1, d_t + i, d_t + i + 1, ui, d, gn, st, [&] {
+          if (dlq) return listed_prep_launch(h, dlq + (i - i_first), 1, st);
           return knn_prep_launch(h, ui, 1, m, n, idx, dist, kws, fws, st);
         }))
       return rc;
-    if (int rc = gp_fit_predict_launch(h, idx, dist, fws, next_queue(h, st), order + (size_t)(i - i_first) * seg_len, 1, m,
+    const long long* nb = drows ? drows + (size_t)(i - i_first) * m : idx;
+    if (int rc = gp_fit_predict_launch(h, nb, dist, fws, next_queue(h, st), order + (size_t)(i - i_first) * seg_len, 1, m,
                                        n_restarts, starts_first + (size_t)(i - i_first) * per_predict, fatol, xatol, un,
                                        gn, d, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, st, j0, dl))
       return rc;
   }
   return 0;
+}
+
+int nngp_sweep_shard(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g,
+                     const double* d_t, int N, int I, int i_first, int i_count, int m, int n_restarts,
+                     const signed char* d_starts, double fatol, double xatol, double* d_u_next,
+                     double* d_uG_next, int d, int j0, int dl, void* stream) {
+  return sweep_shard_impl(h, sys, method_g, h_mode, steps_g, d_t, N, I, i_first, i_count, m, nullptr, n_restarts,
+                          d_starts, fatol, xatol, d_u_next, d_uG_next, d, j0, dl, stream);
+}
+
+int nngp_sweep_listed_shard(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g,
+                            const double* d_t, int N, int I, int i_first, int i_count, int m, const long long* rows,
+                            int n_restarts, const signed char* d_starts, double fatol, double xatol,
+                            double* d_u_next, double* d_uG_next, int d, int j0, int dl, void* stream) {
+  if (rows == nullptr) return nngp_fail(h, "sweep_listed: rows is NULL");
+  return sweep_shard_impl(h, sys, method_g, h_mode, steps_g, d_t, N, I, i_first, i_count, m, rows, n_restarts,
+                          d_starts, fatol, xatol, d_u_next, d_uG_next, d, j0, dl, stream);
 }
 
 // ---- ensembles: segmented store, segmented kNN, ensemble sweep -------------------------
@@ -1107,17 +1168,20 @@ static int mixed_fit_group(nngp_handle_t h, MixedGroups& G, int g, int n, int d,
                                D.fvals, D.thetas, st);
 }
 
-// The copies that hand predict p (rank r of group g) its inputs: the first m_g neighbours of its row of the kNN at
-// row stride mm, the leading m_g x m_g block of its mm x mm neighbour matrix, its starts and (optional) added term.
-static void mixed_gather_spans(std::vector<CopySpan>& sp, MixedGroups& G, int p, const long long* idx,
+// The copies that hand predict p (rank r of group g) its inputs: the first m_g neighbours of row `src` of the kNN at
+// row stride mm, the leading m_g x m_g block of its mm x mm neighbour matrix (idx == nullptr: these three are already
+// in place, written by the listed prep), its starts and (optional) added term.
+static void mixed_gather_spans(std::vector<CopySpan>& sp, MixedGroups& G, int p, int src, const long long* idx,
                                const double* dist, const double* r2, int mm, const signed char* starts, size_t per_predict,
                                const double* add, long long ld_add, int d) {
   const int g = G.grp[p], r = G.rank[p], mg = G.m[g];
   const MixedGroups::Dev& D = G.dev[g];
-  sp.push_back(copy_span(idx + (size_t)p * mm, D.idx + (size_t)r * mg, sizeof(long long) * mg));
-  sp.push_back(copy_span(dist + (size_t)p * mm, D.dist + (size_t)r * mg, sizeof(double) * mg));
-  sp.push_back(copy_span(r2 + (size_t)p * mm * mm, D.fws + sizeof(double) * (size_t)r * mg * mg, sizeof(double) * mg, mg,
-                    (long long)sizeof(double) * mm, (long long)sizeof(double) * mg));
+  if (idx) {
+    sp.push_back(copy_span(idx + (size_t)src * mm, D.idx + (size_t)r * mg, sizeof(long long) * mg));
+    sp.push_back(copy_span(dist + (size_t)src * mm, D.dist + (size_t)r * mg, sizeof(double) * mg));
+    sp.push_back(copy_span(r2 + (size_t)src * mm * mm, D.fws + sizeof(double) * (size_t)r * mg * mg, sizeof(double) * mg,
+                           mg, (long long)sizeof(double) * mm, (long long)sizeof(double) * mg));
+  }
   sp.push_back(copy_span(starts + (size_t)p * per_predict, D.starts + (size_t)r * per_predict, per_predict));
   if (add) sp.push_back(copy_span(add + (size_t)p * ld_add, D.add + (size_t)r * d, sizeof(double) * d));
 }
@@ -1145,7 +1209,7 @@ int nngp_fit_predict_mixed(nngp_handle_t h, const double* d_q, const long long* 
   G.carve(ws + br, d, R, true);
   double* r2 = (double*)ws;
   std::vector<CopySpan> sp;
-  for (int q = 0; q < nq; q++) mixed_gather_spans(sp, G, q, d_idx, d_dist, r2, ld, d_starts, per_predict, nullptr, 0, d);
+  for (int q = 0; q < nq; q++) mixed_gather_spans(sp, G, q, q, d_idx, d_dist, r2, ld, d_starts, per_predict, nullptr, 0, d);
   const size_t n_gather = sp.size();
   const size_t nd = sizeof(double) * d, nt = (size_t)seg_len;
   for (int q = 0; q < nq; q++) {
@@ -1169,12 +1233,14 @@ int nngp_fit_predict_mixed(nngp_handle_t h, const double* d_q, const long long* 
   return copy_spans_launch(h, dsp + n_gather, (int)(sp.size() - n_gather), st);
 }
 
-// nngp_ensemble_sweep (m_pos == nullptr: one m and the shared grid d_t) and nngp_ensemble_sweep_mixed (m_pos[E] and
-// the per-position grids d_t_pos[E, N+1]).
+// nngp_ensemble_sweep (m_pos == nullptr: one m and the shared grid d_t), nngp_ensemble_sweep_mixed (m_pos[E] and
+// the per-position grids d_t_pos[E, N+1]) and nngp_ensemble_sweep_listed (the mixed sweep where the positions with
+// listed[p] != 0 take their neighbours from the host lists `rows` instead of the segmented kNN).
 static int ensemble_sweep_impl(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g, const double* d_t,
                                const double* d_t_pos, int N, int E, const int* members, const int* I, int m,
-                               const int* m_pos, int n_restarts, const signed char* d_starts, double fatol,
-                               double xatol, double* d_u_next, double* d_uG_next, int d, void* stream) {
+                               const int* m_pos, const int* listed, const long long* rows, int n_restarts,
+                               const signed char* d_starts, double fatol, double xatol, double* d_u_next,
+                               double* d_uG_next, int d, void* stream) {
   NNGP_USE_DEVICE(h);
   const SystemDesc* s;
   if (int rc = get_sys(h, sys, &s)) return rc;
@@ -1204,18 +1270,46 @@ static int ensemble_sweep_impl(nngp_handle_t h, int sys, int method_g, int h_mod
     tab[p] = (long long)e * h->seg_cap;
     tab[E + p] = h->seg_rows[e];
   }
+  // the kNN positions (all of them without `listed`) in position order, and their segment table: the kNN of a slice
+  // runs over the active ones, a prefix of them
+  auto is_listed = [&](int p) { return listed != nullptr && listed[p] != 0; };
+  std::vector<int> kpos;
+  for (int p = 0; p < E; p++)
+    if (!is_listed(p)) kpos.push_back(p);
+  const int nk = (int)kpos.size();
+  std::vector<long long> ktab(2 * (size_t)nk);
+  for (int r = 0; r < nk; r++) {
+    ktab[r] = tab[kpos[r]];
+    ktab[nk + r] = tab[E + kpos[r]];
+  }
+  // listed positions: block [(N - I_p), m_p] of `rows` in position order, every row inside the member's segment
+  std::vector<size_t> row_at(E, 0);
+  size_t n_listed_rows = 0;
+  for (int p = 0; p < E; p++) {
+    if (!is_listed(p)) continue;
+    row_at[p] = n_listed_rows;
+    const size_t cnt = (size_t)(N - I[p]) * m_pos[p];
+    if (cnt > 0 && rows == nullptr) return nngp_fail(h, "ensemble_sweep_listed: rows is NULL");
+    for (size_t a = 0; a < cnt; a++) {
+      const long long r = rows[n_listed_rows + a];
+      if (r < tab[p] || r >= tab[p] + tab[E + p])
+        return nngp_fail(h, "ensemble_sweep_listed: member %d, slice %d lists row %lld, outside its segment [%lld,%lld)",
+                         members[p], I[p] + (int)(a / m_pos[p]), r, tab[p], tab[p] + tab[E + p]);
+    }
+    n_listed_rows += cnt;
+  }
   if (I[0] >= N) return 0;
   if (mixed) {
-    // each slice searches its runs' neighbours at the largest m among them: a run whose segment is shorter would
+    // each slice searches its kNN runs' neighbours at the largest m among them: a run whose segment is shorter would
     // read padding indices as rows.  Refused before anything is enqueued.
     int n_act = 0, mm = 0, short_p = -1;
     for (int i = I[0]; i < N; i++) {
-      while (n_act < E && I[n_act] <= i) {
+      for (; n_act < E && I[n_act] <= i; n_act++) {
+        if (is_listed(n_act)) continue;
         mm = std::max(mm, m_pos[n_act]);
         if (short_p < 0 || tab[E + n_act] < tab[E + short_p]) short_p = n_act;
-        n_act++;
       }
-      if (tab[E + short_p] < mm)
+      if (short_p >= 0 && tab[E + short_p] < mm)
         return nngp_fail(h, "ensemble_sweep: member %d holds %lld rows, fewer than m=%d, the largest m of slice %d",
                          members[short_p], tab[E + short_p], mm, i);
     }
@@ -1236,17 +1330,24 @@ static int ensemble_sweep_impl(nngp_handle_t h, int sys, int method_g, int h_mod
   const size_t bi = Carver::pad(sizeof(long long) * (size_t)E * m), bd = Carver::pad(sizeof(double) * (size_t)E * m);
   const size_t bo = Carver::pad(sizeof(int) * (size_t)E * seg_len);
   const size_t bt = Carver::pad(sizeof(double) * (size_t)(N + 1) * E);
-  char* ws = (char*)nngp_workspace(h, bk + bf + bi + bd + bo + bt);
+  const size_t bq = listed ? Carver::pad(sizeof(double) * (size_t)nk * d) : 0;  // gathered kNN queries
+  char* ws = (char*)nngp_workspace(h, bk + bf + bi + bd + bo + bt + bq);
   unsigned int* tickets = seg_tickets(h, E);
   if (!ws || !tickets) return nngp_fail(h, "ensemble_sweep: out of device memory");
-  const long long* dtab = (const long long*)upload_table(h, 1, tab.data(), sizeof(long long) * tab.size(), st);
-  if (!dtab) return nngp_fail(h, "ensemble_sweep: out of memory for the segment table");
+  const long long* dtab = nullptr;
+  if (nk > 0 && !(dtab = (const long long*)upload_table(h, 1, ktab.data(), sizeof(long long) * ktab.size(), st)))
+    return nngp_fail(h, "ensemble_sweep: out of memory for the segment table");
+  const long long* drows = nullptr;
+  if (n_listed_rows > 0 &&
+      !(drows = (const long long*)upload_table(h, 3, rows, sizeof(long long) * n_listed_rows, st)))
+    return nngp_fail(h, "ensemble_sweep_listed: out of memory for the neighbour lists");
   void* kws = ws;
   void* fws = ws + bk;
   long long* idx = (long long*)(ws + bk + bf);
   double* dist = (double*)(ws + bk + bf + bi);
   int* order = (int*)(ws + bk + bf + bi + bd);
   double* t_rep = (double*)(ws + bk + bf + bi + bd + bo);
+  double* q_knn = (double*)(ws + bk + bf + bi + bd + bo + bt);
   {
     const long long tot = (long long)(N + 1) * E;
     if (d_t_pos)
@@ -1256,40 +1357,65 @@ static int ensemble_sweep_impl(nngp_handle_t h, int sys, int method_g, int h_mod
     h->launches++;
     NNGP_CUDA(h, cudaGetLastError());
   }
-  // mixed: every slice's gather and scatter copies, in one table for the whole sweep
+  // mixed: every slice's gather and scatter copies, in one table for the whole sweep; listed: every slice's listed
+  // preps, which write straight into their fit groups' inputs, and the gathers of the kNN queries when the slice has
+  // listed positions (its kNN positions are then no prefix of the state)
   std::vector<CopySpan> sp;
   std::vector<size_t> sp_at;  // per slice: start of its gather spans, start of its scatter spans
+  std::vector<ListedQuery> lq;
+  std::vector<size_t> lq_at;  // per slice: start of its listed preps
   if (mixed) {
     G.carve((char*)fws + Carver::pad(gp_prep_bytes(E, m)), d, n_restarts, false);
     size_t done_predicts = 0;
-    int n_act = 0, mm = 0;
+    int n_act = 0, nk_act = 0, mm = 0;
     for (int i = I[0]; i < N; i++) {
-      while (n_act < E && I[n_act] <= i) mm = std::max(mm, m_pos[n_act++]);
+      for (; n_act < E && I[n_act] <= i; n_act++)
+        if (!is_listed(n_act)) mm = std::max(mm, m_pos[n_act]), nk_act++;
       const signed char* starts_i = d_starts + done_predicts * per_predict;
+      const double* ui = d_u_next + (long long)i * d;
       const double* gn = d_uG_next + (long long)(i + 1) * d;
       double* un = d_u_next + (long long)(i + 1) * d;
       sp_at.push_back(sp.size());
-      for (int p = 0; p < n_act; p++)
-        mixed_gather_spans(sp, G, p, idx, dist, (const double*)fws, mm, starts_i, per_predict, gn, ld, d);
+      lq_at.push_back(lq.size());
+      for (int p = 0, rk = 0; p < n_act; p++) {
+        if (!is_listed(p)) {
+          mixed_gather_spans(sp, G, p, rk++, idx, dist, (const double*)fws, mm, starts_i, per_predict, gn, ld, d);
+          continue;
+        }
+        const int r = G.rank[p], mg = G.m[G.grp[p]];
+        const MixedGroups::Dev& D = G.dev[G.grp[p]];
+        lq.push_back(ListedQuery{ui + p * ld, drows + row_at[p] + (size_t)(i - I[p]) * mg, D.idx + (size_t)r * mg,
+                                 D.dist + (size_t)r * mg, (double*)D.fws + (size_t)r * mg * mg, nullptr, mg, mg});
+        mixed_gather_spans(sp, G, p, 0, nullptr, nullptr, nullptr, 0, starts_i, per_predict, gn, ld, d);
+      }
+      if (lq.size() > lq_at.back())
+        for (int r = 0; r < nk_act; r++)
+          lq.push_back(ListedQuery{ui + kpos[r] * ld, nullptr, nullptr, nullptr, nullptr, q_knn + (size_t)r * d, 0, 0});
       sp_at.push_back(sp.size());
       for (int p = 0; p < n_act; p++)
         sp.push_back(copy_span(G.dev[G.grp[p]].pred + (size_t)G.rank[p] * d, un + (size_t)p * ld, sizeof(double) * d));
       done_predicts += n_act;
     }
     sp_at.push_back(sp.size());
+    lq_at.push_back(lq.size());
   }
   const CopySpan* dsp = nullptr;
   if (mixed && !(dsp = (const CopySpan*)upload_table(h, 2, sp.data(), sizeof(CopySpan) * sp.size(), st)))
     return nngp_fail(h, "ensemble_sweep: out of memory for the copy table");
+  const ListedQuery* dlq = nullptr;
+  if (!lq.empty() && !(dlq = (const ListedQuery*)upload_table(h, 4, lq.data(), sizeof(ListedQuery) * lq.size(), st)))
+    return nngp_fail(h, "ensemble_sweep_listed: out of memory for the query table");
   // The members active at slice i (I <= i) are a prefix of the positions: every launch below reaches them with the
   // member stride (N+1) d of the state, and their predicts' starts are consecutive in d_starts (slice-major).
   size_t done_predicts = 0;
-  int n_act = 0, mm = 0;
+  int n_act = 0, nk_act = 0, mm = 0;
   long long n_max = 0;
   for (int i = I[0]; i < N; i++) {
-    while (n_act < E && I[n_act] <= i) {
+    for (; n_act < E && I[n_act] <= i; n_act++) {
+      if (is_listed(n_act)) continue;
       if (mixed) mm = std::max(mm, m_pos[n_act]);
-      n_max = std::max(n_max, tab[E + n_act++]);
+      n_max = std::max(n_max, tab[E + n_act]);
+      nk_act++;
     }
     const signed char* starts_i = d_starts + done_predicts * per_predict;
     double* ui = d_u_next + (long long)i * d;
@@ -1297,9 +1423,13 @@ static int ensemble_sweep_impl(nngp_handle_t h, int sys, int method_g, int h_mod
     double* gn = d_uG_next + (long long)(i + 1) * d;
     if (mixed) {
       const size_t* at = sp_at.data() + 2 * (size_t)(i - I[0]);
+      const size_t l0 = lq_at[i - I[0]], nl = lq_at[i - I[0] + 1] - l0;
       if (int rc = sweep_slice_prologue(h, *s, method_g, h_mode, steps_g, n_act, t_rep + (size_t)i * E,
                                         t_rep + (size_t)(i + 1) * E, ui, ld, gn, st, [&] {
-            return knn_seg_launch(h, ui, ld, n_act, mm, dtab, dtab + E, n_max, idx, dist, (double*)fws, tickets, kws, st);
+            if (int rc = listed_prep_launch(h, dlq + l0, (int)nl, st)) return rc;
+            if (nk_act == 0) return 0;
+            return knn_seg_launch(h, nl ? q_knn : ui, nl ? d : ld, nk_act, mm, dtab, dtab + nk, n_max, idx, dist,
+                                  (double*)fws, tickets, kws, st);
           }))
         return rc;
       if (int rc = copy_spans_launch(h, dsp + at[0], (int)(at[1] - at[0]), st)) return rc;
@@ -1316,7 +1446,7 @@ static int ensemble_sweep_impl(nngp_handle_t h, int sys, int method_g, int h_mod
     if (int rc = gp_order_launch(h, starts_i, n_act, seg_len, 1, order, st)) return rc;
     if (int rc = sweep_slice_prologue(h, *s, method_g, h_mode, steps_g, n_act, t_rep + (size_t)i * E,
                                       t_rep + (size_t)(i + 1) * E, ui, ld, gn, st, [&] {
-          return knn_seg_launch(h, ui, ld, n_act, m, dtab, dtab + E, n_max, idx, dist, (double*)fws, tickets, kws, st);
+          return knn_seg_launch(h, ui, ld, n_act, m, dtab, dtab + nk, n_max, idx, dist, (double*)fws, tickets, kws, st);
         }))
       return rc;
     if (int rc = gp_fit_predict_launch(h, idx, dist, fws, next_queue(h, st), order, n_act, m, n_restarts, starts_i, fatol,
@@ -1330,8 +1460,8 @@ static int ensemble_sweep_impl(nngp_handle_t h, int sys, int method_g, int h_mod
 int nngp_ensemble_sweep(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g, const double* d_t, int N,
                         int E, const int* members, const int* I, int m, int n_restarts, const signed char* d_starts,
                         double fatol, double xatol, double* d_u_next, double* d_uG_next, int d, void* stream) {
-  return ensemble_sweep_impl(h, sys, method_g, h_mode, steps_g, d_t, nullptr, N, E, members, I, m, nullptr, n_restarts,
-                             d_starts, fatol, xatol, d_u_next, d_uG_next, d, stream);
+  return ensemble_sweep_impl(h, sys, method_g, h_mode, steps_g, d_t, nullptr, N, E, members, I, m, nullptr, nullptr,
+                             nullptr, n_restarts, d_starts, fatol, xatol, d_u_next, d_uG_next, d, stream);
 }
 
 int nngp_ensemble_sweep_mixed(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g,
@@ -1339,8 +1469,18 @@ int nngp_ensemble_sweep_mixed(nngp_handle_t h, int sys, int method_g, int h_mode
                               int n_restarts, const signed char* d_starts, double fatol, double xatol,
                               double* d_u_next, double* d_uG_next, int d, void* stream) {
   if (m == nullptr || d_t_pos == nullptr) return nngp_fail(h, "ensemble_sweep_mixed: m and d_t_pos are required");
-  return ensemble_sweep_impl(h, sys, method_g, h_mode, steps_g, nullptr, d_t_pos, N, E, members, I, 0, m, n_restarts,
-                             d_starts, fatol, xatol, d_u_next, d_uG_next, d, stream);
+  return ensemble_sweep_impl(h, sys, method_g, h_mode, steps_g, nullptr, d_t_pos, N, E, members, I, 0, m, nullptr,
+                             nullptr, n_restarts, d_starts, fatol, xatol, d_u_next, d_uG_next, d, stream);
+}
+
+int nngp_ensemble_sweep_listed(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g,
+                               const double* d_t_pos, int N, int E, const int* members, const int* I, const int* m,
+                               const int* listed, const long long* rows, int n_restarts, const signed char* d_starts,
+                               double fatol, double xatol, double* d_u_next, double* d_uG_next, int d, void* stream) {
+  if (m == nullptr || d_t_pos == nullptr || listed == nullptr)
+    return nngp_fail(h, "ensemble_sweep_listed: m, listed and d_t_pos are required");
+  return ensemble_sweep_impl(h, sys, method_g, h_mode, steps_g, nullptr, d_t_pos, N, E, members, I, 0, m, listed, rows,
+                             n_restarts, d_starts, fatol, xatol, d_u_next, d_uG_next, d, stream);
 }
 
 int nngp_selftest_math(nngp_handle_t h, const double* d_x, int n, double* d_exp_neg, double* d_rcp,

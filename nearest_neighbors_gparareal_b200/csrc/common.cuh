@@ -92,7 +92,9 @@ struct nngp_handle_s {
   // small host->device tables of the segmented entry points: pinned staging, re-used once the copy that last read it
   // has completed (event)
   struct Upload { void* host = nullptr; void* dev = nullptr; size_t bytes = 0; cudaEvent_t done = nullptr; };
-  Upload up[3];  // 0 row tables, 1 segment tables, 2 copy spans of the mixed ensemble sweep
+  // 0 row tables, 1 segment tables, 2 copy spans of the mixed ensemble sweep, 3 neighbour lists and 4 ListedQuery
+  // tables of the listed sweeps
+  Upload up[5];
   // device counters: [0] Nelder-Mead runs, [1] objective (nll) evaluations
   unsigned long long* d_counters = nullptr;
   // task-queue heads of the persistent fit kernel: one zeroed counter per launch
@@ -161,12 +163,27 @@ int copy_rows_launch(nngp_handle_t h, const double* src, const long long* si, do
 int rowwise_maxabs_launch(nngp_handle_t h, const double* a, const double* b, int rows, int d,
                           double* err, cudaStream_t st);
 
+// One predict of a listed sweep (nngp_sweep_listed_shard, nngp_ensemble_sweep_listed): the GP inputs of query q from
+// the m dataset rows a neighbour rule chose on the host, instead of from a kNN.  m == 0: the entry only copies the
+// query row to q_copy (the queries of the nearest-neighbour positions of a mixed slice, gathered to one row stride for
+// the segmented kNN that follows).  All pointers are device pointers.
+struct ListedQuery {
+  const double* q;        // the query, d doubles
+  const long long* rows;  // its m dataset rows, in the rule's order
+  long long* idx;         // the rows are copied here (nullptr: the fit reads `rows` itself)
+  double* dist;           // dist[a] = ||x_rows[a] - q||^2
+  double* r2;             // r2[a ld + b] = ||x_rows[a] - x_rows[b]||^2 for a, b < m
+  double* q_copy;
+  int m, ld;
+};
+
 // gpfit.cu
 size_t gp_prep_bytes(int nq, int m);
 size_t gp_fit_ws_bytes(int nq, int d, int m, int R);      // [r2 | per-search results | done counters]
 size_t gp_fit_done_offset(int nq, int d, int m, int R);   // byte offset of the done counters
 int gp_prep_launch(nngp_handle_t h, const long long* d_idx, int nq, int m, double* d_r2,
                    cudaStream_t st);
+int listed_prep_launch(nngp_handle_t h, const ListedQuery* d_lq, int n, cudaStream_t st);
 int gp_order_launch(nngp_handle_t h, const signed char* d_starts, int nseg, int seg_len, int global_ids,
                     int* d_order, cudaStream_t st);
 int gp_fit_predict_launch(nngp_handle_t h, const long long* d_idx, const double* d_dist, void* ws,

@@ -1368,6 +1368,99 @@ gp_prep_kernel(const long long* __restrict__ idx, const double* __restrict__ X, 
   }
 }
 
+// The GP inputs of host-chosen neighbour lists (position-based rules, models_alt.py), one CTA per ListedQuery:
+// distances to the query and the neighbour matrix, both summed strictly left to right without FMA, so dist has the
+// bits of NumPy's `dist + diff * diff` and r2 those of gp_prep_kernel / gp_prep_big_kernel on the same list.  m <= 32
+// stages the listed rows and the query through shared memory in column chunks (gp_prep_kernel's pair mapping);
+// larger m reads them from global memory, one thread per distance or pair (gp_prep_big_kernel's).
+__global__ void __launch_bounds__(256)
+listed_prep_kernel(const ListedQuery* __restrict__ lq, const double* __restrict__ X, int d) {
+  constexpr int JC = 64;
+  __shared__ double tile[NNGP_MAX_NEIGHBOURS][JC + 1];
+  __shared__ double qt[JC];
+  const ListedQuery L = lq[blockIdx.x];
+  const int m = L.m, ld = L.ld, npairs = m * (m + 1) / 2;
+  if (m == 0) {
+    for (int j = threadIdx.x; j < d; j += 256) L.q_copy[j] = L.q[j];
+    return;
+  }
+  if (L.idx)
+    for (int a = threadIdx.x; a < m; a += 256) L.idx[a] = L.rows[a];
+  auto pair_of = [](int pidx, int& a, int& b) {
+    a = (int)((sqrt(8.0 * pidx + 1.0) - 1.0) * 0.5);
+    while ((a + 1) * (a + 2) / 2 <= pidx) a++;
+    while (a * (a + 1) / 2 > pidx) a--;
+    b = pidx - a * (a + 1) / 2;
+  };
+  if (m > NNGP_MAX_NEIGHBOURS) {
+    for (int a = threadIdx.x; a < m; a += 256) {
+      const double* xa = X + L.rows[a] * d;
+      double s = 0.0;
+      for (int j = 0; j < d; j++) {
+        const double diff = __dsub_rn(xa[j], L.q[j]);
+        s = __dadd_rn(s, __dmul_rn(diff, diff));
+      }
+      L.dist[a] = s;
+    }
+    for (int pidx = threadIdx.x; pidx < npairs; pidx += 256) {
+      int a, b;
+      pair_of(pidx, a, b);
+      const double* xa = X + L.rows[a] * d;
+      const double* xb = X + L.rows[b] * d;
+      double s = 0.0;
+      for (int j = 0; j < d; j++) {
+        const double diff = __dsub_rn(xa[j], xb[j]);
+        s = __dadd_rn(s, __dmul_rn(diff, diff));
+      }
+      L.r2[(long long)a * ld + b] = s;
+      L.r2[(long long)b * ld + a] = s;
+    }
+    return;
+  }
+  int pa[3], pb[3];
+  double acc[3] = {0.0, 0.0, 0.0}, dq = 0.0;
+#pragma unroll
+  for (int u = 0; u < 3; u++) {
+    pa[u] = pb[u] = 0;
+    if (threadIdx.x + u * 256 < npairs) pair_of(threadIdx.x + u * 256, pa[u], pb[u]);
+  }
+  for (int j0 = 0; j0 < d; j0 += JC) {
+    const int jn = min(JC, d - j0);
+    __syncthreads();
+    for (int e = threadIdx.x; e < m * JC; e += 256) {
+      const int r = e / JC, jj = e - r * JC;
+      if (jj < jn) tile[r][jj] = X[L.rows[r] * d + j0 + jj];
+    }
+    if (threadIdx.x < jn) qt[threadIdx.x] = L.q[j0 + threadIdx.x];
+    __syncthreads();
+#pragma unroll
+    for (int u = 0; u < 3; u++) {
+      if (threadIdx.x + u * 256 < npairs) {
+        double s = acc[u];
+        for (int jj = 0; jj < jn; jj++) {
+          const double diff = __dsub_rn(tile[pa[u]][jj], tile[pb[u]][jj]);
+          s = __dadd_rn(s, __dmul_rn(diff, diff));
+        }
+        acc[u] = s;
+      }
+    }
+    if (threadIdx.x < m) {
+      for (int jj = 0; jj < jn; jj++) {
+        const double diff = __dsub_rn(tile[threadIdx.x][jj], qt[jj]);
+        dq = __dadd_rn(dq, __dmul_rn(diff, diff));
+      }
+    }
+  }
+#pragma unroll
+  for (int u = 0; u < 3; u++) {
+    if (threadIdx.x + u * 256 < npairs) {
+      L.r2[(long long)pa[u] * ld + pb[u]] = acc[u];
+      L.r2[(long long)pb[u] * ld + pa[u]] = acc[u];
+    }
+  }
+  if (threadIdx.x < m) L.dist[threadIdx.x] = dq;
+}
+
 // Queue order of the searches (longest first).  A search that starts at a large log-amplitude
 // sigma_y runs to the evaluation limit far more often than one that starts at a small one (measured
 // on the FHN target: >= 400 evaluations for about half of the starts with sigma_y = -1, never for
@@ -1438,6 +1531,15 @@ int gp_prep_launch(nngp_handle_t h, const long long* d_idx, int nq, int m, doubl
     return 0;
   }
   gp_prep_kernel<<<nq, 256, 0, st>>>(d_idx, h->ds_x, h->ds_d, m, d_r2);
+  h->launches++;
+  NNGP_CUDA(h, cudaGetLastError());
+  return 0;
+}
+
+int listed_prep_launch(nngp_handle_t h, const ListedQuery* d_lq, int n, cudaStream_t st) {
+  if (n <= 0) return 0;
+  ProfScope prof(h, 2, st);
+  listed_prep_kernel<<<n, 256, 0, st>>>(d_lq, h->ds_x, h->ds_d);
   h->launches++;
   NNGP_CUDA(h, cudaGetLastError());
   return 0;

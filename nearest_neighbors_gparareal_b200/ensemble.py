@@ -1,7 +1,8 @@
 """Many independent nnGParareal runs as one device-resident ensemble.
 
 `PararealEnsemble.run(seeds=[...])` runs E solves of the same system, solver, N, `n_restarts`, `fatol` and `xatol` in
-lockstep; the runs may differ in seed, initial condition, epsilon, early_stop, neighbour count `nn` and time span.  Every
+lockstep; the runs may differ in seed, initial condition, epsilon, early_stop, neighbour count `nn`, neighbour rule
+`nntype` (models_alt.py; nngp_ensemble_sweep_listed when a running member uses a position rule) and time span.  Every
 iteration makes the launches of one `PararealDevice` iteration, each over all runs at once: one fine-step launch, one
 dataset append, and per slice of the sweep one coarse step, one kNN (each run searches its own rows of a segmented
 store, csrc/knn.cu) and one fit over all the runs' predicts -- one fit per distinct neighbour count when the runs'
@@ -20,6 +21,7 @@ import numpy as np
 
 from . import _lib
 from .models import CudaNNGP, N_JITTER
+from .models_alt import NNTYPES, CudaNNGPAlt
 from .parareal import advance
 from .solver import CudaSolverRK
 from .systems import ODE
@@ -36,9 +38,10 @@ def _check_nn(nn):
         raise ValueError(f'nn={nn}: 1 to {MAX_NEIGHBOURS} neighbours are supported')
 
 
-def check_run_args(E_lists, model='nngp', store_int=False, nn='adaptive'):
+def check_run_args(E_lists, model='nngp', store_int=False, nn='adaptive', nntype='nn'):
     """Validates the per-member lists of `PararealEnsemble.run` (dict name -> list or None); returns E.
-    `nn` is one value for every member or a list with one per member; E_lists['tspans'] entries are [t0, t1] or None."""
+    `nn` and `nntype` are one value for every member or a list with one per member; E_lists['tspans'] entries are
+    [t0, t1] or None."""
     if not isinstance(model, str) or model.lower() != 'nngp':
         raise ValueError(f"PararealEnsemble runs the 'nngp' model only (got {model!r})")
     if store_int:
@@ -50,15 +53,33 @@ def check_run_args(E_lists, model='nngp', store_int=False, nn='adaptive'):
     lists = dict(E_lists)
     if isinstance(nn, (list, tuple, np.ndarray)):
         lists['nn'] = nn
+    if isinstance(nntype, (list, tuple, np.ndarray)):
+        lists['nntype'] = nntype
     for name, v in lists.items():
         if v is not None and len(v) != E:
             raise ValueError(f'{name} has {len(v)} entries, seeds has {E}: give one per member')
     for v in (nn if isinstance(nn, (list, tuple, np.ndarray)) else [nn]):
         _check_nn(v)
+    nns = list(nn) if isinstance(nn, (list, tuple, np.ndarray)) else [nn] * E
+    rules = list(nntype) if isinstance(nntype, (list, tuple, np.ndarray)) else [nntype] * E
+    for e, (rule, v) in enumerate(zip(rules, nns)):
+        if rule not in NNTYPES:
+            raise ValueError(f'member {e}: unknown nntype {rule!r} (one of {", ".join(NNTYPES)})')
+        if rule in ('row_col', 'row', 'col_full') and v == 'adaptive':
+            raise ValueError(f"member {e}: nntype {rule!r} needs an integer nn, not 'adaptive'")
     for ts in E_lists.get('tspans') or []:
         if ts is not None and not (len(ts) == 2 and float(ts[1]) > float(ts[0])):
             raise ValueError(f'tspan {list(ts)}: give [t0, t1] with t1 > t0')
     return E
+
+
+def listed_rows(mdl, e, first, I, base):
+    """Member e's neighbour lists [N - I, m] for the sweep of iteration len(first) - 1, as global store rows (base = e
+    cap): CudaNNGPAlt.neighbour_table, the rules of the member's solo run; a refusal names the member."""
+    try:
+        return mdl.neighbour_table(first, I) + base
+    except Exception as exc:
+        raise ValueError(f'member {e}: {exc}') from exc
 
 
 def sweep_tables(m_members, t_members, sw):
@@ -140,14 +161,16 @@ class PararealEnsemble:
         return self._h
 
     def run(self, model='nngp', seeds=None, nn='adaptive', n_restarts=1, fatol=None, xatol=None, epsilons=None,
-            early_stops=None, init_conds=None, tspans=None, max_rows=None, store_int=False):
+            early_stops=None, init_conds=None, tspans=None, max_rows=None, store_int=False, nntype='nn'):
         """Returns one output dict per seed (the keys of PararealDevice.run, n_rows included).
 
-        nn: 'adaptive', an int in 1..160, or a list with one of those per member.  tspans: None or a list with one
-        [t0, t1] (or None: the ensemble's tspan) per member; member e's output 't' is its own grid.  n_restarts,
-        fatol and xatol are common to all members."""
+        nn: 'adaptive', an int in 1..160, or a list with one of those per member.  nntype: the neighbour rule of
+        models_alt.py ('nn', 'col+rnd', 'col_only', 'row_col', 'row', 'col_full') or a list with one per member; a
+        position-based member equals PararealDevice(...).run(model='nngp', nntype=..., seed=...).  tspans: None or a
+        list with one [t0, t1] (or None: the ensemble's tspan) per member; member e's output 't' is its own grid.
+        n_restarts, fatol and xatol are common to all members."""
         E = check_run_args(dict(seeds=seeds, epsilons=epsilons, early_stops=early_stops, init_conds=init_conds,
-                                tspans=tspans), model=model, store_int=store_int, nn=nn)
+                                tspans=tspans), model=model, store_int=store_int, nn=nn, nntype=nntype)
         solver = self.solver
         if max(solver.Nf, solver.Ng) > solver.thresh:
             raise Exception('steps > thresh (RK paging, solver.py:89-96) is only supported by the host driver')
@@ -158,9 +181,13 @@ class PararealEnsemble:
         nns = list(nn) if isinstance(nn, (list, tuple, np.ndarray)) else [nn] * E
         spans = [self.tspan if tspans is None or tspans[e] is None else tspans[e] for e in range(E)]
         t_members = np.stack([np.linspace(ts[0], ts[1], num=self.N + 1) for ts in spans])
+        rules = list(nntype) if isinstance(nntype, (list, tuple, np.ndarray)) else [nntype] * E
         h = self.handle()
-        models = [CudaNNGP(n=self.n, N=self.N, seed=s, nn=v if v == 'adaptive' else int(v), n_restarts=n_restarts,
-                           fatol=fatol, xatol=xatol, handle=h) for s, v in zip(seeds, nns)]
+        models = []
+        for s, v, rule in zip(seeds, nns, rules):
+            kw = dict(n=self.n, N=self.N, seed=s, nn=v if v == 'adaptive' else int(v), n_restarts=n_restarts,
+                      fatol=fatol, xatol=xatol, handle=h)
+            models.append(CudaNNGP(**kw) if rule == 'nn' else CudaNNGPAlt(nntype=rule, **kw))
         return self._run(h, models, eps, stops, u0s, max_rows, t_members)
 
     def _run(self, h, models, eps, stops, u0s, max_rows, t_members):
@@ -201,6 +228,8 @@ class PararealEnsemble:
         rows = np.zeros(E, dtype=np.int64)
         last_k = np.zeros(E, dtype=np.int64)
         conv_int = [[] for _ in range(E)]
+        first = [[] for _ in range(E)]  # first unconverged slice of every iteration a member appended (listed rules)
+        listed = np.array([getattr(mdl, 'nntype', 'nn') != 'nn' for mdl in models])
         err = [np.full((N + 1, N), np.nan) for _ in range(E)]
         pos = np.arange(E)  # pos[p] = member at state position p
         for k in range(N):
@@ -244,16 +273,23 @@ class PararealEnsemble:
                 h.seg_reserve(E, cap, n)
             h.seg_append_iteration(live, I[live], st['u_cur'], st['uF'], st['uG_cur'], ld, N, n, stream)
             rows[live] = need
+            for e in live:
+                first[e].append(int(I[e]) - 1)
             n_sweep = int(np.count_nonzero(I[live] < N))  # the members with I == N sort last among the running ones
             if n_sweep > 0:
                 sw = live[:n_sweep]
                 mdl0 = models[sw[0]]
-                m_pos, t_pos = sweep_tables([mdl.neighbours(k) for mdl in models], t_members, sw)
+                lists = [listed_rows(models[e], e, first[e], I[e], e * cap) if listed[e] else None for e in sw]
+                m_members = [mdl.neighbours(k) for mdl in models]
+                for e, tab in zip(sw, lists):
+                    if tab is not None:
+                        m_members[e] = tab.shape[1]
+                m_pos, t_pos = sweep_tables(m_members, t_members, sw)
                 if m_pos.max() > MAX_NEIGHBOURS:
                     raise Exception('nn > 160 neighbours is not supported (include/nngpara.h: NNGP_MAX_NEIGHBOURS_BIG)')
                 m = int(m_pos[0])
                 short = [e for e in sw if rows[e] < m]
-                if short and np.all(m_pos == m):
+                if short and np.all(m_pos == m) and not listed[sw].any():
                     raise Exception(f'members {short} hold fewer dataset rows ({rows[short].min()}) than the common m={m}: '
                                     'an ensemble needs one m per launch')
                 blocks = []
@@ -263,8 +299,14 @@ class PararealEnsemble:
                     blocks.append(mdl.draw_starts(N - I[e]))
                     mdl.train_count += (N - I[e]) * n * N_JITTER * mdl.n_restarts
                 starts = torch.from_numpy(pack_starts(blocks, I[sw], N)).to(dev)
-                launch_sweep(h, t_dev, sysid, mG, hm, solver.Ng, N, sw, I[sw], m_pos, t_pos, mdl0, starts, st['u_next'],
-                             st['uG_next'], n, stream)
+                if listed[sw].any():
+                    t_sw = t_dev.index_select(0, torch.from_numpy(np.asarray(sw, dtype=np.int64)).to(dev))
+                    h.ensemble_sweep_listed(sysid, mG, hm, solver.Ng, t_sw, N, sw, I[sw], m_pos, listed[sw], lists,
+                                            mdl0.n_restarts, starts, mdl0.fatol, mdl0.xatol, st['u_next'],
+                                            st['uG_next'], n, stream)
+                else:
+                    launch_sweep(h, t_dev, sysid, mG, hm, solver.Ng, N, sw, I[sw], m_pos, t_pos, mdl0, starts,
+                                 st['u_next'], st['uG_next'], n, stream)
             # parareal.py:402: one error launch over the running members and ONE device->host read
             h.rowwise_maxabs_diff(st['u_next'], st['u_cur'], n_live * (N + 1), n, err_dev, stream)
             errs = err_dev[:n_live * (N + 1)].cpu().numpy().reshape(n_live, N + 1)

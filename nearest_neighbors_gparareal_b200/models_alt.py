@@ -12,7 +12,9 @@ are the same device launch as for the nearest-neighbour rule (nngp_fit_predict o
     'col_full'  slice i first (iterations k, k-1, ...), then slices i+1, i-1, ... (:137-171)
 
 The model needs the driver's observation cube `data_x` [N, n, K] (NaN where a slice was already converged), which the
-reference passes to `fit` (parareal.py:351); the drivers of this package pass it when `wants_data_cube` is set.
+reference passes to `fit` (parareal.py:351); the host drivers of this package pass it when `wants_data_cube` is set.
+The device drivers (PararealDevice, PararealEnsemble) keep only the first unconverged slice of every iteration and ask
+`neighbour_table` for the lists of a whole sweep, which the listed sweeps of csrc/api.cu then run on the device.
 """
 import numpy as np
 
@@ -51,12 +53,25 @@ class CudaNNGPAlt(CudaNNGP):
         if self.nntype != 'nn' and self.data_x is None:
             raise Exception("the driver must pass data_x to fit() for a position-based neighbour rule")
         if self.data_x is not None:
-            # dataset row of observation (slice i, iteration j): rows of iteration j are the slices first[j] .. N-1
             N = self.data_x.shape[0]
             present = ~np.isnan(self.data_x[:, 0, :k + 1])
-            self._first = np.array([int(np.argmax(present[:, j])) if present[:, j].any() else N for j in range(k + 1)])
-            self._offset = np.concatenate([[0], np.cumsum(N - self._first)])[:k + 1]
-            self._present = present
+            self.set_positions([int(np.argmax(present[:, j])) if present[:, j].any() else N for j in range(k + 1)], k)
+
+    def set_positions(self, first, k):
+        """The position state of iteration k from first[j], the first unconverged slice of iteration j <= k: the rows of
+        iteration j are the slices first[j] .. N-1, appended in that order (parareal.py:336-339).  fit() derives first
+        from data_x; the device drivers, which hold no observation cube, pass the list they keep."""
+        N = self.N
+        self.k = k
+        self._first = np.asarray(first[:k + 1], dtype=np.int64)
+        self._offset = np.concatenate([[0], np.cumsum(N - self._first)])[:k + 1]
+        self._present = np.arange(N)[:, None] >= self._first[None, :]
+
+    def neighbour_table(self, first, I):
+        """[N - I, m] int64: the rows neighbour_rows chooses for the predicts at slices I .. N-1 of iteration
+        len(first) - 1, in slice order (so 'col+rnd' draws rng2 as the host driver does)"""
+        self.set_positions(first, len(first) - 1)
+        return np.array([self.neighbour_rows(i) for i in range(I, self.N)], dtype=np.int64).reshape(self.N - I, -1)
 
     def _row(self, i, j):
         return int(self._offset[j] + i - self._first[j])
@@ -64,7 +79,7 @@ class CudaNNGPAlt(CudaNNGP):
     def neighbour_rows(self, i):
         """dataset row indices chosen by the rule for a predict at slice i of iteration self.k"""
         k, nn, nt = self.k, self.nn, self.nntype
-        N = self.data_x.shape[0]
+        N = self._present.shape[0]
         have = lambda s, j: 0 <= s < N and self._present[s, j]
         if nt == 'col_only':
             return [self._row(i, j) for j in range(k + 1)]
@@ -72,7 +87,8 @@ class CudaNNGPAlt(CudaNNGP):
             nn = max(10, k + 2) if nn == 'adaptive' else nn
             on_col = min(nn, k + 1)
             col = [self._row(i, j) for j in range(k + 1 - on_col, k + 1)]
-            cands = self.rng2.permutation(np.arange(self.x.shape[0]))[:nn]
+            n_rows = int(self._offset[k] + N - self._first[k])  # the dataset's rows: iterations 0 .. k
+            cands = self.rng2.permutation(np.arange(n_rows))[:nn]
             near = [int(c) for c in cands if int(c) not in col][:nn - on_col]
             rows = col + near
             assert len(rows) == nn

@@ -366,7 +366,9 @@ class PararealLight(Parareal):
 class PararealDevice(Parareal):
     """Device-resident nnGParareal: the whole iteration of parareal.py:301-439 on the GPU.
 
-    Needs a CudaSolverRK and either the 'nngp' or the 'parareal' model.  With an initialised
+    Needs a CudaSolverRK and either the 'nngp' or the 'parareal' model; 'nngp' with a position-based `nntype`
+    (models_alt.py) builds each iteration's neighbour lists on the host with the model's own rules and sweeps them
+    with nngp_sweep_listed_shard.  With an initialised
     torch.distributed process group of W>1 ranks (one per GPU) the fine solves are sharded by
     time slice: rank r propagates a contiguous block of the unconverged slices, writing straight
     into its part of the gather buffer, and ONE all-gather per iteration makes every rank hold
@@ -419,6 +421,10 @@ class PararealDevice(Parareal):
         st['err'] = torch.zeros(N + 1, **f64)
         for key in ('u_cur', 'uG_cur', 'uF'):
             st[key][0] = u0
+        # position-based neighbour rule (models_alt.py): the host chooses each predict's rows from the first unconverged
+        # slice of every iteration so far, kept here as the dataset grows
+        st['listed'] = st['is_gp'] and getattr(model, 'nntype', 'nn') != 'nn'
+        st['first'] = []
         if st['is_gp']:
             model._handle = h
             h.dataset_reset()
@@ -465,12 +471,18 @@ class PararealDevice(Parareal):
                 h.dataset_reserve(st['cap'], n)
             h.append_iteration(st['u_cur'], st['uF'], st['uG_cur'], N, I, n, st['stream'])
             model._n_dev = h.dataset_rows()
+            st['first'].append(I - 1)
         if I == N:
             return
         if st['is_gp']:
             model.k = k
             model.time_k = k
-            m = min(model.neighbours(k), h.dataset_rows())
+            rows = None
+            if st['listed']:
+                rows = model.neighbour_table(st['first'], I)
+                m = rows.shape[1]
+            else:
+                m = min(model.neighbours(k), h.dataset_rows())
             if m > 160:
                 raise Exception('nn > 160 neighbours is not supported (include/nngpara.h: NNGP_MAX_NEIGHBOURS_BIG)')
             if starts is None:
@@ -481,14 +493,23 @@ class PararealDevice(Parareal):
                 import torch.distributed as dist
                 j0, dl = dim_block(n, st['rank'], world)
                 for i in range(I, N):
-                    h.sweep_shard(st['sys'], st['mG'], solver.h_mode, solver.Ng, st['t'], N, I, i, 1, m,
-                                  model.n_restarts, starts, model.fatol, model.xatol, st['u_next'], st['uG_next'],
-                                  n, j0, dl, st['stream'])
+                    if rows is None:
+                        h.sweep_shard(st['sys'], st['mG'], solver.h_mode, solver.Ng, st['t'], N, I, i, 1, m,
+                                      model.n_restarts, starts, model.fatol, model.xatol, st['u_next'], st['uG_next'],
+                                      n, j0, dl, st['stream'])
+                    else:
+                        h.sweep_listed_shard(st['sys'], st['mG'], solver.h_mode, solver.Ng, st['t'], N, I, i, 1, rows,
+                                             model.n_restarts, starts, model.fatol, model.xatol, st['u_next'],
+                                             st['uG_next'], n, j0, dl, st['stream'])
                     row = st['u_next'][i + 1]
                     dist.all_gather_into_tensor(row, row[j0:j0 + dl], group=self.group)
-            else:
+            elif rows is None:
                 h.sweep(st['sys'], st['mG'], solver.h_mode, solver.Ng, st['t'], N, I, m, model.n_restarts, starts,
                         model.fatol, model.xatol, st['u_next'], st['uG_next'], n, st['stream'])
+            else:
+                h.sweep_listed_shard(st['sys'], st['mG'], solver.h_mode, solver.Ng, st['t'], N, I, I, N - I, rows,
+                                     model.n_restarts, starts, model.fatol, model.xatol, st['u_next'], st['uG_next'],
+                                     n, 0, n, st['stream'])
             model.train_count += (N - I) * n * N_JITTER * model.n_restarts
         else:
             for i in range(I, N):
@@ -514,6 +535,9 @@ class PararealDevice(Parareal):
         import torch
         N, eps = self.N, self.epsilon
         verbose = kwargs.get('verbose', self.verbose)
+        if store_int and getattr(model, 'nntype', 'nn') != 'nn':
+            raise Exception(f"PararealDevice does not write intermediate checkpoints of the position-based neighbour rule "
+                            f"nntype={model.nntype!r} (store_int=True): run it with the host driver Parareal")
         tic = time.time()
         st = self.device_setup(model, max_rows=max_rows)
         torch.cuda.synchronize(st['dev'])

@@ -30,7 +30,7 @@ extern "C" {
 
 typedef struct nngp_handle_s* nngp_handle_t;
 
-#define NNGP_ABI_VERSION 1
+#define NNGP_ABI_VERSION 2
 #define NNGP_MAX_NEIGHBOURS 32 /* m <= 32: one lane per neighbour row (the fast kernels) */
 #define NNGP_MAX_NEIGHBOURS_BIG 160 /* 32 < m <= 160 (nn='adaptive' past iteration 30): one CTA per search, matrix in shared memory */
 #define NNGP_N_JITTER 9        /* models.py:186  jitter = arange(-20,-11) */
@@ -233,34 +233,28 @@ int nngp_knn_segmented(nngp_handle_t h, const double* d_q, long long ld_q, int n
  * identity.  Device pointers; gathers and scatters the rows of an ensemble's state. */
 int nngp_copy_rows(nngp_handle_t h, const double* d_src, const long long* d_src_idx, double* d_dst,
                    const long long* d_dst_idx, long long rows, long long d, void* stream);
-/* nngp_sweep for E runs in lockstep, slices min(I) .. N-1, enqueued with no host round trip.  State u_next,
- * uG_next: device [E, N+1, d]; position p belongs to segment members[p] (host) and sweeps slices I[p] .. N-1 (host,
- * ascending in p, so the runs active at a slice are a prefix).  Per slice: one coarse launch over the active runs,
- * one segmented kNN, one fit over all their predicts.  d_starts: the starts of every predict, slice-major -- for
- * slice i the [d,9,R,2] blocks of the active positions in order.  Each run's results equal its nngp_sweep. */
-int nngp_ensemble_sweep(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g, const double* d_t, int N,
-                        int E, const int* members, const int* I, int m, int n_restarts, const signed char* d_starts,
-                        double fatol, double xatol, double* d_u_next, double* d_uG_next, int d, void* stream);
-/* nngp_ensemble_sweep for runs that differ in neighbour count and time grid: m[E] (host) the neighbour count of each
- * position, d_t_pos (device [E, N+1]) the slice boundaries of each position.  Per slice one segmented kNN at the
- * largest m of the active runs (the first m_p neighbours of a top-m_max list are the top-m_p), then one fit per
- * distinct m over the runs that use it, each seeing exactly the neighbour set and matrix of its nngp_sweep.  A slice
- * in which an active run holds fewer rows than the slice's largest m is refused before anything is enqueued. */
-int nngp_ensemble_sweep_mixed(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g,
-                              const double* d_t_pos, int N, int E, const int* members, const int* I, const int* m,
-                              int n_restarts, const signed char* d_starts, double fatol, double xatol,
-                              double* d_u_next, double* d_uG_next, int d, void* stream);
-/* nngp_ensemble_sweep_mixed where each position has its own neighbour rule: listed[p] != 0 (host) marks the positions
- * whose neighbours the host chose (nngp_sweep_listed_shard); the others take the m_p nearest rows of their segment.
- * rows (host, int64): for every listed position in position order, its lists of slices I_p .. N-1, [(N - I_p), m_p],
- * as global rows of the store (members[p] cap + the member's row, inside its held rows).  Per slice at most one
- * listed-prep launch (which also gathers the queries of the kNN positions when the slice has both kinds) and one
- * segmented kNN over the kNN positions; the "fewer rows than the slice's largest m" refusal applies to those only.
- * Everything is validated before anything is enqueued; each run's results equal its solo listed or kNN sweep. */
-int nngp_ensemble_sweep_listed(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g,
-                               const double* d_t_pos, int N, int E, const int* members, const int* I, const int* m,
-                               const int* listed, const long long* rows, int n_restarts, const signed char* d_starts,
-                               double fatol, double xatol, double* d_u_next, double* d_uG_next, int d, void* stream);
+/* nngp_sweep for E runs in lockstep, slices min(I) .. N-1, enqueued with no host round trip.  Every refusal happens
+ * before anything is enqueued.
+ * Layout: state u_next, uG_next: device [E, N+1, d].  Position p belongs to segment members[p] (host) and sweeps
+ * slices I[p] .. N-1 (host, ascending in p, so the runs active at a slice are a prefix of the positions, reached with
+ * the member stride (N+1) d).  d_t_pos (device [E, N+1]): the slice boundaries of each position.  m[E] (host, each in
+ * 1..160): the neighbour count of each position.  d_starts: the starts of every predict, slice-major -- for slice i the
+ * [d,9,R,2] blocks of the active positions in position order.
+ * Neighbours: per slice one segmented kNN over the active kNN positions at the largest m among them (the first m_p
+ * neighbours of a top-m_max list are the top-m_p); a slice in which such a member holds fewer rows than that m is
+ * refused.  listed (host, NULL: no position) marks with listed[p] != 0 the positions whose neighbours the host chose
+ * instead (nngp_sweep_listed_shard): rows (host, int64) holds, for every listed position in position order, its lists of
+ * slices I_p .. N-1, [(N - I_p), m_p], as global rows of the store (members[p] cap + a row the member holds); a row
+ * outside that range is refused.  Each run's results equal its solo kNN or listed sweep, bit for bit.
+ * Routes, chosen once per call from the inputs: when no swept position is listed and all share one m, per slice one
+ * coarse launch over the active runs beside the kNN, and one fit over all their predicts straight into the state;
+ * otherwise per slice at most one listed-prep launch (which also gathers the kNN queries when the slice has both
+ * kinds), the kNN, one gather, one fit per distinct m over the runs that use it (each sees exactly the neighbour set
+ * and matrix of its solo sweep) and one scatter. */
+int nngp_ensemble_sweep(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g, const double* d_t_pos,
+                        int N, int E, const int* members, const int* I, const int* m, const int* listed,
+                        const long long* rows, int n_restarts, const signed char* d_starts, double fatol, double xatol,
+                        double* d_u_next, double* d_uG_next, int d, void* stream);
 /* nngp_fit_predict with one neighbour count per predict: m[nq] (host); d_idx / d_dist rows ld = max m apart, the
  * first m[q] entries of row q used; the neighbour matrix is formed at ld.  Outputs as nngp_fit_predict. */
 int nngp_fit_predict_mixed(nngp_handle_t h, const double* d_q, const long long* d_idx, const double* d_dist, int nq,

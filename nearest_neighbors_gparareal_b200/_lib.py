@@ -71,14 +71,11 @@ SIGNATURES = {
     "nngp_seg_append_iteration": (ci, [vp, ci, vp, vp, vp, vp, vp, cll, ci, ci, vp]),
     "nngp_knn_segmented": (ci, [vp, vp, cll, ci, ci, vp, vp, vp, vp, vp, vp]),
     "nngp_copy_rows": (ci, [vp, vp, vp, vp, vp, cll, cll, vp]),
-    "nngp_ensemble_sweep": (ci, [vp, ci, ci, ci, cll, vp, ci, ci, vp, vp, ci, ci, vp, cd, cd, vp, vp, ci, vp]),
-    "nngp_ensemble_sweep_mixed": (ci, [vp, ci, ci, ci, cll, vp, ci, ci, vp, vp, vp, ci, vp, cd, cd, vp, vp, ci, vp]),
+    "nngp_ensemble_sweep": (ci, [vp, ci, ci, ci, cll, vp, ci, ci, vp, vp, vp, vp, vp, ci, vp, cd, cd, vp, vp, ci, vp]),
     "nngp_fit_predict_mixed": (ci, [vp, vp, vp, vp, ci, vp, ci, vp, cd, cd, vp, vp, vp, vp, vp, vp, vp, vp]),
     "nngp_listed_prep": (ci, [vp, vp, cll, ci, ci, vp, ci, vp, vp, vp]),
     "nngp_sweep_listed_shard": (ci, [vp, ci, ci, ci, cll, vp, ci, ci, ci, ci, ci, vp, ci, vp, cd, cd, vp, vp, ci, ci, ci,
                                      vp]),
-    "nngp_ensemble_sweep_listed": (ci, [vp, ci, ci, ci, cll, vp, ci, ci, vp, vp, vp, vp, vp, ci, vp, cd, cd, vp, vp, ci,
-                                        vp]),
 }
 
 SYSTEM_IDS = {"FHN_ODE": 0, "Rossler": 1, "Hopf": 2, "DblPend": 3, "Brusselator": 4, "Lorenz": 5,
@@ -354,43 +351,29 @@ class Handle:
         self.check(self.lib.nngp_copy_rows(self.h, _ptr(d_src), _ptr(d_src_idx), _ptr(d_dst), _ptr(d_dst_idx),
                                            int(rows), int(d), stream))
 
-    def ensemble_sweep(self, sys, method_g, h_mode, steps_g, d_t, N, members, I, m, n_restarts, d_starts, fatol, xatol,
-                       d_u_next, d_uG_next, d, stream=None):
-        members, I = np.ascontiguousarray(members, dtype=np.int32), np.ascontiguousarray(I, dtype=np.int32)
-        self.check(self.lib.nngp_ensemble_sweep(self.h, sys, method_g, h_mode, int(steps_g), _ptr(d_t), int(N),
-                                                members.size, _ptr(members), _ptr(I), int(m), int(n_restarts),
-                                                _ptr(d_starts), float(fatol), float(xatol), _ptr(d_u_next),
-                                                _ptr(d_uG_next), int(d), stream))
-
-    def ensemble_sweep_mixed(self, sys, method_g, h_mode, steps_g, d_t_pos, N, members, I, m, n_restarts, d_starts,
-                             fatol, xatol, d_u_next, d_uG_next, d, stream=None):
-        """ensemble_sweep with one neighbour count m[p] and one time grid d_t_pos[p] (device [E, N+1]) per position"""
+    def ensemble_sweep(self, sys, method_g, h_mode, steps_g, d_t_pos, N, members, I, m, n_restarts, d_starts, fatol,
+                       xatol, d_u_next, d_uG_next, d, listed=None, rows=None, stream=None):
+        """Position p sweeps member members[p] from slice I[p] with m[p] neighbours on its grid d_t_pos[p] (device
+        [E, N+1]).  listed (None: no position) marks the positions that take the host lists rows[p] ([N - I[p], m[p]]
+        global store rows; None for the others) instead of the segmented kNN."""
         members, I = np.ascontiguousarray(members, dtype=np.int32), np.ascontiguousarray(I, dtype=np.int32)
         m = np.ascontiguousarray(m, dtype=np.int32)
         assert m.size == members.size
-        self.check(self.lib.nngp_ensemble_sweep_mixed(self.h, sys, method_g, h_mode, int(steps_g), _ptr(d_t_pos), int(N),
-                                                      members.size, _ptr(members), _ptr(I), _ptr(m), int(n_restarts),
-                                                      _ptr(d_starts), float(fatol), float(xatol), _ptr(d_u_next),
-                                                      _ptr(d_uG_next), int(d), stream))
-
-    def ensemble_sweep_listed(self, sys, method_g, h_mode, steps_g, d_t_pos, N, members, I, m, listed, rows, n_restarts,
-                              d_starts, fatol, xatol, d_u_next, d_uG_next, d, stream=None):
-        """ensemble_sweep_mixed where the positions with listed[p] take the host lists rows[p] ([N - I[p], m[p]] global
-        store rows; None for the others) instead of the segmented kNN"""
-        members, I = np.ascontiguousarray(members, dtype=np.int32), np.ascontiguousarray(I, dtype=np.int32)
-        m, listed = np.ascontiguousarray(m, dtype=np.int32), np.ascontiguousarray(listed, dtype=np.int32)
-        assert m.size == members.size and listed.size == members.size and len(rows) == members.size
-        blocks = []
-        for p in range(members.size):
-            if listed[p]:
-                b = np.asarray(rows[p], dtype=np.int64).reshape(-1, int(m[p]))
-                assert b.shape[0] == N - I[p], "the lists of position p must be [N - I[p], m[p]]"
-                blocks.append(b.ravel())
-        flat = np.ascontiguousarray(np.concatenate(blocks) if blocks else np.zeros(0, np.int64))
-        self.check(self.lib.nngp_ensemble_sweep_listed(self.h, sys, method_g, h_mode, int(steps_g), _ptr(d_t_pos), int(N),
-                                                       members.size, _ptr(members), _ptr(I), _ptr(m), _ptr(listed),
-                                                       _ptr(flat), int(n_restarts), _ptr(d_starts), float(fatol),
-                                                       float(xatol), _ptr(d_u_next), _ptr(d_uG_next), int(d), stream))
+        flat = None
+        if listed is not None:
+            listed = np.ascontiguousarray(listed, dtype=np.int32)
+            assert listed.size == members.size and len(rows) == members.size
+            blocks = []
+            for p in range(members.size):
+                if listed[p]:
+                    b = np.asarray(rows[p], dtype=np.int64).reshape(-1, int(m[p]))
+                    assert b.shape[0] == N - I[p], "the lists of position p must be [N - I[p], m[p]]"
+                    blocks.append(b.ravel())
+            flat = np.ascontiguousarray(np.concatenate(blocks) if blocks else np.zeros(0, np.int64))
+        self.check(self.lib.nngp_ensemble_sweep(self.h, sys, method_g, h_mode, int(steps_g), _ptr(d_t_pos), int(N),
+                                                members.size, _ptr(members), _ptr(I), _ptr(m), _ptr(listed), _ptr(flat),
+                                                int(n_restarts), _ptr(d_starts), float(fatol), float(xatol),
+                                                _ptr(d_u_next), _ptr(d_uG_next), int(d), stream))
 
     def selftest_math(self, d_x, n, d_exp, d_rcp, d_exp10=None, stream=None):
         self.check(self.lib.nngp_selftest_math(self.h, _ptr(d_x), int(n), _ptr(d_exp), _ptr(d_rcp),

@@ -71,14 +71,14 @@ static unsigned int* next_queue(nngp_handle_t h, cudaStream_t st) {
   return p;
 }
 
-// the fit kernel leaves its completion counters zero; they only need clearing when they move
-static int ensure_done_zero(nngp_handle_t h, void* ws_fit, int nq, int d, int m, int R, cudaStream_t st) {
+// the fit kernel leaves its completion counters zero; they only need clearing when they move (t: where they last were)
+static int ensure_done_zero(nngp_handle_t h, DoneTracker& t, void* ws_fit, int nq, int d, int m, int R, cudaStream_t st) {
   const char* ptr = (const char*)ws_fit + gp_fit_done_offset(nq, d, m, R);
   const size_t bytes = sizeof(unsigned int) * (size_t)nq * d;
-  if (h->done_ptr != ptr || h->done_bytes != bytes) {
+  if (t.ptr != ptr || t.bytes != bytes) {
     NNGP_CUDA(h, cudaMemsetAsync((void*)ptr, 0, bytes, st));
-    h->done_ptr = ptr;
-    h->done_bytes = bytes;
+    t.ptr = ptr;
+    t.bytes = bytes;
   }
   return 0;
 }
@@ -86,7 +86,7 @@ static int ensure_done_zero(nngp_handle_t h, void* ws_fit, int nq, int d, int m,
 void* nngp_workspace(nngp_handle_t h, size_t bytes) {
   // whoever asks for the block may overwrite the (left-zero) completion counters of an earlier fit:
   // the next fit clears them again (ensure_done_zero)
-  h->done_ptr = nullptr;
+  h->done = DoneTracker{};
   if (bytes <= h->ws_bytes) return h->ws;
   // grow: work already enqueued may still use the old block
   cudaDeviceSynchronize();
@@ -660,7 +660,7 @@ int nngp_fit_predict(nngp_handle_t h, const double* d_q, const long long* d_idx,
   int* order;
   if (int rc = fit_workspace(h, nq, h->ds_rows, m, n_restarts, &kws, &fws, &order)) return rc;
   cudaStream_t st = as_stream(stream);
-  if (int rc = ensure_done_zero(h, fws, nq, h->ds_d, m, n_restarts, st)) return rc;
+  if (int rc = ensure_done_zero(h, h->done, fws, nq, h->ds_d, m, n_restarts, st)) return rc;
   if (int rc = gp_prep_launch(h, d_idx, nq, m, (double*)fws, st)) return rc;
   if (int rc = gp_order_launch(h, d_starts, nq, h->ds_d * NNGP_N_JITTER * n_restarts, 1, order, st)) return rc;
   return gp_fit_predict_launch(h, d_idx, d_dist, fws, next_queue(h, st), order, nq, m, n_restarts, d_starts, fatol,
@@ -763,7 +763,7 @@ int nngp_predict_host_block(nngp_handle_t h, const double* q, int nq, int m, lon
   void *kws, *fws;
   int* order;
   if (int rc = fit_workspace(h, nq, n, m, R, &kws, &fws, &order)) return rc;
-  if (int rc = ensure_done_zero(h, fws, nq, d, m, R, st)) return rc;
+  if (int rc = ensure_done_zero(h, h->done, fws, nq, d, m, R, st)) return rc;
   if (int rc = knn_prep_launch(h, gq, nq, m, n, gidx, gdist, kws, fws, st)) return rc;
   if (dl == d) {
     if (int rc = gp_order_launch(h, gst, nq, d * NNGP_N_JITTER * R, 1, order, st)) return rc;
@@ -862,7 +862,7 @@ static int sweep_shard_impl(nngp_handle_t h, int sys, int method_g, int h_mode, 
     if (!(dlq = (const ListedQuery*)upload_table(h, 4, lq.data(), sizeof(ListedQuery) * lq.size(), st)))
       return nngp_fail(h, "sweep_listed: out of memory for the query table");
   }
-  if (int rc = ensure_done_zero(h, fws, 1, d, m, n_restarts, st)) return rc;
+  if (int rc = ensure_done_zero(h, h->done, fws, 1, d, m, n_restarts, st)) return rc;
   // queue order of every predict of the call in one launch (the starts are all known up front); with dl = d the
   // blocks of consecutive predicts are contiguous, with dl < d there is one
   const signed char* starts_first = d_starts + (size_t)(i_first - I) * per_predict;
@@ -1021,13 +1021,8 @@ int nngp_copy_rows(nngp_handle_t h, const double* d_src, const long long* d_src_
   return copy_rows_launch(h, d_src, d_src_idx, d_dst, d_dst_idx, rows, d, as_stream(stream));
 }
 
-// t_rep[i, p] = t[i]: the per-slice time arrays of a launch over the members of one slice
-__global__ void repeat_t_kernel(const double* __restrict__ t, int n_t, int E, double* __restrict__ t_rep) {
-  const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (e < (long long)n_t * E) t_rep[e] = t[e / E];
-}
-
-// t_rep[i, p] = t_pos[p, i]: per-position time grids in the layout of repeat_t_kernel
+// t_rep[i, p] = t_pos[p, i]: row i holds the slice boundaries t_i of every position, so the coarse step of the first n
+// positions at slice i reads its t0 and t1 from rows i and i + 1
 __global__ void transpose_t_kernel(const double* __restrict__ t_pos, int n_t, int E, double* __restrict__ t_rep) {
   const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (e < (long long)n_t * E) {
@@ -1091,8 +1086,7 @@ struct MixedGroups {
     double *dist, *add, *pred, *theta_opt, *jitter_opt, *fval_opt, *fvals, *thetas;
     int* nfev;
     signed char* starts;
-    const char* done_ptr = nullptr;  // the fit leaves its completion counters zero; clear them when they move
-    size_t done_bytes = 0;
+    DoneTracker done;
   };
   std::vector<Dev> dev;
 
@@ -1145,7 +1139,7 @@ struct MixedGroups {
       out->fvals = details ? (double*)(b + o_fs) : nullptr;
       out->thetas = details ? (double*)(b + o_ts) : nullptr;
       out->fws = b + o_f;
-      out->done_ptr = nullptr;
+      out->done = DoneTracker{};
     }
     return off;
   }
@@ -1155,13 +1149,7 @@ static int mixed_fit_group(nngp_handle_t h, MixedGroups& G, int g, int n, int d,
                            bool add_on, cudaStream_t st) {
   MixedGroups::Dev& D = G.dev[g];
   const int mg = G.m[g], seg_len = d * NNGP_N_JITTER * R;
-  const char* done = D.fws + gp_fit_done_offset(n, d, mg, R);
-  const size_t done_bytes = sizeof(unsigned int) * (size_t)n * d;
-  if (D.done_ptr != done || D.done_bytes != done_bytes) {
-    NNGP_CUDA(h, cudaMemsetAsync((void*)done, 0, done_bytes, st));
-    D.done_ptr = done;
-    D.done_bytes = done_bytes;
-  }
+  if (int rc = ensure_done_zero(h, D.done, D.fws, n, d, mg, R, st)) return rc;
   if (int rc = gp_order_launch(h, D.starts, n, seg_len, 1, D.order, st)) return rc;
   return gp_fit_predict_launch(h, D.idx, D.dist, D.fws, next_queue(h, st), D.order, n, mg, R, D.starts, fatol, xatol,
                                D.pred, add_on ? D.add : nullptr, d, D.theta_opt, D.jitter_opt, D.fval_opt, D.nfev,
@@ -1233,14 +1221,22 @@ int nngp_fit_predict_mixed(nngp_handle_t h, const double* d_q, const long long* 
   return copy_spans_launch(h, dsp + n_gather, (int)(sp.size() - n_gather), st);
 }
 
-// nngp_ensemble_sweep (m_pos == nullptr: one m and the shared grid d_t), nngp_ensemble_sweep_mixed (m_pos[E] and
-// the per-position grids d_t_pos[E, N+1]) and nngp_ensemble_sweep_listed (the mixed sweep where the positions with
-// listed[p] != 0 take their neighbours from the host lists `rows` instead of the segmented kNN).
-static int ensemble_sweep_impl(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g, const double* d_t,
-                               const double* d_t_pos, int N, int E, const int* members, const int* I, int m,
-                               const int* m_pos, const int* listed, const long long* rows, int n_restarts,
-                               const signed char* d_starts, double fatol, double xatol, double* d_u_next,
-                               double* d_uG_next, int d, void* stream) {
+// One slice of an ensemble sweep, planned before anything is enqueued: the active positions (a prefix, n_act), the kNN
+// positions among them (the first nk_act of the sweep's kNN positions, searched at their largest m, mm, over segments
+// of at most n_max rows), the starts of its first predict and, on the grouped route, where its gather and scatter
+// copies and its listed preps lie in the sweep's tables.
+struct SlicePlan {
+  int n_act, nk_act, mm;
+  long long n_max;
+  const signed char* starts;
+  size_t gather, scatter, end;  // copies: gather [gather, scatter), scatter [scatter, end)
+  size_t lq, lq_end;            // listed preps [lq, lq_end)
+};
+
+int nngp_ensemble_sweep(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g, const double* d_t_pos,
+                        int N, int E, const int* members, const int* I, const int* m, const int* listed,
+                        const long long* rows, int n_restarts, const signed char* d_starts, double fatol, double xatol,
+                        double* d_u_next, double* d_uG_next, int d, void* stream) {
   NNGP_USE_DEVICE(h);
   const SystemDesc* s;
   if (int rc = get_sys(h, sys, &s)) return rc;
@@ -1248,99 +1244,53 @@ static int ensemble_sweep_impl(nngp_handle_t h, int sys, int method_g, int h_mod
   if (d != s->d || d != h->ds_d) return nngp_fail(h, "ensemble_sweep: d=%d, system d=%d, store d=%d", d, s->d, h->ds_d);
   if (E < 1) return nngp_fail(h, "ensemble_sweep: E=%d < 1", E);
   if (n_restarts < 1) return nngp_fail(h, "ensemble_sweep: n_restarts=%d < 1", n_restarts);
-  const bool mixed = m_pos != nullptr;
-  if (mixed) {
-    m = 0;
-    for (int p = 0; p < E; p++) {
-      if (m_pos[p] < 1 || m_pos[p] > NNGP_MAX_NEIGHBOURS_BIG)
-        return nngp_fail(h, "ensemble_sweep: position %d: m=%d outside [1,%d]", p, m_pos[p], NNGP_MAX_NEIGHBOURS_BIG);
-      if (I[p] < N) m = std::max(m, m_pos[p]);
-    }
-  } else if (m < 1 || m > NNGP_MAX_NEIGHBOURS_BIG) {
-    return nngp_fail(h, "ensemble_sweep: m=%d outside [1,%d]", m, NNGP_MAX_NEIGHBOURS_BIG);
-  }
-  std::vector<long long> tab(2 * (size_t)E);
+  if (m == nullptr || d_t_pos == nullptr) return nngp_fail(h, "ensemble_sweep: m and d_t_pos are required");
+  auto is_listed = [&](int p) { return listed != nullptr && listed[p] != 0; };
+  // per position: the kNN positions in position order, where a listed position's block of `rows` starts, and what
+  // sizes the workspace
+  std::vector<int> kpos;
+  std::vector<size_t> row_at(E, 0);
+  size_t n_listed_rows = 0;
+  int n_sw = 0, m_max = 0;  // positions that sweep at least one slice, their largest m
+  long long n_max_all = 0;
+  bool in_place = true;  // the route: no swept position is listed and all of them share one m
   for (int p = 0; p < E; p++) {
     const int e = members[p];
+    if (m[p] < 1 || m[p] > NNGP_MAX_NEIGHBOURS_BIG)
+      return nngp_fail(h, "ensemble_sweep: position %d: m=%d outside [1,%d]", p, m[p], NNGP_MAX_NEIGHBOURS_BIG);
     if (e < 0 || e >= h->seg_E) return nngp_fail(h, "ensemble_sweep: member %d outside [0,%d)", e, h->seg_E);
     if (I[p] < 0 || I[p] > N || (p > 0 && I[p] < I[p - 1]))
       return nngp_fail(h, "ensemble_sweep: I must be ascending in [0,%d] (position %d: %d)", N, p, I[p]);
-    if (!mixed && I[p] < N && h->seg_rows[e] < m)
-      return nngp_fail(h, "ensemble_sweep: member %d holds %lld rows, fewer than m=%d", e, h->seg_rows[e], m);
-    tab[p] = (long long)e * h->seg_cap;
-    tab[E + p] = h->seg_rows[e];
-  }
-  // the kNN positions (all of them without `listed`) in position order, and their segment table: the kNN of a slice
-  // runs over the active ones, a prefix of them
-  auto is_listed = [&](int p) { return listed != nullptr && listed[p] != 0; };
-  std::vector<int> kpos;
-  for (int p = 0; p < E; p++)
-    if (!is_listed(p)) kpos.push_back(p);
-  const int nk = (int)kpos.size();
-  std::vector<long long> ktab(2 * (size_t)nk);
-  for (int r = 0; r < nk; r++) {
-    ktab[r] = tab[kpos[r]];
-    ktab[nk + r] = tab[E + kpos[r]];
-  }
-  // listed positions: block [(N - I_p), m_p] of `rows` in position order, every row inside the member's segment
-  std::vector<size_t> row_at(E, 0);
-  size_t n_listed_rows = 0;
-  for (int p = 0; p < E; p++) {
-    if (!is_listed(p)) continue;
-    row_at[p] = n_listed_rows;
-    const size_t cnt = (size_t)(N - I[p]) * m_pos[p];
-    if (cnt > 0 && rows == nullptr) return nngp_fail(h, "ensemble_sweep_listed: rows is NULL");
-    for (size_t a = 0; a < cnt; a++) {
-      const long long r = rows[n_listed_rows + a];
-      if (r < tab[p] || r >= tab[p] + tab[E + p])
-        return nngp_fail(h, "ensemble_sweep_listed: member %d, slice %d lists row %lld, outside its segment [%lld,%lld)",
-                         members[p], I[p] + (int)(a / m_pos[p]), r, tab[p], tab[p] + tab[E + p]);
+    n_max_all = std::max(n_max_all, h->seg_rows[e]);
+    if (is_listed(p)) {
+      row_at[p] = n_listed_rows;
+      n_listed_rows += (size_t)(N - I[p]) * m[p];
+    } else {
+      kpos.push_back(p);
     }
-    n_listed_rows += cnt;
+    if (I[p] < N) {
+      n_sw++;
+      m_max = std::max(m_max, m[p]);
+      in_place = in_place && !is_listed(p) && m[p] == m[0];
+    }
   }
+  if (n_listed_rows > 0 && rows == nullptr) return nngp_fail(h, "ensemble_sweep: rows is NULL");
   if (I[0] >= N) return 0;
-  if (mixed) {
-    // each slice searches its kNN runs' neighbours at the largest m among them: a run whose segment is shorter would
-    // read padding indices as rows.  Refused before anything is enqueued.
-    int n_act = 0, mm = 0, short_p = -1;
-    for (int i = I[0]; i < N; i++) {
-      for (; n_act < E && I[n_act] <= i; n_act++) {
-        if (is_listed(n_act)) continue;
-        mm = std::max(mm, m_pos[n_act]);
-        if (short_p < 0 || tab[E + n_act] < tab[E + short_p]) short_p = n_act;
-      }
-      if (short_p >= 0 && tab[E + short_p] < mm)
-        return nngp_fail(h, "ensemble_sweep: member %d holds %lld rows, fewer than m=%d, the largest m of slice %d",
-                         members[short_p], tab[E + short_p], mm, i);
-    }
-  }
-  cudaStream_t st = as_stream(stream);
-  const long long ld = (long long)(N + 1) * d;
-  long long n_max_all = 0;
-  for (int p = 0; p < E; p++) n_max_all = std::max(n_max_all, tab[E + p]);
-  const int seg_len = d * NNGP_N_JITTER * n_restarts;
+  const int nk = (int)kpos.size(), seg_len = d * NNGP_N_JITTER * n_restarts;
   const size_t per_predict = (size_t)seg_len * 2;
-  int n_sw = 0;  // positions that sweep at least one slice
-  while (n_sw < E && I[n_sw] < N) n_sw++;
-  const size_t bk = Carver::pad(knn_seg_workspace_bytes(E, n_max_all, m));
-  // mixed: the kNN's neighbour matrices get their own block; the fits work in the groups' blocks
-  MixedGroups G(m_pos, mixed ? n_sw : 0);
-  const size_t bf = mixed ? Carver::pad(gp_prep_bytes(E, m)) + G.bytes(d, n_restarts, false)
-                          : Carver::pad(gp_fit_ws_bytes(E, d, m, n_restarts));
-  const size_t bi = Carver::pad(sizeof(long long) * (size_t)E * m), bd = Carver::pad(sizeof(double) * (size_t)E * m);
+  const long long ld = (long long)(N + 1) * d;
+  // in place: the kNN writes its neighbour matrices into the fit's block; grouped: they get their own block (br) and
+  // the fits work in the groups' blocks
+  MixedGroups G(m, in_place ? 0 : n_sw);
+  const size_t bk = Carver::pad(knn_seg_workspace_bytes(E, n_max_all, m_max));
+  const size_t br = Carver::pad(gp_prep_bytes(E, m_max));
+  const size_t bf = in_place ? Carver::pad(gp_fit_ws_bytes(E, d, m_max, n_restarts)) : br + G.bytes(d, n_restarts, false);
+  const size_t bi = Carver::pad(sizeof(long long) * (size_t)E * m_max), bd = Carver::pad(sizeof(double) * (size_t)E * m_max);
   const size_t bo = Carver::pad(sizeof(int) * (size_t)E * seg_len);
   const size_t bt = Carver::pad(sizeof(double) * (size_t)(N + 1) * E);
   const size_t bq = listed ? Carver::pad(sizeof(double) * (size_t)nk * d) : 0;  // gathered kNN queries
   char* ws = (char*)nngp_workspace(h, bk + bf + bi + bd + bo + bt + bq);
-  unsigned int* tickets = seg_tickets(h, E);
-  if (!ws || !tickets) return nngp_fail(h, "ensemble_sweep: out of device memory");
-  const long long* dtab = nullptr;
-  if (nk > 0 && !(dtab = (const long long*)upload_table(h, 1, ktab.data(), sizeof(long long) * ktab.size(), st)))
-    return nngp_fail(h, "ensemble_sweep: out of memory for the segment table");
-  const long long* drows = nullptr;
-  if (n_listed_rows > 0 &&
-      !(drows = (const long long*)upload_table(h, 3, rows, sizeof(long long) * n_listed_rows, st)))
-    return nngp_fail(h, "ensemble_sweep_listed: out of memory for the neighbour lists");
+  if (!ws) return nngp_fail(h, "ensemble_sweep: out of device memory");
   void* kws = ws;
   void* fws = ws + bk;
   long long* idx = (long long*)(ws + bk + bf);
@@ -1348,139 +1298,133 @@ static int ensemble_sweep_impl(nngp_handle_t h, int sys, int method_g, int h_mod
   int* order = (int*)(ws + bk + bf + bi + bd);
   double* t_rep = (double*)(ws + bk + bf + bi + bd + bo);
   double* q_knn = (double*)(ws + bk + bf + bi + bd + bo + bt);
-  {
-    const long long tot = (long long)(N + 1) * E;
-    if (d_t_pos)
-      transpose_t_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(d_t_pos, N + 1, E, t_rep);
-    else
-      repeat_t_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(d_t, N + 1, E, t_rep);
-    h->launches++;
-    NNGP_CUDA(h, cudaGetLastError());
-  }
-  // mixed: every slice's gather and scatter copies, in one table for the whole sweep; listed: every slice's listed
-  // preps, which write straight into their fit groups' inputs, and the gathers of the kNN queries when the slice has
-  // listed positions (its kNN positions are then no prefix of the state)
+  if (!in_place) G.carve(ws + bk + br, d, n_restarts, false);
+  // The plan, in one pass over the slices.  The positions active at slice i (I <= i) are a prefix: every launch reaches
+  // them with the member stride (N+1) d of the state, and their predicts' starts are consecutive in d_starts
+  // (slice-major).  Grouped: every slice's gather and scatter copies go to one table for the whole sweep, its listed
+  // preps (which write straight into their fit groups' inputs) to another, followed by the gathers of the kNN queries
+  // when the slice has listed positions (its kNN positions are then no prefix of the state).
+  std::vector<SlicePlan> plan;
   std::vector<CopySpan> sp;
-  std::vector<size_t> sp_at;  // per slice: start of its gather spans, start of its scatter spans
-  std::vector<ListedQuery> lq;
-  std::vector<size_t> lq_at;  // per slice: start of its listed preps
-  if (mixed) {
-    G.carve((char*)fws + Carver::pad(gp_prep_bytes(E, m)), d, n_restarts, false);
-    size_t done_predicts = 0;
-    int n_act = 0, nk_act = 0, mm = 0;
-    for (int i = I[0]; i < N; i++) {
-      for (; n_act < E && I[n_act] <= i; n_act++)
-        if (!is_listed(n_act)) mm = std::max(mm, m_pos[n_act]), nk_act++;
-      const signed char* starts_i = d_starts + done_predicts * per_predict;
+  std::vector<ListedQuery> lq;  // `rows` of an entry points into the host lists until they are uploaded
+  int n_act = 0, nk_act = 0, mm = 0, short_p = -1;
+  long long n_max = 0;
+  const signed char* starts_i = d_starts;
+  for (int i = I[0]; i < N; i++) {
+    for (; n_act < E && I[n_act] <= i; n_act++) {
+      if (is_listed(n_act)) continue;
+      const long long held = h->seg_rows[members[n_act]];
+      mm = std::max(mm, m[n_act]);
+      n_max = std::max(n_max, held);
+      if (short_p < 0 || held < h->seg_rows[members[short_p]]) short_p = n_act;
+      nk_act++;
+    }
+    // the kNN searches at the slice's largest m: a shorter segment would read padding indices as rows
+    if (short_p >= 0 && h->seg_rows[members[short_p]] < mm)
+      return nngp_fail(h, "ensemble_sweep: member %d holds %lld rows, fewer than m=%d, the largest m of slice %d",
+                       members[short_p], h->seg_rows[members[short_p]], mm, i);
+    SlicePlan P{n_act, nk_act, mm, n_max, starts_i, sp.size(), sp.size(), sp.size(), lq.size(), lq.size()};
+    if (!in_place) {
       const double* ui = d_u_next + (long long)i * d;
       const double* gn = d_uG_next + (long long)(i + 1) * d;
       double* un = d_u_next + (long long)(i + 1) * d;
-      sp_at.push_back(sp.size());
-      lq_at.push_back(lq.size());
       for (int p = 0, rk = 0; p < n_act; p++) {
         if (!is_listed(p)) {
           mixed_gather_spans(sp, G, p, rk++, idx, dist, (const double*)fws, mm, starts_i, per_predict, gn, ld, d);
           continue;
         }
-        const int r = G.rank[p], mg = G.m[G.grp[p]];
+        const int r = G.rank[p], mg = m[p];
         const MixedGroups::Dev& D = G.dev[G.grp[p]];
-        lq.push_back(ListedQuery{ui + p * ld, drows + row_at[p] + (size_t)(i - I[p]) * mg, D.idx + (size_t)r * mg,
-                                 D.dist + (size_t)r * mg, (double*)D.fws + (size_t)r * mg * mg, nullptr, mg, mg});
+        const long long base = (long long)members[p] * h->seg_cap, held = h->seg_rows[members[p]];
+        const long long* lr = rows + row_at[p] + (size_t)(i - I[p]) * mg;
+        for (int a = 0; a < mg; a++)
+          if (lr[a] < base || lr[a] >= base + held)
+            return nngp_fail(h, "ensemble_sweep: member %d, slice %d lists row %lld, outside its segment [%lld,%lld)",
+                             members[p], i, lr[a], base, base + held);
+        lq.push_back(ListedQuery{ui + p * ld, lr, D.idx + (size_t)r * mg, D.dist + (size_t)r * mg,
+                                 (double*)D.fws + (size_t)r * mg * mg, nullptr, mg, mg});
         mixed_gather_spans(sp, G, p, 0, nullptr, nullptr, nullptr, 0, starts_i, per_predict, gn, ld, d);
       }
-      if (lq.size() > lq_at.back())
+      if (lq.size() > P.lq)
         for (int r = 0; r < nk_act; r++)
           lq.push_back(ListedQuery{ui + kpos[r] * ld, nullptr, nullptr, nullptr, nullptr, q_knn + (size_t)r * d, 0, 0});
-      sp_at.push_back(sp.size());
+      P.scatter = sp.size();
       for (int p = 0; p < n_act; p++)
         sp.push_back(copy_span(G.dev[G.grp[p]].pred + (size_t)G.rank[p] * d, un + (size_t)p * ld, sizeof(double) * d));
-      done_predicts += n_act;
+      P.end = sp.size();
+      P.lq_end = lq.size();
     }
-    sp_at.push_back(sp.size());
-    lq_at.push_back(lq.size());
+    plan.push_back(P);
+    starts_i += (size_t)n_act * per_predict;
+  }
+  cudaStream_t st = as_stream(stream);
+  unsigned int* tickets = seg_tickets(h, E);
+  if (!tickets) return nngp_fail(h, "ensemble_sweep: out of device memory");
+  std::vector<long long> ktab(2 * (size_t)nk);  // [base | rows] of the kNN positions' segments
+  for (int r = 0; r < nk; r++) {
+    ktab[r] = (long long)members[kpos[r]] * h->seg_cap;
+    ktab[nk + r] = h->seg_rows[members[kpos[r]]];
+  }
+  const long long* dtab = nullptr;
+  if (nk > 0 && !(dtab = (const long long*)upload_table(h, 1, ktab.data(), sizeof(long long) * ktab.size(), st)))
+    return nngp_fail(h, "ensemble_sweep: out of memory for the segment table");
+  if (n_listed_rows > 0) {
+    const long long* drows = (const long long*)upload_table(h, 3, rows, sizeof(long long) * n_listed_rows, st);
+    if (!drows) return nngp_fail(h, "ensemble_sweep: out of memory for the neighbour lists");
+    for (ListedQuery& q : lq)
+      if (q.rows) q.rows = drows + (q.rows - rows);
   }
   const CopySpan* dsp = nullptr;
-  if (mixed && !(dsp = (const CopySpan*)upload_table(h, 2, sp.data(), sizeof(CopySpan) * sp.size(), st)))
+  if (!sp.empty() && !(dsp = (const CopySpan*)upload_table(h, 2, sp.data(), sizeof(CopySpan) * sp.size(), st)))
     return nngp_fail(h, "ensemble_sweep: out of memory for the copy table");
   const ListedQuery* dlq = nullptr;
   if (!lq.empty() && !(dlq = (const ListedQuery*)upload_table(h, 4, lq.data(), sizeof(ListedQuery) * lq.size(), st)))
-    return nngp_fail(h, "ensemble_sweep_listed: out of memory for the query table");
-  // The members active at slice i (I <= i) are a prefix of the positions: every launch below reaches them with the
-  // member stride (N+1) d of the state, and their predicts' starts are consecutive in d_starts (slice-major).
-  size_t done_predicts = 0;
-  int n_act = 0, nk_act = 0, mm = 0;
-  long long n_max = 0;
-  for (int i = I[0]; i < N; i++) {
-    for (; n_act < E && I[n_act] <= i; n_act++) {
-      if (is_listed(n_act)) continue;
-      if (mixed) mm = std::max(mm, m_pos[n_act]);
-      n_max = std::max(n_max, tab[E + n_act]);
-      nk_act++;
-    }
-    const signed char* starts_i = d_starts + done_predicts * per_predict;
+    return nngp_fail(h, "ensemble_sweep: out of memory for the query table");
+  {
+    const long long tot = (long long)(N + 1) * E;
+    transpose_t_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(d_t_pos, N + 1, E, t_rep);
+    h->launches++;
+    NNGP_CUDA(h, cudaGetLastError());
+  }
+  for (size_t k = 0; k < plan.size(); k++) {
+    const SlicePlan& P = plan[k];
+    const int i = I[0] + (int)k;
     double* ui = d_u_next + (long long)i * d;
     double* un = d_u_next + (long long)(i + 1) * d;
     double* gn = d_uG_next + (long long)(i + 1) * d;
-    if (mixed) {
-      const size_t* at = sp_at.data() + 2 * (size_t)(i - I[0]);
-      const size_t l0 = lq_at[i - I[0]], nl = lq_at[i - I[0] + 1] - l0;
-      if (int rc = sweep_slice_prologue(h, *s, method_g, h_mode, steps_g, n_act, t_rep + (size_t)i * E,
-                                        t_rep + (size_t)(i + 1) * E, ui, ld, gn, st, [&] {
-            if (int rc = listed_prep_launch(h, dlq + l0, (int)nl, st)) return rc;
-            if (nk_act == 0) return 0;
-            return knn_seg_launch(h, nl ? q_knn : ui, nl ? d : ld, nk_act, mm, dtab, dtab + nk, n_max, idx, dist,
-                                  (double*)fws, tickets, kws, st);
+    const double* t0 = t_rep + (size_t)i * E;
+    if (in_place) {
+      // the queue order needs only the starts: enqueued first, it stays off the path from the kNN to the fit
+      if (int rc = ensure_done_zero(h, h->done, fws, P.n_act, d, P.mm, n_restarts, st)) return rc;
+      if (int rc = gp_order_launch(h, P.starts, P.n_act, seg_len, 1, order, st)) return rc;
+      if (int rc = sweep_slice_prologue(h, *s, method_g, h_mode, steps_g, P.n_act, t0, t0 + E, ui, ld, gn, st, [&] {
+            return knn_seg_launch(h, ui, ld, P.n_act, P.mm, dtab, dtab + nk, P.n_max, idx, dist, (double*)fws, tickets,
+                                  kws, st);
           }))
         return rc;
-      if (int rc = copy_spans_launch(h, dsp + at[0], (int)(at[1] - at[0]), st)) return rc;
-      for (size_t g = 0; g < G.m.size(); g++) {
-        const int n_g = (int)(std::lower_bound(G.pos[g].begin(), G.pos[g].end(), n_act) - G.pos[g].begin());
-        if (n_g > 0)
-          if (int rc = mixed_fit_group(h, G, (int)g, n_g, d, n_restarts, fatol, xatol, true, st)) return rc;
-      }
-      if (int rc = copy_spans_launch(h, dsp + at[1], (int)(at[2] - at[1]), st)) return rc;
-      done_predicts += n_act;
+      if (int rc = gp_fit_predict_launch(h, idx, dist, fws, next_queue(h, st), order, P.n_act, P.mm, n_restarts,
+                                         P.starts, fatol, xatol, un, gn, ld, nullptr, nullptr, nullptr, nullptr, nullptr,
+                                         nullptr, st))
+        return rc;
       continue;
     }
-    if (int rc = ensure_done_zero(h, fws, n_act, d, m, n_restarts, st)) return rc;
-    if (int rc = gp_order_launch(h, starts_i, n_act, seg_len, 1, order, st)) return rc;
-    if (int rc = sweep_slice_prologue(h, *s, method_g, h_mode, steps_g, n_act, t_rep + (size_t)i * E,
-                                      t_rep + (size_t)(i + 1) * E, ui, ld, gn, st, [&] {
-          return knn_seg_launch(h, ui, ld, n_act, m, dtab, dtab + nk, n_max, idx, dist, (double*)fws, tickets, kws, st);
+    const int nl = (int)(P.lq_end - P.lq);
+    if (int rc = sweep_slice_prologue(h, *s, method_g, h_mode, steps_g, P.n_act, t0, t0 + E, ui, ld, gn, st, [&] {
+          if (int rc = listed_prep_launch(h, dlq + P.lq, nl, st)) return rc;
+          if (P.nk_act == 0) return 0;
+          return knn_seg_launch(h, nl ? q_knn : ui, nl ? d : ld, P.nk_act, P.mm, dtab, dtab + nk, P.n_max, idx, dist,
+                                (double*)fws, tickets, kws, st);
         }))
       return rc;
-    if (int rc = gp_fit_predict_launch(h, idx, dist, fws, next_queue(h, st), order, n_act, m, n_restarts, starts_i, fatol,
-                                       xatol, un, gn, ld, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, st))
-      return rc;
-    done_predicts += n_act;
+    if (int rc = copy_spans_launch(h, dsp + P.gather, (int)(P.scatter - P.gather), st)) return rc;
+    for (size_t g = 0; g < G.m.size(); g++) {
+      const int n_g = (int)(std::lower_bound(G.pos[g].begin(), G.pos[g].end(), P.n_act) - G.pos[g].begin());
+      if (n_g > 0)
+        if (int rc = mixed_fit_group(h, G, (int)g, n_g, d, n_restarts, fatol, xatol, true, st)) return rc;
+    }
+    if (int rc = copy_spans_launch(h, dsp + P.scatter, (int)(P.end - P.scatter), st)) return rc;
   }
   return 0;
-}
-
-int nngp_ensemble_sweep(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g, const double* d_t, int N,
-                        int E, const int* members, const int* I, int m, int n_restarts, const signed char* d_starts,
-                        double fatol, double xatol, double* d_u_next, double* d_uG_next, int d, void* stream) {
-  return ensemble_sweep_impl(h, sys, method_g, h_mode, steps_g, d_t, nullptr, N, E, members, I, m, nullptr, nullptr,
-                             nullptr, n_restarts, d_starts, fatol, xatol, d_u_next, d_uG_next, d, stream);
-}
-
-int nngp_ensemble_sweep_mixed(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g,
-                              const double* d_t_pos, int N, int E, const int* members, const int* I, const int* m,
-                              int n_restarts, const signed char* d_starts, double fatol, double xatol,
-                              double* d_u_next, double* d_uG_next, int d, void* stream) {
-  if (m == nullptr || d_t_pos == nullptr) return nngp_fail(h, "ensemble_sweep_mixed: m and d_t_pos are required");
-  return ensemble_sweep_impl(h, sys, method_g, h_mode, steps_g, nullptr, d_t_pos, N, E, members, I, 0, m, nullptr,
-                             nullptr, n_restarts, d_starts, fatol, xatol, d_u_next, d_uG_next, d, stream);
-}
-
-int nngp_ensemble_sweep_listed(nngp_handle_t h, int sys, int method_g, int h_mode, long long steps_g,
-                               const double* d_t_pos, int N, int E, const int* members, const int* I, const int* m,
-                               const int* listed, const long long* rows, int n_restarts, const signed char* d_starts,
-                               double fatol, double xatol, double* d_u_next, double* d_uG_next, int d, void* stream) {
-  if (m == nullptr || d_t_pos == nullptr || listed == nullptr)
-    return nngp_fail(h, "ensemble_sweep_listed: m, listed and d_t_pos are required");
-  return ensemble_sweep_impl(h, sys, method_g, h_mode, steps_g, nullptr, d_t_pos, N, E, members, I, 0, m, listed, rows,
-                             n_restarts, d_starts, fatol, xatol, d_u_next, d_uG_next, d, stream);
 }
 
 int nngp_selftest_math(nngp_handle_t h, const double* d_x, int n, double* d_exp_neg, double* d_rcp,

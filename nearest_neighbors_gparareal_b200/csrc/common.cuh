@@ -34,6 +34,13 @@ struct SysArgs {
   const double* mx;
 };
 
+// Where a fit block's per-(query, dim) completion counters last lived: the fit leaves them zero, so they are cleared
+// only when they move (ensure_done_zero).  Owned by whoever owns the block: the handle's workspace, a fit group.
+struct DoneTracker {
+  const void* ptr = nullptr;
+  size_t bytes = 0;
+};
+
 struct nngp_handle_s {
   int device = 0;
   std::string err;
@@ -92,7 +99,7 @@ struct nngp_handle_s {
   // small host->device tables of the segmented entry points: pinned staging, re-used once the copy that last read it
   // has completed (event)
   struct Upload { void* host = nullptr; void* dev = nullptr; size_t bytes = 0; cudaEvent_t done = nullptr; };
-  // 0 row tables, 1 segment tables, 2 copy spans of the mixed ensemble sweep, 3 neighbour lists and 4 ListedQuery
+  // 0 row tables, 1 segment tables, 2 copy spans of the grouped fits, 3 neighbour lists and 4 ListedQuery
   // tables of the listed sweeps
   Upload up[5];
   // device counters: [0] Nelder-Mead runs, [1] objective (nll) evaluations
@@ -100,9 +107,8 @@ struct nngp_handle_s {
   // task-queue heads of the persistent fit kernel: one zeroed counter per launch
   unsigned int* d_queues = nullptr;
   int queue_next = 0;
-  // where the (zero on exit) per-(query,dim) completion counters of the last fit lived
-  const void* done_ptr = nullptr;
-  size_t done_bytes = 0;
+  // where the completion counters of the last fit in the handle's workspace lived (ensure_done_zero)
+  DoneTracker done;
   // optional per-kernel-class timing with CUDA events on the launching stream
   bool profiling = false;
   struct ProfRec { int cls; cudaEvent_t a, b; };
@@ -163,7 +169,7 @@ int copy_rows_launch(nngp_handle_t h, const double* src, const long long* si, do
 int rowwise_maxabs_launch(nngp_handle_t h, const double* a, const double* b, int rows, int d,
                           double* err, cudaStream_t st);
 
-// One predict of a listed sweep (nngp_sweep_listed_shard, nngp_ensemble_sweep_listed): the GP inputs of query q from
+// One predict of a listed sweep (nngp_sweep_listed_shard, nngp_ensemble_sweep): the GP inputs of query q from
 // the m dataset rows a neighbour rule chose on the host, instead of from a kNN.  m == 0: the entry only copies the
 // query row to q_copy (the queries of the nearest-neighbour positions of a mixed slice, gathered to one row stride for
 // the segmented kNN that follows).  All pointers are device pointers.

@@ -2,11 +2,11 @@
 
 `PararealEnsemble.run(seeds=[...])` runs E solves of the same system, solver, N, `n_restarts`, `fatol` and `xatol` in
 lockstep; the runs may differ in seed, initial condition, epsilon, early_stop, neighbour count `nn`, neighbour rule
-`nntype` (models_alt.py; nngp_ensemble_sweep_listed when a running member uses a position rule) and time span.  Every
-iteration makes the launches of one `PararealDevice` iteration, each over all runs at once: one fine-step launch, one
-dataset append, and per slice of the sweep one coarse step, one kNN (each run searches its own rows of a segmented
-store, csrc/knn.cu) and one fit over all the runs' predicts -- one fit per distinct neighbour count when the runs'
-counts differ (nngp_ensemble_sweep_mixed).  Run e's output dict equals, bit for bit, what
+`nntype` (models_alt.py) and time span.  Every iteration makes the launches of one `PararealDevice` iteration, each
+over all runs at once: one fine-step launch, one dataset append and one nngp_ensemble_sweep, which per slice makes one
+coarse step, one kNN (each run searches its own rows of a segmented store, csrc/knn.cu; the runs with a position rule
+take the host's neighbour lists instead) and one fit over all the runs' predicts -- one fit per distinct neighbour
+count when the runs' counts differ.  Run e's output dict equals, bit for bit, what
 `PararealDevice(...).run(model='nngp', seed=seeds[e], ...)` returns with its settings.
 
 Layout: the state is [E, N+1, d] per array.  At the start of every iteration the member axis is re-ordered by
@@ -82,23 +82,21 @@ def listed_rows(mdl, e, first, I, base):
         raise ValueError(f'member {e}: {exc}') from exc
 
 
-def sweep_tables(m_members, t_members, sw):
-    """Per-position neighbour counts and time grids of a sweep over the members sw (state order)."""
-    sw = np.asarray(sw, dtype=np.int64)
-    return np.asarray(m_members, dtype=np.int32)[sw], np.ascontiguousarray(np.asarray(t_members)[sw])
+def sweep_tables(m_members, sw):
+    """Per-position neighbour counts of a sweep over the members sw (state order)."""
+    return np.asarray(m_members, dtype=np.int32)[np.asarray(sw, dtype=np.int64)]
 
 
-def launch_sweep(h, t_dev, sysid, mG, hm, steps, N, sw, I_sw, m_pos, t_pos, mdl0, starts, u_next, uG_next, n, stream):
-    """nngp_ensemble_sweep when every position has the same m and grid, otherwise nngp_ensemble_sweep_mixed.
-    t_dev: the members' grids [E, N+1], uploaded once per run; rows are selected on the device."""
+def launch_sweep(h, t_dev, sysid, mG, hm, steps, N, sw, I_sw, m_pos, listed_sw, lists, mdl0, starts, u_next, uG_next, n,
+                 stream):
+    """The sweep over the members sw (state order).  t_dev: the members' grids [E, N+1], uploaded once per run; the
+    swept members' rows are selected on the device.  listed_sw: which of them take the neighbour lists `lists`."""
     import torch
-    if np.all(m_pos == m_pos[0]) and np.all(t_pos == t_pos[0]):
-        h.ensemble_sweep(sysid, mG, hm, steps, t_dev[int(sw[0])], N, sw, I_sw, int(m_pos[0]), mdl0.n_restarts, starts,
-                         mdl0.fatol, mdl0.xatol, u_next, uG_next, n, stream)
-    else:
-        rows = torch.from_numpy(np.asarray(sw, dtype=np.int64)).to(t_dev.device)
-        h.ensemble_sweep_mixed(sysid, mG, hm, steps, t_dev.index_select(0, rows), N, sw, I_sw, m_pos,
-                               mdl0.n_restarts, starts, mdl0.fatol, mdl0.xatol, u_next, uG_next, n, stream)
+    rows = torch.from_numpy(np.asarray(sw, dtype=np.int64)).to(t_dev.device)
+    if not np.any(listed_sw):
+        listed_sw = lists = None
+    h.ensemble_sweep(sysid, mG, hm, steps, t_dev.index_select(0, rows), N, sw, I_sw, m_pos, mdl0.n_restarts, starts,
+                     mdl0.fatol, mdl0.xatol, u_next, uG_next, n, listed_sw, lists, stream)
 
 
 def member_order(I, done):
@@ -284,14 +282,9 @@ class PararealEnsemble:
                 for e, tab in zip(sw, lists):
                     if tab is not None:
                         m_members[e] = tab.shape[1]
-                m_pos, t_pos = sweep_tables(m_members, t_members, sw)
+                m_pos = sweep_tables(m_members, sw)
                 if m_pos.max() > MAX_NEIGHBOURS:
                     raise Exception('nn > 160 neighbours is not supported (include/nngpara.h: NNGP_MAX_NEIGHBOURS_BIG)')
-                m = int(m_pos[0])
-                short = [e for e in sw if rows[e] < m]
-                if short and np.all(m_pos == m) and not listed[sw].any():
-                    raise Exception(f'members {short} hold fewer dataset rows ({rows[short].min()}) than the common m={m}: '
-                                    'an ensemble needs one m per launch')
                 blocks = []
                 for e in sw:
                     mdl = models[e]
@@ -299,14 +292,8 @@ class PararealEnsemble:
                     blocks.append(mdl.draw_starts(N - I[e]))
                     mdl.train_count += (N - I[e]) * n * N_JITTER * mdl.n_restarts
                 starts = torch.from_numpy(pack_starts(blocks, I[sw], N)).to(dev)
-                if listed[sw].any():
-                    t_sw = t_dev.index_select(0, torch.from_numpy(np.asarray(sw, dtype=np.int64)).to(dev))
-                    h.ensemble_sweep_listed(sysid, mG, hm, solver.Ng, t_sw, N, sw, I[sw], m_pos, listed[sw], lists,
-                                            mdl0.n_restarts, starts, mdl0.fatol, mdl0.xatol, st['u_next'],
-                                            st['uG_next'], n, stream)
-                else:
-                    launch_sweep(h, t_dev, sysid, mG, hm, solver.Ng, N, sw, I[sw], m_pos, t_pos, mdl0, starts,
-                                 st['u_next'], st['uG_next'], n, stream)
+                launch_sweep(h, t_dev, sysid, mG, hm, solver.Ng, N, sw, I[sw], m_pos, listed[sw], lists, mdl0, starts,
+                             st['u_next'], st['uG_next'], n, stream)
             # parareal.py:402: one error launch over the running members and ONE device->host read
             h.rowwise_maxabs_diff(st['u_next'], st['u_cur'], n_live * (N + 1), n, err_dev, stream)
             errs = err_dev[:n_live * (N + 1)].cpu().numpy().reshape(n_live, N + 1)

@@ -147,14 +147,9 @@ def test_burgers_published_slice_as_one_ensemble():
         _same(outs[e], ref, (T, nnb, seed))
 
 
-def test_row_shortfall_is_refused_before_the_slice_is_launched():
-    """nn=60 beside nn=11 at the first iteration, where every member holds N = 50 rows"""
-    cfg, eps, key, kw, mkw = _setup("lorenz_N50_m11")
-    mkw.pop('nn', None)
-    ode = device_system(key, **kw)
-    ens = nn.PararealEnsemble(ode, _solver(ode, cfg), tspan=cfg["tspan"], N=cfg["N"], epsilon=eps, verbose='')
-    h = ens.handle()
-    sweep, launches = h.ensemble_sweep_mixed, []
+def _counted(h):
+    """wraps h.ensemble_sweep: the list it returns gets the launches of every call"""
+    sweep, launches = h.ensemble_sweep, []
 
     def counted_sweep(*args):
         c0 = h.launch_count()
@@ -163,7 +158,34 @@ def test_row_shortfall_is_refused_before_the_slice_is_launched():
         finally:
             launches.append(h.launch_count() - c0)
 
-    h.ensemble_sweep_mixed = counted_sweep
-    with pytest.raises(Exception, match=r"member \d+ holds 50 rows, fewer than m=60"):
-        ens.run(model='nngp', seeds=[45, 46], nn=[11, 60], **mkw)
-    assert launches == [0], launches
+    h.ensemble_sweep = counted_sweep
+    return launches
+
+
+def test_one_nn_with_their_own_tspans_sweeps_in_place():
+    """one m for all, two time spans: the in-place route reads each member's grid from the per-position table"""
+    cfg, eps, key, kw, mkw = _setup("burgers_d32_N32_m12")
+    mkw.pop('nn', None)
+    Ts, seeds = [5.0, 5.9, 5.0, 5.9], [45, 46, 47, 48]
+    ode = device_system(key, **kw)
+    ens = nn.PararealEnsemble(ode, _solver(ode, cfg), tspan=cfg["tspan"], N=cfg["N"], epsilon=eps, verbose='')
+    launches = _counted(ens.handle())
+    outs = ens.run(model='nngp', seeds=seeds, nn=12, tspans=[[0, T] for T in Ts], **mkw)
+    # the first sweep, all four members at I = 1: the time table, then per slice the queue order, the coarse step,
+    # the segmented kNN and the grouped fit (searches, then selection and mean)
+    assert launches[0] == 1 + 5 * (cfg["N"] - 1), launches
+    for s, T, o in zip(seeds, Ts, outs):
+        _same(o, _solo(key, kw, dict(cfg, tspan=[0, T]), eps, dict(mkw, nn=12), s), (s, T))
+
+
+def test_row_shortfall_is_refused_by_the_library_before_any_launch():
+    """nn=60 beside nn=11, and nn=60 for both, at the first iteration, where every member holds N = 50 rows"""
+    cfg, eps, key, kw, mkw = _setup("lorenz_N50_m11")
+    mkw.pop('nn', None)
+    for nns in ([11, 60], [60, 60]):
+        ode = device_system(key, **kw)
+        ens = nn.PararealEnsemble(ode, _solver(ode, cfg), tspan=cfg["tspan"], N=cfg["N"], epsilon=eps, verbose='')
+        launches = _counted(ens.handle())
+        with pytest.raises(_lib.NNGPError, match=r"member \d+ holds 50 rows, fewer than m=60"):
+            ens.run(model='nngp', seeds=[45, 46], nn=nns, **mkw)
+        assert launches == [0], (nns, launches)
